@@ -2,7 +2,7 @@
 """bench.py — SCoNe train trajectories/s on B200 (BASELINE.json metric), one JSON line on rank 0.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg5|cfg4|cfg1|cfg3-ebli|cfg3-bunch]
-                    [--scaling strong|weak]
+                    [--scaling strong|weak] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -200,6 +200,17 @@ def make_dataset(name, cfg, n_traj, seed):
     return sdg.generate_sparse_dataset(cfg['n_nodes'], n_traj, seed=seed, n_waypoints=24, cuts_per_walk=cfg['cuts']), None
 
 
+def dump_outputs(path, grad_buffer, weights=None):
+    """What a caller of the timed step receives from its last run: the flat [grads | nll_sum | count] buffer of that step and, when
+    the step ends with an Adam update, the flat weights after it.  The inputs are seeded, so two builds run with the same arguments
+    compare file for file."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, 'grad_buffer.npy'), np.asarray(grad_buffer, np.float32))
+    if weights is not None:
+        np.save(os.path.join(path, 'weights.npy'), np.asarray(weights, np.float32))
+
+
 def tri_lists(sp):
     from scone_gcn_b200.complex import incidence_lists_from_simplices
     return incidence_lists_from_simplices(sp.edges, sp.faces)
@@ -243,6 +254,8 @@ def run_reference(args, cfg, rank, world):
     W = [0.01 * rs.randn(*s) for s in [(1, C)] * 3 + [(C, C)] * 6 + [(C, 1)]]
     n_sample = sample_size(E)
     lp, nll, grads, times, threads = oracle_sample(sp, model, W, n_sample, args.warmup + args.steps)
+    if args.dump_outputs:                                  # the oracle step has no optimizer update: gradients and loss only
+        dump_outputs(args.dump_outputs, np.concatenate([g.ravel() for g in grads] + [np.array([nll, n_sample])]))
     times = times[args.warmup:] or times
     tps = n_sample / (sum(times) / len(times))
     sample = '%d trajectories fwd+bwd per step on the same complex (E=%d), sparse CSR CPU port of the reference maths' % (n_sample, E)
@@ -275,7 +288,12 @@ def main():
     ap.add_argument('--e2e-steps', type=int, default=10)
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-extras', dest='extras', action='store_false', help='skip the dense-tile roofline measurement')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed (grad_buffer.npy, and weights.npy after the Adam update; '
+                         'float32) to DIR')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     cfg = dict(CONFIGS[args.config])
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -424,6 +442,8 @@ def main():
     net.check_overflow(stream)                             # a truncated step would have been timed silently otherwise
     if exchange is not None:
         exchange.status(stream)                            # ... and so would a step whose peers never delivered their gradients
+    if args.dump_outputs and rank == 0:                    # before the passes below run more steps on the same model
+        dump_outputs(args.dump_outputs, net.read_grads(stream), net.flatten(net.get_weights()))
     ms_per_step = ms_total / args.steps
     value = gb * args.steps / (ms_total / 1e3)
 
@@ -729,6 +749,8 @@ def bench_bunch(args, cfg, sp, ds, hp, h2d_bytes, B, gb, world, rank, dev, strea
     torch.cuda.synchronize()
     ms = ev0.elapsed_time(ev1)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, net.read_grads(stream), net.flatten(net.get_weights()))
     value = B * args.steps / (ms / 1e3)
     peak, peak_src = load_peaks()
     out = {'metric': 'SCoNe train trajectories/sec', 'value': value, 'unit': 'trajectories/s', 'n_gpus': world, 'steps': args.steps,

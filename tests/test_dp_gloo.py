@@ -63,7 +63,8 @@ def test_two_rank_allreduce_matches_single_process(tmp_path):
 
 
 def _shard_worker(rank, world, port, out):
-    os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
+    # no visible GPU: dp.init_from_env would otherwise take NCCL with one GPU per rank, and this test is about the gloo path
+    os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), CUDA_VISIBLE_DEVICES='')
     from scone_gcn_b200 import dp
     assert dp.init_from_env() == (rank, world) and dp.is_distributed()
     rows = np.arange(100, 137)                              # the batch rows every rank derives from the shared RNG stream
