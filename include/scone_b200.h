@@ -27,6 +27,9 @@ extern "C" {
 #endif
 
 #define SCONE_B200_VERSION 100
+/* Largest maximum node degree D (width of the neighbour table) the model entry points support: the readout, cone and plan kernels
+ * keep per-slot arrays of this size in shared memory.  scone_model_create rejects a complex with a larger D (error code 2). */
+#define SCONE_MAX_DEGREE 128
 
 typedef struct scone_complex scone_complex;   /* simplicial complex: device-resident index arrays */
 typedef struct scone_model scone_model;       /* weights + Adam state + activation workspace     */

@@ -32,7 +32,7 @@ namespace {
 #include "slab_common.cuh"
 
 constexpr int kTrajThreads = 256;
-constexpr int kFuMaxD = 128;
+constexpr int kFuMaxD = SCONE_MAX_DEGREE;
 constexpr uint32_t kNoRow = 0xFFFFu;
 constexpr uint32_t kFlaggedKey = 0xFFFFFFu;   // sort key of a trajectory the plan kernel flagged (overflow): belongs to no launch
 

@@ -1117,7 +1117,7 @@ __global__ void flows_to_dense_kernel(const int32_t* __restrict__ traj_ptr, cons
 // =================================================================================================================
 // Readout: one CTA per trajectory.
 // =================================================================================================================
-constexpr int kReadoutMaxD = 128, kReadoutMaxCper = 4;   // D <= 128, C <= 128
+constexpr int kReadoutMaxD = SCONE_MAX_DEGREE, kReadoutMaxCper = 4;   // D <= 128, C <= 128
 
 // One CTA (4 warps) per trajectory; warp w owns the neighbour slots j = w, w + 4, ...  A row of GL receives at most two
 // contributions (an edge has two end nodes), added with atomicAdd onto a zeroed row: a + b == b + a, so the result does not

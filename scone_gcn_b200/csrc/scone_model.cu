@@ -472,6 +472,8 @@ extern "C" int scone_model_create(const scone_complex* cx, int32_t n_layers, con
     *out = nullptr;
     SCONE_REQUIRE(cx && hidden && n_layers >= 1 && micro_batch >= 1, "scone_model_create: bad arguments");
     SCONE_REQUIRE(!cx->host_only, "scone_model_create: index-only complex has no device arrays");
+    SCONE_REQUIRE(cx->D <= SCONE_MAX_DEGREE, "scone_model_create: max node degree %d exceeds the supported maximum of %d", cx->D,
+                  SCONE_MAX_DEGREE);
     scone_model* m = new scone_model();
     m->cx = cx;
     m->L = n_layers;

@@ -30,7 +30,7 @@ constexpr int kTbLC = 16384;             // cone entries one build CTA can hold 
 constexpr uint32_t kEdgeMask = 0x3FFFFFFFu;
 constexpr uint32_t kEmpty = 0xFFFFFFFFu;
 constexpr uint32_t kNoRow = 0xFFFFu;
-constexpr int kTbMaxD = 128;
+constexpr int kTbMaxD = SCONE_MAX_DEGREE;
 constexpr int kTbBuckets = 1024;
 
 __device__ __forceinline__ int align2(int x) { return (x + 1) & ~1; }

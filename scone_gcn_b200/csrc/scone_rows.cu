@@ -25,7 +25,7 @@ namespace {
 
 #include "slab_common.cuh"
 
-constexpr int kRoWarps = 8, kRoMaxD = 128, kRoMaxCper = 4;     // readout / cone kernels: max degree, channels per lane
+constexpr int kRoWarps = 8, kRoMaxD = SCONE_MAX_DEGREE, kRoMaxCper = 4;     // readout / cone kernels: max degree, channels per lane
 constexpr int kRoItems = 1024;                                  // (neighbour, incident edge) pairs of a trajectory staged in shared memory
 
 template <int ACT>

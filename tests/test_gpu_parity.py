@@ -359,7 +359,8 @@ def test_model_results_identical_with_and_without_zero_fill(small, zero_fill):
 
 
 @pytest.mark.parametrize('model,hidden,mb', [('scone', [16, 16, 16], 32), ('scone', [32, 32, 32], 7), ('ebli', [16, 32, 16], 64),
-                                             ('scone', [32], 16), ('scone', [16, 32], 5)])
+                                             ('scone', [32], 16), ('scone', [16, 32], 5), ('scone', [16, 16, 16, 16], 13),
+                                             ('ebli', [32, 32, 32, 32], 40)])
 def test_row_list_pipeline_matches_unit_kernel_pipeline(small, model, hidden, mb):
     """Model level: the bitmap-native row-list pipelines (tensor-core kernels; 3 = compact tensors over the readout cone,
     2 = compact tensors over the whole support, 1 = dense tensors) against the unit-kernel pipeline (0: fp32 SIMT, byte flags):

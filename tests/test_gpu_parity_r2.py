@@ -79,13 +79,28 @@ def test_ebli_hidden32_on_sparse_complex_vs_sparse_oracle():
 
 
 @pytest.mark.parametrize('model,hidden,scale', [('ebli', [32, 32, 32], 0.05), ('scone', [16, 32, 16], 0.3), ('ebli', [32, 16], 0.05),
-                                                ('scone', [32], 0.3)])
+                                                ('scone', [32], 0.3), ('scone', [8, 8, 8], 0.4), ('scone', [64, 64, 64], 0.15),
+                                                ('scone', [8, 16, 32], 0.3), ('ebli', [64, 32, 16], 0.03), ('scone', [32, 64], 0.2),
+                                                ('scone', [8], 0.4), ('scone', [64], 0.2), ('scone', [16, 16, 16, 16], 0.3),
+                                                ('scone', [32, 32, 32, 32, 32], 0.2)])
 def test_widths_and_depths_vs_dense_oracle(model, hidden, scale):
-    """ebli h32, mixed widths, 1- and 2-layer nets against the DENSE oracle (the reference formulation) on the small complex."""
+    """ebli h32, mixed widths (ratio-2 chains through 8 and 64), widths 8 and 64, 1- and 2-layer nets and nets deeper than 3 layers
+    against the DENSE oracle (the reference formulation) on the small complex, on the pipeline each starts on: widths 8 / 64 only run
+    on the unit kernels (0) and every other pipeline refuses them; more than 3 layers or mixed widths are not fused and start on the
+    cone pipeline (3, D = 9 here); uniform 16 / 32 with at most 3 layers start fused (4)."""
     import scone_gcn_b200 as sg
+    from scone_gcn_b200._lib import SconeError
     ds = Dataset('dataset_small.npz')
     cx = sg.SimplicialComplex.from_dense(ds.B1, ds.B2, model)
     net = sg.SconeModel(cx, hidden, micro_batch=40)
+    if any(c in (8, 64) for c in hidden):
+        assert net.pipeline == 0
+        for which in (1, 2, 3, 4):
+            with pytest.raises(SconeError):
+                net.set_pipeline(which)
+        assert net.pipeline == 0
+    else:
+        assert net.pipeline == (4 if len(set(hidden)) == 1 and len(hidden) <= 3 else 3)
     rs = np.random.RandomState(9)
     W = [scale * rs.randn(*s) for s in net.shapes]
     net.set_weights(W)
