@@ -298,6 +298,11 @@ int scone_model_read_rows_done(scone_model* m, int64_t* out /* [2] */);
  * reference order S_00, S_10, S_01, S_11, S_21, S_12, S_22.  Edge rows keep the CALLER's order on this path.
  * hidden[i] = width of hidden layer i; the model has n_hidden + 1 layers of 7 weights (the last maps to 1 channel),
  * weights flat in list order.  Same [grads | nll_sum | count] / Adam contract as scone_model.
+ * Operators may have zero rows or columns: a complex without triangles (F = 0) has S_21 E x 0, S_12 0 x E and S_22 0 x 0, and
+ * runs like any other (the weights of those operators get a zero gradient).  There is no degree limit on this path.
+ * Checked (error code 2, nothing copied or launched): every hidden width >= 1 and every nbrhoods entry in [-1, N) at creation;
+ * every last_nodes entry in [0, N) and every target_idx entry in [0, D) in the host entry points (an O(B) loop over host arrays).
+ * B = 0: forward writes nothing; loss_grad only clears the buffer when zero_first != 0 and otherwise leaves it as it is.
  * ------------------------------------------------------------------------------------------- */
 typedef struct scone_csr scone_csr;
 typedef struct scone_bunch scone_bunch;

@@ -366,7 +366,8 @@ int up(T** dst, const T* src, size_t n) {
 }  // namespace
 
 extern "C" int scone_csr_create(int32_t rows, int32_t cols, const int32_t* rowptr, const int32_t* col, const float* val, scone_csr** out) {
-    SCONE_REQUIRE(out && rowptr && rows > 0 && cols > 0, "scone_csr_create: bad arguments");
+    // rows / cols may be 0: a complex without triangles has F = 0, so S_21 is E x 0, S_12 is 0 x E and S_22 is 0 x 0
+    SCONE_REQUIRE(out && rowptr && rows >= 0 && cols >= 0, "scone_csr_create: bad arguments");
     *out = nullptr;
     const int64_t nnz = rowptr[rows];
     SCONE_REQUIRE(nnz == 0 || (col && val), "scone_csr_create: NULL col/val");
@@ -443,6 +444,11 @@ extern "C" int scone_bunch_create(const scone_csr* const* S7, int32_t N, int32_t
                                   int32_t n_hidden, const int32_t* hidden, int32_t micro_batch, scone_bunch** out) {
     SCONE_REQUIRE(out && S7 && nbrhoods && hidden && n_hidden >= 1 && micro_batch >= 1 && D >= 1, "scone_bunch_create: bad arguments");
     *out = nullptr;
+    for (int i = 0; i < n_hidden; ++i) SCONE_REQUIRE(hidden[i] >= 1, "scone_bunch_create: hidden width %d of layer %d is below 1", hidden[i], i);
+    // the readout gathers node rows through this table: an entry outside [-1, N) would read outside the node state
+    for (int64_t p = 0; p < (int64_t)N * D; ++p)
+        SCONE_REQUIRE(nbrhoods[p] >= -1 && nbrhoods[p] < N, "scone_bunch_create: nbrhoods[%lld][%lld] = %d is outside [-1, %d)",
+                      (long long)(p / D), (long long)(p % D), nbrhoods[p], N);
     const int32_t rows_of[3] = {N, E, F};
     for (int k = 0; k < 7; ++k) {
         SCONE_REQUIRE(S7[k] != nullptr, "scone_bunch_create: shift %d is NULL", k);
@@ -533,10 +539,20 @@ int ensure_staging(scone_bunch* m, int64_t B, int64_t nnz) {
     return 0;
 }
 
+// The readout uses both arrays as device indices: every last node must be a node, every target a slot of the neighbour table.
+int check_readout_indices(const char* fn, const scone_bunch* m, int32_t B, const int32_t* last, const int32_t* tgt) {
+    for (int32_t t = 0; t < B; ++t) {
+        SCONE_REQUIRE(last[t] >= 0 && last[t] < m->n[0], "%s: last_nodes[%d] = %d is outside [0, %d)", fn, t, last[t], m->n[0]);
+        if (tgt) SCONE_REQUIRE(tgt[t] >= 0 && tgt[t] < m->D, "%s: target_idx[%d] = %d is outside [0, %d)", fn, t, tgt[t], m->D);
+    }
+    return 0;
+}
+
 bool fused_width(int c) { return c == 1 || c == 8 || c == 16; }
 
 template <bool FWD>
 int launch_level(const BunchOps& o, float* out, int rows, int b, int cin, int cout, cudaStream_t st) {
+    if (rows == 0) return 0;                                  // an empty level (F = 0): nothing to write
     const unsigned grid = (unsigned)(((long long)rows * b + kBT - 1) / kBT);
 #define SCONE_BUNCH_CASE(CI, CO)                                                                          \
     if (cin == CI && cout == CO) {                                                                       \
@@ -576,6 +592,7 @@ int bunch_forward_mb(scone_bunch* m, int b, const int32_t* ptr, const int32_t* e
         bool first[3] = {true, true, true};
         for (int k = 0; k < 7; ++k) {
             const scone_csr* S = m->S[k];
+            if (S->rows == 0) continue;                       // writes an empty level (F = 0)
             const int ol = kOutLevel[k], il = kInLevel[k];
             const int wdt = b * cin;
             csr_spmm_kernel<<<nblk((long long)S->rows * wdt), kBT, 0, st>>>(S->d_rowptr, S->d_col, S->d_val, m->act[il][i], m->d_U, S->rows,
@@ -589,6 +606,7 @@ int bunch_forward_mb(scone_bunch* m, int b, const int32_t* ptr, const int32_t* e
         }
         for (int lv = 0; lv < 3; ++lv) {
             const long long n = (long long)m->n[lv] * b * cout;
+            if (n == 0) continue;
             relu_kernel<<<nblk(n), kBT, 0, st>>>(m->act[lv][i + 1], n);
             SCONE_LAUNCHED();
         }
@@ -601,6 +619,7 @@ int bunch_forward_mb(scone_bunch* m, int b, const int32_t* ptr, const int32_t* e
 extern "C" int scone_bunch_forward_host(scone_bunch* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
                                         const int32_t* last, float* logprobs_out, void* stream) {
     SCONE_REQUIRE(m && ptr && last && logprobs_out && B >= 0, "scone_bunch_forward_host: bad arguments");
+    if (check_readout_indices("scone_bunch_forward_host", m, B, last, nullptr)) return 2;
     if (B == 0) return 0;
     cudaStream_t st = as_stream(stream);
     const int64_t nnz = ptr[B];
@@ -626,20 +645,20 @@ extern "C" int scone_bunch_forward_host(scone_bunch* m, int32_t B, const int32_t
 extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
                                           const int32_t* last, const int32_t* tgt, const float* mask, int32_t zero_first, void* stream) {
     SCONE_REQUIRE(m && ptr && last && tgt && mask && B >= 0, "scone_bunch_loss_grad_host: bad arguments");
+    if (check_readout_indices("scone_bunch_loss_grad_host", m, B, last, tgt)) return 2;
     cudaStream_t st = as_stream(stream);
-    const int64_t nnz = B > 0 ? ptr[B] : 0;
+    if (zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * 4, st));
+    if (B == 0) return 0;                                     // nothing to add: the buffer is cleared (zero_first) or left as it is
+    const int64_t nnz = ptr[B];
     if (ensure_staging(m, B, nnz)) return 1;
     SCONE_CUDA(cudaMemcpyAsync(m->d_ptr, ptr, (B + 1) * 4, cudaMemcpyHostToDevice, st));
     if (nnz) {
         SCONE_CUDA(cudaMemcpyAsync(m->d_edge, edge, nnz * 4, cudaMemcpyHostToDevice, st));
         SCONE_CUDA(cudaMemcpyAsync(m->d_val, val, nnz * 4, cudaMemcpyHostToDevice, st));
     }
-    if (B) {
-        SCONE_CUDA(cudaMemcpyAsync(m->d_last, last, B * 4, cudaMemcpyHostToDevice, st));
-        SCONE_CUDA(cudaMemcpyAsync(m->d_tgt, tgt, B * 4, cudaMemcpyHostToDevice, st));
-        SCONE_CUDA(cudaMemcpyAsync(m->d_mask, mask, B * 4, cudaMemcpyHostToDevice, st));
-    }
-    if (zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * 4, st));
+    SCONE_CUDA(cudaMemcpyAsync(m->d_last, last, B * 4, cudaMemcpyHostToDevice, st));
+    SCONE_CUDA(cudaMemcpyAsync(m->d_tgt, tgt, B * 4, cudaMemcpyHostToDevice, st));
+    SCONE_CUDA(cudaMemcpyAsync(m->d_mask, mask, B * 4, cudaMemcpyHostToDevice, st));
     const int L = m->L;
     for (int32_t off = 0; off < B; off += m->mb) {
         const int b = B - off < m->mb ? B - off : m->mb;
@@ -657,6 +676,7 @@ extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32
             // G = dX * relu'(output of layer i)
             for (int lv = 0; lv < 3; ++lv) {
                 const long long n = (long long)m->n[lv] * b * cout;
+                if (n == 0) continue;
                 relu_bwd_kernel<<<nblk(n), kBT, 0, st>>>(m->d_dX[lv], m->act[lv][i + 1], m->d_G[cur][lv], n);
                 SCONE_LAUNCHED();
             }
@@ -666,6 +686,7 @@ extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32
                     const scone_csr* S = m->S[k];
                     const int ol = kOutLevel[k], il = kInLevel[k];
                     const long long M = (long long)S->rows * b;
+                    if (M == 0) continue;                     // an operator into an empty level: its weight gradient stays 0
                     const int tiles = ((cin + kOT - 1) / kOT) * ((cout + kOT - 1) / kOT);
                     const int nb = (int)std::min<long long>(kOuterBlocks, (M + kBT - 1) / kBT);
                     outer_tile_spmm_kernel<<<dim3(nb, tiles), kBT, 0, st>>>(S->d_rowptr, S->d_col, S->d_val, m->act[il][i], m->d_G[cur][ol],
@@ -693,6 +714,7 @@ extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32
                 for (int lv = 0; lv < 3; ++lv) SCONE_CUDA(cudaMemsetAsync(m->d_dX[lv], 0, (size_t)m->n[lv] * b * cin * 4, st));
             for (int k = 0; k < 7; ++k) {
                 const scone_csr* S = m->S[k];
+                if (S->rows == 0) continue;                   // an operator into an empty level: no weight or input gradient
                 const int ol = kOutLevel[k], il = kInLevel[k];
                 const int wdt = b * cin;
                 const long long M = (long long)S->rows * b;
@@ -713,7 +735,7 @@ extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32
                         SCONE_LAUNCHED();
                     }
                 }
-                if (i > 0) {
+                if (i > 0 && S->cols > 0) {
                     rows_times_wt_kernel<<<nblk(M * cin), kBT, 0, st>>>(m->d_G[cur][ol], m->d_w + m->w_off[7 * i + k], m->d_dU, M, cin, cout);
                     SCONE_LAUNCHED();
                     csr_spmm_kernel<<<nblk((long long)S->cols * wdt), kBT, 0, st>>>(S->d_t_rowptr, S->d_t_col, S->d_t_val, m->d_dU,
