@@ -47,10 +47,11 @@ struct ScopedProf {
     ~ScopedProf() { if (g_scone_prof) scone_prof_end_impl(kind, st); }
 };
 
-// Hints the model-level code gives to the next flagged kernel-level call on this thread (consumed by scone_hints_take):
+// Hints the model-level code passes to one flagged kernel-level call (the *_hinted functions and scone_readout_ws below; nullptr =
+// none, which is what the public C entry points pass):
 //   in_wl/in_tt   the previous call's output worklist (index in the scratch, unit width) describes occ_in -> no re-compaction
 //   skip_fill     the caller zero-fills the output tensor itself (e.g. on a side stream)
-// out_wl/out_tt are written back by the call.
+// out_wl/out_tt are written back by the call (out_wl stays -1 when it built no output worklist).
 //   in_bm         row bitmap of occ_in (bit e*b + t set <=> flag byte set): compaction reads it instead of the E*b flag bytes
 //   out_bm        row bitmap the producer call (scone_flows_to_dense, scone_readout) should set next to the flags it writes
 struct SconeLaunchHints {
@@ -61,7 +62,6 @@ struct SconeLaunchHints {
     uint32_t* cand_bm = nullptr;     // readout: also mark the candidate rows one hop beyond the rows of G_L it writes
 };
 static inline size_t scone_bitmap_words(size_t E, size_t b) { return ((E * b + 31) / 32 + 31) / 16 * 16; }   // padded to whole 64-byte groups
-extern thread_local SconeLaunchHints g_scone_hints;
 
 // Integer-valued shift operator in CSR form.  ent[p] = {column, float bits of the coefficient};
 // columns ascending inside a row (fixed, deterministic summation order).
@@ -103,16 +103,26 @@ int scone_zero_fill(const scone_complex* cx, void* p, size_t bytes, cudaStream_t
 // internal kernels-level helpers implemented in scone_kernels.cu
 int scone_layer0_forward(const scone_complex* cx, int32_t act, int32_t b, int32_t cout, const float* X_dev,
                          const float* W0, const float* W1, const float* W2, float* Hout, const uint8_t* occ_in, uint8_t* occ_out,
-                         uint8_t* scratch, void* stream);
+                         uint8_t* scratch, void* stream, SconeLaunchHints* hints);
 int64_t scone_layer0_backward_workspace_bytes(int32_t cout);
 int scone_layer0_backward(const scone_complex* cx, int32_t b, int32_t cout, const float* G_dev, const float* X_dev,
                           float* dW_dev, int32_t accumulate, void* workspace, const uint8_t* occ_g, uint8_t* scratch,
-                          void* stream);
+                          void* stream, const SconeLaunchHints* hints);
 int64_t scone_readout_workspace_bytes(int32_t b, int32_t C);
+// scone_flows_to_dense, scone_layer_forward, scone_layer_backward and scone_readout of scone_b200.h, with launch hints
+int scone_flows_to_dense_hinted(const scone_complex* cx, int32_t b, const int32_t* traj_ptr, const int32_t* flow_edge,
+                                const float* flow_val, float* X, uint8_t* occX, void* stream, const SconeLaunchHints* hints);
+int scone_layer_forward_hinted(const scone_complex* cx, int32_t act, int32_t b, int32_t cin, int32_t cout, const float* Hin,
+                               const float* W0, const float* W1, const float* W2, float* Hout, const uint8_t* occ_in,
+                               uint8_t* occ_out, uint8_t* occ_scratch, void* stream, SconeLaunchHints* hints);
+int scone_layer_backward_hinted(const scone_complex* cx, int32_t act, int32_t b, int32_t cin, int32_t cout, const float* G,
+                                const float* Hin, const float* W0, const float* W1, const float* W2, float* Gprev, float* dW,
+                                int32_t accumulate, void* workspace, const uint8_t* occ_g, const uint8_t* occ_hin,
+                                uint8_t* occ_prev, uint8_t* occ_scratch, void* stream, SconeLaunchHints* hints);
 int scone_readout_ws(const scone_complex* cx, int32_t act, int32_t b, int32_t C, const float* HL, const float* wout,
                      const int32_t* last_nodes, float* logprobs, const int32_t* target_idx, const float* mask,
                      float scale, float* GL, float* dwout, float* nll_sum, float* count, int32_t accumulate,
-                     void* workspace, const uint8_t* occ_HL, uint8_t* occ_GL, void* stream);
+                     void* workspace, const uint8_t* occ_HL, uint8_t* occ_GL, void* stream, const SconeLaunchHints* hints);
 // data-parallel exchange fused with Adam (scone_dp.cu)
 struct scone_dp;
 int scone_dp_allreduce_adam(scone_dp* d, float* W, float* m, float* v, float* grad, int64_t n_params, const int* overflow_dev,

@@ -1273,7 +1273,6 @@ __global__ void adam_kernel(float* __restrict__ W, float* __restrict__ m, float*
 }  // namespace
 
 bool g_scone_zero_fill = true;
-thread_local SconeLaunchHints g_scone_hints;
 
 namespace {
 
@@ -1355,23 +1354,23 @@ int compact_bitmap(const scone_complex* cx, int b, const uint32_t* bm, uint32_t*
 
 // Input worklist: the caller's hint (the previous launch's output worklist, same flags, same TT) or a fresh compaction.
 template <int TT>
-int input_worklist(const scone_complex* cx, int b, const uint8_t* occ_in, const UnitScratch& sc, cudaStream_t st, int* in) {
-    SconeLaunchHints& h = g_scone_hints;
-    if (h.in_wl >= 0 && h.in_tt == TT) {
-        *in = h.in_wl;
+int input_worklist(const scone_complex* cx, int b, const uint8_t* occ_in, const UnitScratch& sc, cudaStream_t st,
+                   const SconeLaunchHints* h, int* in) {
+    if (h && h->in_wl >= 0 && h->in_tt == TT) {
+        *in = h->in_wl;
         return 0;
     }
     *in = 0;
-    if (h.in_bm != nullptr && bitmap_ok(TT, b)) return compact_bitmap<TT>(cx, b, h.in_bm, sc.wl[0], sc.n[0], sc.tickets, st);
+    if (h && h->in_bm != nullptr && bitmap_ok(TT, b)) return compact_bitmap<TT>(cx, b, h->in_bm, sc.wl[0], sc.n[0], sc.tickets, st);
     return compact_units<TT>(cx, b, occ_in, sc.wl[0], sc.counts, sc.n[0], st);
 }
 
-// worklist(occ_in) -> one-hop scatter into occ_out -> worklist(occ_out); *out = index of that worklist in sc
+// worklist(occ_in) -> one-hop scatter into occ_out -> worklist(occ_out); *out = index of that worklist in sc (also h->out_wl)
 template <int TT>
 int prepare_units(const scone_complex* cx, int b, const uint8_t* occ_in, uint8_t* occ_out, const UnitScratch& sc, cudaStream_t st,
-                  int* out) {
+                  SconeLaunchHints* h, int* out) {
     int in = 0;
-    if (input_worklist<TT>(cx, b, occ_in, sc, st, &in)) return 1;
+    if (input_worklist<TT>(cx, b, occ_in, sc, st, h, &in)) return 1;
     SCONE_CUDA(cudaMemsetAsync(occ_out, 0, (size_t)cx->E * b, st));
     uint32_t* bm = bitmap_ok(TT, b) ? sc.bm : nullptr;
     if (bm) SCONE_CUDA(cudaMemsetAsync(bm, 0, scone_bitmap_words(cx->E, b) * 4, st));
@@ -1379,18 +1378,19 @@ int prepare_units(const scone_complex* cx, int b, const uint8_t* occ_in, uint8_t
                                                                      (b + TT - 1) / TT, b);
     SCONE_LAUNCHED();
     *out = 1 - in;
-    g_scone_hints.out_wl = *out;
-    g_scone_hints.out_tt = TT;
+    if (h) {
+        h->out_wl = *out;
+        h->out_tt = TT;
+    }
     if (bm) return compact_bitmap<TT>(cx, b, bm, sc.wl[*out], sc.n[*out], sc.tickets, st);
     return compact_units<TT>(cx, b, occ_out, sc.wl[*out], sc.counts, sc.n[*out], st);
 }
 
-bool zero_fill_here() { return g_scone_zero_fill && !g_scone_hints.skip_fill; }
-
+bool zero_fill_here(const SconeLaunchHints* h) { return g_scone_zero_fill && !(h && h->skip_fill); }
 
 template <int CIN, int COUT, int ACT>
 int launch_fwd(const scone_complex* cx, int b, const float* Hin, const float* W0, const float* W1, const float* W2, float* Hout,
-               const uint8_t* occ_in, uint8_t* occ_out, uint8_t* scratch, cudaStream_t st) {
+               const uint8_t* occ_in, uint8_t* occ_out, uint8_t* scratch, cudaStream_t st, SconeLaunchHints* h) {
     constexpr int TT = kTileCols / CIN, TE = kTileRows / TT, KD = 3 * CIN, LDT = KD + 4;
     ScopedProf prof(SCONE_K_LAYER_FWD, st);
     if (occ_in == nullptr) {                                  // dense path
@@ -1414,8 +1414,8 @@ int launch_fwd(const scone_complex* cx, int b, const float* Hin, const float* W0
     SCONE_REQUIRE(occ_out != nullptr && scratch != nullptr, "scone_layer_forward: occ_in needs occ_out and occ_scratch");
     const UnitScratch sc = carve_scratch(cx, b, scratch);
     int wo = 0;
-    if (prepare_units<TT>(cx, b, occ_in, occ_out, sc, st, &wo)) return 1;
-    if (zero_fill_here() && scone_zero_fill(cx, Hout, (size_t)cx->E * b * COUT * sizeof(float), st)) return 1;
+    if (prepare_units<TT>(cx, b, occ_in, occ_out, sc, st, h, &wo)) return 1;
+    if (zero_fill_here(h) && scone_zero_fill(cx, Hout, (size_t)cx->E * b * COUT * sizeof(float), st)) return 1;
     if (scone_slab_supported(cx, CIN, COUT) && bitmap_ok(TT, b)) {
         // candidate ROWS of the output (row bitmap of occ_out, still in the scratch) -> compacted list -> row-list kernel.  The
         // list goes where the consumed input worklist was; the output unit worklist (hint for the next call) stays intact.
@@ -1436,11 +1436,11 @@ int launch_fwd(const scone_complex* cx, int b, const float* Hin, const float* W0
 
 template <int CIN, int COUT>
 int dispatch_fwd_act(const scone_complex* cx, int act, int b, const float* Hin, const float* W0, const float* W1, const float* W2,
-                     float* Hout, const uint8_t* occ_in, uint8_t* occ_out, uint8_t* scratch, cudaStream_t st) {
+                     float* Hout, const uint8_t* occ_in, uint8_t* occ_out, uint8_t* scratch, cudaStream_t st, SconeLaunchHints* h) {
     switch (act) {
-        case SCONE_ACT_TANH: return launch_fwd<CIN, COUT, SCONE_ACT_TANH>(cx, b, Hin, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
-        case SCONE_ACT_LEAKY_RELU: return launch_fwd<CIN, COUT, SCONE_ACT_LEAKY_RELU>(cx, b, Hin, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
-        case SCONE_ACT_RELU: return launch_fwd<CIN, COUT, SCONE_ACT_RELU>(cx, b, Hin, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
+        case SCONE_ACT_TANH: return launch_fwd<CIN, COUT, SCONE_ACT_TANH>(cx, b, Hin, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, h);
+        case SCONE_ACT_LEAKY_RELU: return launch_fwd<CIN, COUT, SCONE_ACT_LEAKY_RELU>(cx, b, Hin, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, h);
+        case SCONE_ACT_RELU: return launch_fwd<CIN, COUT, SCONE_ACT_RELU>(cx, b, Hin, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, h);
     }
     scone_set_error("unknown activation %d", act);
     return 2;
@@ -1451,7 +1451,7 @@ constexpr int kBwdMaxCtas = 148 * 8;     // upper bound on persistent CTAs (work
 template <int CIN, int COUT, int ACT, bool WG>
 int launch_bwd(const scone_complex* cx, int b, const float* G, const float* Hin, const float* W0, const float* W1, const float* W2,
                float* Gprev, float* dW, int accumulate, float* ws, const uint8_t* occ_g, const uint8_t* occ_h, uint8_t* occ_prev,
-               uint8_t* scratch, cudaStream_t st) {
+               uint8_t* scratch, cudaStream_t st, SconeLaunchHints* h) {
     using Sh = BwdShape<CIN, COUT>;
     ScopedProf prof(SCONE_K_LAYER_BWD, st);
     int grid = 1;
@@ -1474,8 +1474,8 @@ int launch_bwd(const scone_complex* cx, int b, const float* G, const float* Hin,
         const UnitScratch sc = carve_scratch(cx, b, scratch);
         uint8_t* cand = WG ? occ_prev : sc.occ_tmp;           // rows whose (G, S0 G, S1 G) can be non-zero
         int wo = 0;
-        if (prepare_units<Us::TT>(cx, b, occ_g, cand, sc, st, &wo)) return 1;
-        if (WG && zero_fill_here() && scone_zero_fill(cx, Gprev, (size_t)cx->E * b * CIN * sizeof(float), st)) return 1;
+        if (prepare_units<Us::TT>(cx, b, occ_g, cand, sc, st, h, &wo)) return 1;
+        if (WG && zero_fill_here(h) && scone_zero_fill(cx, Gprev, (size_t)cx->E * b * CIN * sizeof(float), st)) return 1;
         const size_t smem = Us::smem_floats * sizeof(float);
         auto kern = layer_bwd_units_kernel<CIN, COUT, ACT, WG>;
         static int occ = 0;
@@ -1494,13 +1494,13 @@ int launch_bwd(const scone_complex* cx, int b, const float* G, const float* Hin,
 template <int CIN, int COUT>
 int dispatch_bwd_act(const scone_complex* cx, int act, int b, const float* G, const float* Hin, const float* W0, const float* W1,
                      const float* W2, float* Gprev, float* dW, int accumulate, float* ws, const uint8_t* occ_g, const uint8_t* occ_h,
-                     uint8_t* occ_prev, uint8_t* scratch, cudaStream_t st) {
+                     uint8_t* occ_prev, uint8_t* scratch, cudaStream_t st, SconeLaunchHints* h) {
 #define SCONE_BWD_CASE(A)                                                                                                          \
     case A:                                                                                                                        \
         return Gprev ? launch_bwd<CIN, COUT, A, true>(cx, b, G, Hin, W0, W1, W2, Gprev, dW, accumulate, ws, occ_g, occ_h, occ_prev, \
-                                                      scratch, st)                                                                 \
+                                                      scratch, st, h)                                                              \
                      : launch_bwd<CIN, COUT, A, false>(cx, b, G, Hin, W0, W1, W2, Gprev, dW, accumulate, ws, occ_g, occ_h, occ_prev, \
-                                                       scratch, st);
+                                                       scratch, st, h);
     switch (act) {
         SCONE_BWD_CASE(SCONE_ACT_TANH)
         SCONE_BWD_CASE(SCONE_ACT_LEAKY_RELU)
@@ -1569,18 +1569,6 @@ extern "C" int scone_get_zero_fill(void) { return g_scone_zero_fill ? 1 : 0; }
         }                                                                           \
     } while (0)
 
-// input hints are consumed by exactly one kernel-level call
-struct HintsReset {
-    ~HintsReset() {
-        g_scone_hints.in_wl = -1;
-        g_scone_hints.in_tt = 0;
-        g_scone_hints.skip_fill = false;
-        g_scone_hints.in_bm = nullptr;
-        g_scone_hints.out_bm = nullptr;
-        g_scone_hints.cand_bm = nullptr;
-    }
-};
-
 extern "C" int64_t scone_occ_scratch_bytes(const scone_complex* cx, int32_t b) {
     if (!cx || b <= 0) return 0;
     const size_t nu = max_units(cx, b);
@@ -1588,20 +1576,24 @@ extern "C" int64_t scone_occ_scratch_bytes(const scone_complex* cx, int32_t b) {
                      align256(kTicketSlots * 8) + align256((size_t)cx->E * b));
 }
 
-extern "C" int scone_layer_forward(const scone_complex* cx, int32_t act, int32_t b, int32_t cin, int32_t cout, const float* Hin,
-                                   const float* W0, const float* W1, const float* W2, float* Hout, const uint8_t* occ_in,
-                                   uint8_t* occ_out, uint8_t* occ_scratch, void* stream) {
-    HintsReset hints_guard;
-    g_scone_hints.out_wl = -1;
+int scone_layer_forward_hinted(const scone_complex* cx, int32_t act, int32_t b, int32_t cin, int32_t cout, const float* Hin,
+                               const float* W0, const float* W1, const float* W2, float* Hout, const uint8_t* occ_in,
+                               uint8_t* occ_out, uint8_t* occ_scratch, void* stream, SconeLaunchHints* hints) {
     SCONE_REQUIRE(cx && Hin && W0 && W1 && W2 && Hout, "scone_layer_forward: NULL argument");
     SCONE_REQUIRE(!cx->host_only, "scone_layer_forward: index-only complex has no device arrays");
     SCONE_REQUIRE(b > 0, "scone_layer_forward: b must be positive");
-    if (cin == 1) return scone_layer0_forward(cx, act, b, cout, Hin, W0, W1, W2, Hout, occ_in, occ_out, occ_scratch, stream);
+    if (cin == 1) return scone_layer0_forward(cx, act, b, cout, Hin, W0, W1, W2, Hout, occ_in, occ_out, occ_scratch, stream, hints);
     SCONE_REQUIRE(width_ok(cin) && width_ok(cout),
                   "scone_layer_forward: hidden widths must be in {8,16,32,64} with |log2 ratio| <= 1 (got %d -> %d)", cin, cout);
-    SCONE_DISPATCH_WIDTHS(dispatch_fwd_act, cx, act, b, Hin, W0, W1, W2, Hout, occ_in, occ_out, occ_scratch, as_stream(stream));
+    SCONE_DISPATCH_WIDTHS(dispatch_fwd_act, cx, act, b, Hin, W0, W1, W2, Hout, occ_in, occ_out, occ_scratch, as_stream(stream), hints);
     scone_set_error("scone_layer_forward: unsupported width pair %d -> %d", cin, cout);
     return 2;
+}
+
+extern "C" int scone_layer_forward(const scone_complex* cx, int32_t act, int32_t b, int32_t cin, int32_t cout, const float* Hin,
+                                   const float* W0, const float* W1, const float* W2, float* Hout, const uint8_t* occ_in,
+                                   uint8_t* occ_out, uint8_t* occ_scratch, void* stream) {
+    return scone_layer_forward_hinted(cx, act, b, cin, cout, Hin, W0, W1, W2, Hout, occ_in, occ_out, occ_scratch, stream, nullptr);
 }
 
 extern "C" int64_t scone_layer_backward_workspace_bytes(int32_t cin, int32_t cout) {
@@ -1609,16 +1601,14 @@ extern "C" int64_t scone_layer_backward_workspace_bytes(int32_t cin, int32_t cou
     return (int64_t)kBwdMaxCtas * 3 * cin * cout * sizeof(float);
 }
 
-extern "C" int scone_layer_backward(const scone_complex* cx, int32_t act, int32_t b, int32_t cin, int32_t cout, const float* G,
-                                    const float* Hin, const float* W0, const float* W1, const float* W2, float* Gprev, float* dW,
-                                    int32_t accumulate, void* workspace, const uint8_t* occ_g, const uint8_t* occ_hin,
-                                    uint8_t* occ_prev, uint8_t* occ_scratch, void* stream) {
-    HintsReset hints_guard;
-    g_scone_hints.out_wl = -1;
+int scone_layer_backward_hinted(const scone_complex* cx, int32_t act, int32_t b, int32_t cin, int32_t cout, const float* G,
+                                const float* Hin, const float* W0, const float* W1, const float* W2, float* Gprev, float* dW,
+                                int32_t accumulate, void* workspace, const uint8_t* occ_g, const uint8_t* occ_hin,
+                                uint8_t* occ_prev, uint8_t* occ_scratch, void* stream, SconeLaunchHints* hints) {
     SCONE_REQUIRE(cx && G && Hin && dW && workspace, "scone_layer_backward: NULL argument");
     SCONE_REQUIRE(!cx->host_only, "scone_layer_backward: index-only complex has no device arrays");
     SCONE_REQUIRE(b > 0, "scone_layer_backward: b must be positive");
-    if (cin == 1) return scone_layer0_backward(cx, b, cout, G, Hin, dW, accumulate, workspace, occ_g, occ_scratch, stream);
+    if (cin == 1) return scone_layer0_backward(cx, b, cout, G, Hin, dW, accumulate, workspace, occ_g, occ_scratch, stream, hints);
     SCONE_REQUIRE(W0 && W1 && W2, "scone_layer_backward: NULL weights");
     SCONE_REQUIRE(width_ok(cin) && width_ok(cout),
                   "scone_layer_backward: hidden widths must be in {8,16,32,64} with |log2 ratio| <= 1 (got %d -> %d)", cin, cout);
@@ -1628,14 +1618,23 @@ extern "C" int scone_layer_backward(const scone_complex* cx, int32_t act, int32_
         return scone_umma_backward(cx, act, b, G, Hin, W0, W1, W2, Gprev, dW, accumulate, (float*)workspace, as_stream(stream));
     }
     SCONE_DISPATCH_WIDTHS(dispatch_bwd_act, cx, act, b, G, Hin, W0, W1, W2, Gprev, dW, accumulate, (float*)workspace, occ_g, occ_hin,
-                          occ_prev, occ_scratch, as_stream(stream));
+                          occ_prev, occ_scratch, as_stream(stream), hints);
     scone_set_error("scone_layer_backward: unsupported width pair %d -> %d", cin, cout);
     return 2;
 }
 
+extern "C" int scone_layer_backward(const scone_complex* cx, int32_t act, int32_t b, int32_t cin, int32_t cout, const float* G,
+                                    const float* Hin, const float* W0, const float* W1, const float* W2, float* Gprev, float* dW,
+                                    int32_t accumulate, void* workspace, const uint8_t* occ_g, const uint8_t* occ_hin,
+                                    uint8_t* occ_prev, uint8_t* occ_scratch, void* stream) {
+    return scone_layer_backward_hinted(cx, act, b, cin, cout, G, Hin, W0, W1, W2, Gprev, dW, accumulate, workspace, occ_g, occ_hin,
+                                       occ_prev, occ_scratch, stream, nullptr);
+}
+
 template <int COUT, int ACT>
 static int launch_l0_fwd_act(const scone_complex* cx, int b, const float* X, const float* W0, const float* W1, const float* W2,
-                             float* Hout, const uint8_t* occ_in, uint8_t* occ_out, uint8_t* scratch, cudaStream_t st) {
+                             float* Hout, const uint8_t* occ_in, uint8_t* occ_out, uint8_t* scratch, cudaStream_t st,
+                             SconeLaunchHints* h) {
     ScopedProf prof(SCONE_K_LAYER0_FWD, st);
     if (occ_in == nullptr) {               // dense: every row is computed; flags (if wanted) are value based
         const long long n_tiles = (long long)((b + 31) / 32) * ((cx->E + kL0Edges - 1) / kL0Edges);
@@ -1648,8 +1647,8 @@ static int launch_l0_fwd_act(const scone_complex* cx, int b, const float* X, con
     constexpr int TT = kTileCols / COUT;
     const UnitScratch sc = carve_scratch(cx, b, scratch);
     int wo = 0;
-    if (prepare_units<TT>(cx, b, occ_in, occ_out, sc, st, &wo)) return 1;
-    if (zero_fill_here() && scone_zero_fill(cx, Hout, (size_t)cx->E * b * COUT * sizeof(float), st)) return 1;
+    if (prepare_units<TT>(cx, b, occ_in, occ_out, sc, st, h, &wo)) return 1;
+    if (zero_fill_here(h) && scone_zero_fill(cx, Hout, (size_t)cx->E * b * COUT * sizeof(float), st)) return 1;
     layer0_fwd_units_kernel<COUT, ACT><<<cx->num_sms * 8, kThreads, 0, st>>>(X, Hout, W0, W1, W2, cx->S(0), cx->S(1), cx->E, b, occ_out,
                                                                             sc.wl[wo], sc.n[wo]);
     SCONE_LAUNCHED();
@@ -1658,11 +1657,11 @@ static int launch_l0_fwd_act(const scone_complex* cx, int b, const float* X, con
 
 template <int COUT>
 static int launch_l0_fwd(const scone_complex* cx, int act, int b, const float* X, const float* W0, const float* W1, const float* W2,
-                         float* Hout, const uint8_t* occ_in, uint8_t* occ_out, uint8_t* scratch, cudaStream_t st) {
+                         float* Hout, const uint8_t* occ_in, uint8_t* occ_out, uint8_t* scratch, cudaStream_t st, SconeLaunchHints* h) {
     switch (act) {
-        case SCONE_ACT_TANH: return launch_l0_fwd_act<COUT, SCONE_ACT_TANH>(cx, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
-        case SCONE_ACT_LEAKY_RELU: return launch_l0_fwd_act<COUT, SCONE_ACT_LEAKY_RELU>(cx, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
-        case SCONE_ACT_RELU: return launch_l0_fwd_act<COUT, SCONE_ACT_RELU>(cx, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
+        case SCONE_ACT_TANH: return launch_l0_fwd_act<COUT, SCONE_ACT_TANH>(cx, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, h);
+        case SCONE_ACT_LEAKY_RELU: return launch_l0_fwd_act<COUT, SCONE_ACT_LEAKY_RELU>(cx, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, h);
+        case SCONE_ACT_RELU: return launch_l0_fwd_act<COUT, SCONE_ACT_RELU>(cx, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, h);
     }
     scone_set_error("unknown activation %d", act);
     return 2;
@@ -1670,13 +1669,13 @@ static int launch_l0_fwd(const scone_complex* cx, int act, int b, const float* X
 
 int scone_layer0_forward(const scone_complex* cx, int32_t act, int32_t b, int32_t cout, const float* X, const float* W0,
                          const float* W1, const float* W2, float* Hout, const uint8_t* occ_in, uint8_t* occ_out, uint8_t* scratch,
-                         void* stream) {
+                         void* stream, SconeLaunchHints* hints) {
     cudaStream_t st = as_stream(stream);
     switch (cout) {
-        case 8: return launch_l0_fwd<8>(cx, act, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
-        case 16: return launch_l0_fwd<16>(cx, act, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
-        case 32: return launch_l0_fwd<32>(cx, act, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
-        case 64: return launch_l0_fwd<64>(cx, act, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st);
+        case 8: return launch_l0_fwd<8>(cx, act, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, hints);
+        case 16: return launch_l0_fwd<16>(cx, act, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, hints);
+        case 32: return launch_l0_fwd<32>(cx, act, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, hints);
+        case 64: return launch_l0_fwd<64>(cx, act, b, X, W0, W1, W2, Hout, occ_in, occ_out, scratch, st, hints);
     }
     scone_set_error("scone_layer_forward: first-layer width must be in {8,16,32,64} (got %d)", cout);
     return 2;
@@ -1687,7 +1686,7 @@ int64_t scone_layer0_backward_workspace_bytes(int32_t cout) { return (int64_t)kL
 
 template <int COUT>
 static int launch_l0_bwd(const scone_complex* cx, int b, const float* G, const float* X, float* dW, int accumulate, float* ws,
-                         const uint8_t* occ_g, uint8_t* scratch, cudaStream_t st) {
+                         const uint8_t* occ_g, uint8_t* scratch, cudaStream_t st, const SconeLaunchHints* h) {
     ScopedProf prof(SCONE_K_LAYER0_BWD, st);
     int grid;
     if (occ_g == nullptr) {
@@ -1700,7 +1699,7 @@ static int launch_l0_bwd(const scone_complex* cx, int b, const float* G, const f
         constexpr int TT = kTileCols / COUT;
         const UnitScratch sc = carve_scratch(cx, b, scratch);
         int wi = 0;
-        if (input_worklist<TT>(cx, b, occ_g, sc, st, &wi)) return 1;
+        if (input_worklist<TT>(cx, b, occ_g, sc, st, h, &wi)) return 1;
         grid = cx->num_sms * 4;
         if (grid > kL0BwdCtas) grid = kL0BwdCtas;
         layer0_bwd_units_kernel<COUT><<<grid, kThreads, 0, st>>>(X, G, ws, cx->S(0), cx->S(1), cx->E, b, occ_g, sc.wl[wi], sc.n[wi]);
@@ -1712,33 +1711,38 @@ static int launch_l0_bwd(const scone_complex* cx, int b, const float* G, const f
 }
 
 int scone_layer0_backward(const scone_complex* cx, int32_t b, int32_t cout, const float* G, const float* X, float* dW,
-                          int32_t accumulate, void* workspace, const uint8_t* occ_g, uint8_t* scratch, void* stream) {
+                          int32_t accumulate, void* workspace, const uint8_t* occ_g, uint8_t* scratch, void* stream,
+                          const SconeLaunchHints* hints) {
     cudaStream_t st = as_stream(stream);
     float* ws = (float*)workspace;
     switch (cout) {
-        case 8: return launch_l0_bwd<8>(cx, b, G, X, dW, accumulate, ws, occ_g, scratch, st);
-        case 16: return launch_l0_bwd<16>(cx, b, G, X, dW, accumulate, ws, occ_g, scratch, st);
-        case 32: return launch_l0_bwd<32>(cx, b, G, X, dW, accumulate, ws, occ_g, scratch, st);
-        case 64: return launch_l0_bwd<64>(cx, b, G, X, dW, accumulate, ws, occ_g, scratch, st);
+        case 8: return launch_l0_bwd<8>(cx, b, G, X, dW, accumulate, ws, occ_g, scratch, st, hints);
+        case 16: return launch_l0_bwd<16>(cx, b, G, X, dW, accumulate, ws, occ_g, scratch, st, hints);
+        case 32: return launch_l0_bwd<32>(cx, b, G, X, dW, accumulate, ws, occ_g, scratch, st, hints);
+        case 64: return launch_l0_bwd<64>(cx, b, G, X, dW, accumulate, ws, occ_g, scratch, st, hints);
     }
     scone_set_error("scone_layer_backward: first-layer width must be in {8,16,32,64} (got %d)", cout);
     return 2;
 }
 
-extern "C" int scone_flows_to_dense(const scone_complex* cx, int32_t b, const int32_t* traj_ptr, const int32_t* flow_edge,
-                                    const float* flow_val, float* X, uint8_t* occX, void* stream) {
+int scone_flows_to_dense_hinted(const scone_complex* cx, int32_t b, const int32_t* traj_ptr, const int32_t* flow_edge,
+                                const float* flow_val, float* X, uint8_t* occX, void* stream, const SconeLaunchHints* hints) {
     SCONE_REQUIRE(cx && traj_ptr && X && b > 0, "scone_flows_to_dense: bad argument");
     SCONE_REQUIRE(!cx->host_only, "scone_flows_to_dense: index-only complex has no device arrays");
     cudaStream_t st = as_stream(stream);
     ScopedProf prof(SCONE_K_OTHER, st);
     SCONE_CUDA(cudaMemsetAsync(X, 0, (size_t)cx->E * b * sizeof(float), st));
     if (occX) SCONE_CUDA(cudaMemsetAsync(occX, 0, (size_t)cx->E * b, st));
-    uint32_t* bm = (occX != nullptr && b % 4 == 0) ? g_scone_hints.out_bm : nullptr;
-    g_scone_hints.out_bm = nullptr;
+    uint32_t* bm = (hints && occX != nullptr && b % 4 == 0) ? hints->out_bm : nullptr;
     if (bm) SCONE_CUDA(cudaMemsetAsync(bm, 0, scone_bitmap_words(cx->E, b) * 4, st));
     flows_to_dense_kernel<<<(b * 32 + 255) / 256, 256, 0, st>>>(traj_ptr, flow_edge, flow_val, cx->d_rank, X, occX, bm, cx->E, b);
     SCONE_LAUNCHED();
     return 0;
+}
+
+extern "C" int scone_flows_to_dense(const scone_complex* cx, int32_t b, const int32_t* traj_ptr, const int32_t* flow_edge,
+                                    const float* flow_val, float* X, uint8_t* occX, void* stream) {
+    return scone_flows_to_dense_hinted(cx, b, traj_ptr, flow_edge, flow_val, X, occX, stream, nullptr);
 }
 
 int64_t scone_readout_workspace_bytes(int32_t b, int32_t C) { return (int64_t)b * (C + 2) * sizeof(float); }
@@ -1746,27 +1750,24 @@ int64_t scone_readout_workspace_bytes(int32_t b, int32_t C) { return (int64_t)b 
 int scone_readout_ws(const scone_complex* cx, int32_t act, int32_t b, int32_t C, const float* HL, const float* wout,
                      const int32_t* last_nodes, float* logprobs, const int32_t* target_idx, const float* mask, float scale,
                      float* GL, float* dwout, float* nll_sum, float* count, int32_t accumulate, void* workspace,
-                     const uint8_t* occ_HL, uint8_t* occ_GL, void* stream) {
-    HintsReset hints_guard;
-    g_scone_hints.out_wl = -1;
+                     const uint8_t* occ_HL, uint8_t* occ_GL, void* stream, const SconeLaunchHints* hints) {
     SCONE_REQUIRE(cx && HL && wout && last_nodes && logprobs, "scone_readout: NULL argument");
     SCONE_REQUIRE(!cx->host_only, "scone_readout: index-only complex has no device arrays");
     SCONE_REQUIRE(C >= 1 && C <= 32 * kReadoutMaxCper, "scone_readout: C must be in [1,%d]", 32 * kReadoutMaxCper);
     SCONE_REQUIRE(cx->D <= kReadoutMaxD, "scone_readout: max degree %d exceeds %d", cx->D, kReadoutMaxD);
     cudaStream_t st = as_stream(stream);
     ScopedProf prof(SCONE_K_READOUT, st);
+    const SconeLaunchHints h = hints ? *hints : SconeLaunchHints{};
     if (GL) {
         SCONE_REQUIRE(target_idx && mask && workspace, "scone_readout: gradient mode needs target_idx, mask, workspace");
         // without flags the consumer reads every row of GL: it must be dense zeros; with flags only when zero-fill is on
-        const bool flagged = occ_GL != nullptr || g_scone_hints.out_bm != nullptr;
-        if ((!flagged || zero_fill_here()) && scone_zero_fill(cx, GL, (size_t)cx->E * b * C * sizeof(float), st)) return 1;
+        const bool flagged = occ_GL != nullptr || h.out_bm != nullptr;
+        if ((!flagged || zero_fill_here(&h)) && scone_zero_fill(cx, GL, (size_t)cx->E * b * C * sizeof(float), st)) return 1;
         if (occ_GL) SCONE_CUDA(cudaMemsetAsync(occ_GL, 0, (size_t)cx->E * b, st));
     }
-    const uint32_t* bm_HL = g_scone_hints.in_bm;           // row-bitmap pipeline: bits instead of flag bytes
-    uint32_t* bm_cand = GL ? g_scone_hints.cand_bm : nullptr;
-    uint32_t* bm = (GL && (occ_GL || bm_HL)) ? g_scone_hints.out_bm : nullptr;
-    g_scone_hints.out_bm = nullptr;
-    g_scone_hints.cand_bm = nullptr;
+    const uint32_t* bm_HL = h.in_bm;                       // row-bitmap pipeline: bits instead of flag bytes
+    uint32_t* bm_cand = GL ? h.cand_bm : nullptr;
+    uint32_t* bm = (GL && (occ_GL || bm_HL)) ? h.out_bm : nullptr;
     if (bm) SCONE_CUDA(cudaMemsetAsync(bm, 0, scone_bitmap_words(cx->E, b) * 4, st));
     if (bm_cand) SCONE_CUDA(cudaMemsetAsync(bm_cand, 0, scone_bitmap_words(cx->E, b) * 4, st));
     readout_kernel<<<b, 32 * kReadoutWarps, 0, st>>>(HL, wout, last_nodes, cx->d_nbrhoods, cx->d_inc_ptr, cx->d_inc_ent, logprobs,
@@ -1787,7 +1788,7 @@ extern "C" int scone_readout(const scone_complex* cx, int32_t act, int32_t b, in
                              float* GL, float* dwout, float* nll_sum, float* count, int32_t accumulate, void* workspace,
                              const uint8_t* occ_HL, uint8_t* occ_GL, void* stream) {
     return scone_readout_ws(cx, act, b, C, HL, wout, last_nodes, logprobs, target_idx, mask, scale, GL, dwout, nll_sum, count,
-                            accumulate, workspace, occ_HL, occ_GL, stream);
+                            accumulate, workspace, occ_HL, occ_GL, stream, nullptr);
 }
 
 int scone_adam_launch(float* W, float* m, float* v, const float* gradbuf, int64_t n, int32_t step, float lr, float wd, void* stream,

@@ -97,6 +97,41 @@ int ensure_staging(scone_model* m, int64_t B, int64_t nnz) {
     return 0;
 }
 
+// Stages the HOST inputs of a *_host entry point on s: ptr [B+1] always; last / n_nbrs / tgt / mask [B] when B > 0 and given; the
+// flow arrays edge / val [ptr[B]] when `flows` (the overlapped fused path copies them itself, on its copy stream).
+int stage_host_inputs(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* last, const int32_t* n_nbrs, const int32_t* tgt,
+                      const float* mask, const int32_t* edge, const float* val, bool flows, cudaStream_t s) {
+    const int64_t nnz = B > 0 ? ptr[B] : 0;
+    if (ensure_staging(m, B, nnz)) return 1;
+    SCONE_CUDA(cudaMemcpyAsync(m->d_ptr, ptr, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    if (B > 0) {
+        if (last) SCONE_CUDA(cudaMemcpyAsync(m->d_last, last, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        if (n_nbrs) SCONE_CUDA(cudaMemcpyAsync(m->d_nn, n_nbrs, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        if (tgt) SCONE_CUDA(cudaMemcpyAsync(m->d_tgt, tgt, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        if (mask) SCONE_CUDA(cudaMemcpyAsync(m->d_mask, mask, B * sizeof(float), cudaMemcpyHostToDevice, s));
+    }
+    if (flows && nnz > 0) {
+        SCONE_CUDA(cudaMemcpyAsync(m->d_edge, edge, nnz * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        SCONE_CUDA(cudaMemcpyAsync(m->d_val, val, nnz * sizeof(float), cudaMemcpyHostToDevice, s));
+    }
+    return 0;
+}
+
+// Reports a row-list capacity overflow of the work enqueued on s so far (error code 4): copies the device flag, synchronises s and,
+// if it is set, clears it.  `what` names the entry point.
+int report_overflow(scone_model* m, cudaStream_t s, const char* what) {
+    int overflow = 0;
+    if (m->d_overflow) SCONE_CUDA(cudaMemcpyAsync(&overflow, m->d_overflow, sizeof(int), cudaMemcpyDeviceToHost, s));
+    SCONE_CUDA(cudaStreamSynchronize(s));
+    if (!overflow) return 0;
+    cudaMemset(m->d_overflow, 0, sizeof(int));
+    m->cone_clean = false;                                 // a truncated cone list: the clearing may have missed bits
+    scone_set_error("%s: a micro-batch exceeded a row-list capacity (%d rows per compact tensor, %d rows of the backward's A buffer, 2048 "
+                    "cone edges per trajectory and layer); results since the last check are incomplete and any Adam step since then was "
+                    "skipped — use a smaller micro-batch or another pipeline (scone_model_set_pipeline)", what, m->row_cap, m->a_cap);
+    return 4;
+}
+
 // Zero-fill of this micro-batch's dense tensors on the side stream (they are only written, never read, before their
 // consumer kernel runs): the fills overlap the small flag / unit kernels of the main stream.
 int start_fills(scone_model* m, int32_t b, bool with_grads, cudaStream_t s) {
@@ -115,8 +150,9 @@ int start_fills(scone_model* m, int32_t b, bool with_grads, cudaStream_t s) {
         }
     return 0;
 }
+// Orders s after the side-stream fill of tensor idx.  The kernel-level call that writes the tensor then gets skip_fill: either the
+// side stream filled it, or nobody does.
 int wait_fill(scone_model* m, int idx, cudaStream_t s) {
-    g_scone_hints.skip_fill = true;          // the kernel-level call never fills: either the side stream did, or nobody does
     if (!m->zero_fill) return 0;
     SCONE_CUDA(cudaStreamWaitEvent(s, m->ev_fill[idx], 0));
     return 0;
@@ -125,22 +161,26 @@ int wait_fill(scone_model* m, int idx, cudaStream_t s) {
 // forward over one micro-batch [off, off+b): X -> H_1 .. H_L (kept) ; returns 0 on success
 int forward_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, void* st) {
     const scone_complex* cx = m->cx;
-    g_scone_hints.out_bm = m->d_bmX;
-    int rc = scone_flows_to_dense(cx, b, ptr, edge, val, m->d_X, m->d_occX, st);
+    SconeLaunchHints xh;
+    xh.out_bm = m->d_bmX;
+    int rc = scone_flows_to_dense_hinted(cx, b, ptr, edge, val, m->d_X, m->d_occX, st, &xh);
     if (rc) return rc;
     const float* in = m->d_X;
     int cin = 1, wl = -1, tt = 0;
     for (int l = 0; l < m->L; ++l) {
         const int cout = m->hidden[l];
         if (wait_fill(m, l, as_stream(st))) return 1;
-        g_scone_hints.in_wl = wl;
-        g_scone_hints.in_tt = tt;
-        if (l == 0) g_scone_hints.in_bm = m->d_bmX;
-        rc = scone_layer_forward(cx, m->act, b, cin, cout, in, m->d_w + m->w_off[3 * l], m->d_w + m->w_off[3 * l + 1],
-                                 m->d_w + m->w_off[3 * l + 2], m->d_H[l], l > 0 ? m->d_occH[l - 1] : m->d_occX, m->d_occH[l], m->d_occS, st);
+        SconeLaunchHints h;                  // the previous layer's output worklist; layer 0 compacts from the bitmap of X
+        h.in_wl = wl;
+        h.in_tt = tt;
+        h.skip_fill = true;
+        if (l == 0) h.in_bm = m->d_bmX;
+        rc = scone_layer_forward_hinted(cx, m->act, b, cin, cout, in, m->d_w + m->w_off[3 * l], m->d_w + m->w_off[3 * l + 1],
+                                        m->d_w + m->w_off[3 * l + 2], m->d_H[l], l > 0 ? m->d_occH[l - 1] : m->d_occX, m->d_occH[l],
+                                        m->d_occS, st, &h);
         if (rc) return rc;
-        wl = g_scone_hints.out_wl;
-        tt = g_scone_hints.out_tt;
+        wl = h.out_wl;
+        tt = h.out_tt;
         in = m->d_H[l];
         cin = cout;
     }
@@ -296,17 +336,18 @@ int rows_readout(scone_model* m, int32_t b, const int32_t* last, float* logprobs
     const float* wout = m->d_w + m->w_off[3 * L];
     ScopedProf prof(SCONE_K_READOUT, s);
     if (m->pipeline == 1) {
-        g_scone_hints.skip_fill = true;
-        g_scone_hints.in_bm = m->d_bmH[L - 1];
+        SconeLaunchHints h;                  // row bitmaps instead of flag bytes; G_L is read only at the rows its bitmap marks: no fill
+        h.skip_fill = true;
+        h.in_bm = m->d_bmH[L - 1];
         if (grad) {
-            g_scone_hints.out_bm = m->d_bmGr[L - 1];
-            g_scone_hints.cand_bm = L >= 2 ? m->d_bmGr[L - 2] : nullptr;
+            h.out_bm = m->d_bmGr[L - 1];
+            h.cand_bm = L >= 2 ? m->d_bmGr[L - 2] : nullptr;
             return scone_readout_ws(cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, tgt, mask, 1.f, m->d_G[L - 1],
                                     m->d_grad + m->w_off[3 * L], m->d_grad + m->n_params, m->d_grad + m->n_params + 1, 1, m->d_ws, nullptr,
-                                    nullptr, s);
+                                    nullptr, s, &h);
         }
         return scone_readout_ws(cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, nullptr, nullptr, 0.f, nullptr, nullptr, nullptr,
-                                nullptr, 0, nullptr, nullptr, nullptr, s);
+                                nullptr, 0, nullptr, nullptr, nullptr, s, &h);
     }
     const size_t bm_bytes = scone_bitmap_words(cx->E, b) * 4;
     uint32_t *bmG = nullptr, *cand = nullptr;
@@ -786,7 +827,7 @@ extern "C" int scone_model_forward_dev(scone_model* m, int32_t B, const int32_t*
         if (!rc)
             rc = scone_readout_ws(cx, m->act, b, m->hidden[m->L - 1], m->d_H[m->L - 1], m->d_w + m->w_off[3 * m->L], last + off,
                                   logprobs + (size_t)off * cx->D, nullptr, nullptr, 0.f, nullptr, nullptr, nullptr, nullptr, 0,
-                                  nullptr, m->d_occH[m->L - 1], nullptr, st);
+                                  nullptr, m->d_occH[m->L - 1], nullptr, st, nullptr);
     }
     return finish_call(m, rc, user_st);
 }
@@ -828,10 +869,12 @@ extern "C" int scone_model_loss_grad_dev(scone_model* m, int32_t B, const int32_
         const int CL = m->hidden[L - 1];
         if (!rc && wait_fill(m, L + (L - 1), s)) rc = 1;
         if (rc) break;
-        g_scone_hints.out_bm = m->d_bmG;
+        SconeLaunchHints rh;                 // G_L: filled on the side stream (or nobody does); its flags also go to the bitmap d_bmG
+        rh.skip_fill = true;
+        rh.out_bm = m->d_bmG;
         rc = scone_readout_ws(cx, m->act, b, CL, m->d_H[L - 1], m->d_w + m->w_off[3 * L], last + off, m->d_logp, tgt + off,
                               mask + off, 1.f, m->d_G[L - 1], m->d_grad + m->w_off[3 * L], m->d_grad + m->n_params,
-                              m->d_grad + m->n_params + 1, 1, m->d_ws, m->d_occH[L - 1], m->d_occG[L - 1], st);
+                              m->d_grad + m->n_params + 1, 1, m->d_ws, m->d_occH[L - 1], m->d_occG[L - 1], st, &rh);
         int wl = -1, tt = 0;
         for (int l = L - 1; l >= 0 && !rc; --l) {
             const int cout = m->hidden[l], cin = l > 0 ? m->hidden[l - 1] : 1;
@@ -840,15 +883,17 @@ extern "C" int scone_model_loss_grad_dev(scone_model* m, int32_t B, const int32_
                 rc = 1;
                 break;
             }
-            g_scone_hints.in_wl = wl;
-            g_scone_hints.in_tt = tt;
-            if (l == L - 1) g_scone_hints.in_bm = m->d_bmG;
-            rc = scone_layer_backward(cx, m->act, b, cin, cout, m->d_G[l], Hin, m->d_w + m->w_off[3 * l],
-                                      m->d_w + m->w_off[3 * l + 1], m->d_w + m->w_off[3 * l + 2], l > 0 ? m->d_G[l - 1] : nullptr,
-                                      m->d_grad + m->w_off[3 * l], 1, m->d_ws, m->d_occG[l], l > 0 ? m->d_occH[l - 1] : nullptr,
-                                      l > 0 ? m->d_occG[l - 1] : nullptr, m->d_occS, st);
-            wl = g_scone_hints.out_wl;
-            tt = g_scone_hints.out_tt;
+            SconeLaunchHints h;              // the previous layer's output worklist; layer L - 1 compacts from the bitmap of G_L
+            h.in_wl = wl;
+            h.in_tt = tt;
+            h.skip_fill = l > 0;             // G_{l-1}: filled on the side stream (or nobody does); layer 0 writes no G_{l-1}
+            if (l == L - 1) h.in_bm = m->d_bmG;
+            rc = scone_layer_backward_hinted(cx, m->act, b, cin, cout, m->d_G[l], Hin, m->d_w + m->w_off[3 * l],
+                                             m->d_w + m->w_off[3 * l + 1], m->d_w + m->w_off[3 * l + 2], l > 0 ? m->d_G[l - 1] : nullptr,
+                                             m->d_grad + m->w_off[3 * l], 1, m->d_ws, m->d_occG[l], l > 0 ? m->d_occH[l - 1] : nullptr,
+                                             l > 0 ? m->d_occG[l - 1] : nullptr, m->d_occS, st, &h);
+            wl = h.out_wl;
+            tt = h.out_tt;
         }
     }
     return finish_call(m, rc, user_st);
@@ -859,32 +904,14 @@ extern "C" int scone_model_forward_host(scone_model* m, int32_t B, const int32_t
     SCONE_REQUIRE(m && ptr && last && logprobs_out && B >= 0, "scone_model_forward_host: bad arguments");
     if (B == 0) return 0;
     cudaStream_t s = as_stream(st);
-    const int64_t nnz = ptr[B];
-    int rc = ensure_staging(m, B, nnz);
+    const bool overlap = fused_host_overlap_ok(m, B, ptr[B]);
+    int rc = stage_host_inputs(m, B, ptr, last, nullptr, nullptr, nullptr, edge, val, !overlap, s);
     if (rc) return rc;
-    SCONE_CUDA(cudaMemcpyAsync(m->d_ptr, ptr, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    SCONE_CUDA(cudaMemcpyAsync(m->d_last, last, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    if (fused_host_overlap_ok(m, B, nnz)) {
-        rc = fused_host_overlapped(m, B, ptr, edge, val, m->d_logp_all, false, 0, s);
-    } else {
-        SCONE_CUDA(cudaMemcpyAsync(m->d_edge, edge, nnz * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-        SCONE_CUDA(cudaMemcpyAsync(m->d_val, val, nnz * sizeof(float), cudaMemcpyHostToDevice, s));
-        rc = scone_model_forward_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, m->d_logp_all, st);
-    }
+    if (overlap) rc = fused_host_overlapped(m, B, ptr, edge, val, m->d_logp_all, false, 0, s);
+    else rc = scone_model_forward_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, m->d_logp_all, st);
     if (rc) return rc;
     SCONE_CUDA(cudaMemcpyAsync(logprobs_out, m->d_logp_all, (size_t)B * m->cx->D * sizeof(float), cudaMemcpyDeviceToHost, s));
-    int overflow = 0;
-    if (m->d_overflow) SCONE_CUDA(cudaMemcpyAsync(&overflow, m->d_overflow, sizeof(int), cudaMemcpyDeviceToHost, s));
-    SCONE_CUDA(cudaStreamSynchronize(s));
-    if (overflow) {
-        cudaMemset(m->d_overflow, 0, sizeof(int));
-        m->cone_clean = false;                             // a truncated cone list: the clearing may have missed bits
-        scone_set_error("scone_model: a micro-batch exceeded a row-list capacity (%d rows per compact tensor, %d cone edges per trajectory "
-                        "and layer); the log-probs are incomplete — use a smaller micro-batch or scone_model_set_pipeline(m, 2 / 0)",
-                        m->row_cap, 2048);
-        return 4;
-    }
-    return 0;
+    return report_overflow(m, s, "scone_model_forward_host");
 }
 
 extern "C" int scone_accuracy_dev(int32_t B, int32_t D, const float* logprobs, const int32_t* n_nbrs, const int32_t* target_idx,
@@ -900,34 +927,14 @@ extern "C" int scone_model_accuracy_host(scone_model* m, int32_t B, const int32_
     out_host[0] = out_host[1] = 0;
     if (B == 0) return 0;
     cudaStream_t s = as_stream(st);
-    const int64_t nnz = ptr[B];
-    int rc = ensure_staging(m, B, nnz);
+    int rc = stage_host_inputs(m, B, ptr, last, n_nbrs, tgt, mask, edge, val, true, s);
     if (rc) return rc;
-    SCONE_CUDA(cudaMemcpyAsync(m->d_ptr, ptr, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    if (nnz) {
-        SCONE_CUDA(cudaMemcpyAsync(m->d_edge, edge, nnz * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-        SCONE_CUDA(cudaMemcpyAsync(m->d_val, val, nnz * sizeof(float), cudaMemcpyHostToDevice, s));
-    }
-    SCONE_CUDA(cudaMemcpyAsync(m->d_last, last, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    SCONE_CUDA(cudaMemcpyAsync(m->d_nn, n_nbrs, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    SCONE_CUDA(cudaMemcpyAsync(m->d_tgt, tgt, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    SCONE_CUDA(cudaMemcpyAsync(m->d_mask, mask, B * sizeof(float), cudaMemcpyHostToDevice, s));
     rc = scone_model_forward_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, m->d_logp_all, st);
     if (rc) return rc;
     rc = scone_accuracy_launch(B, m->cx->D, m->d_logp_all, m->d_nn, m->d_tgt, m->d_mask, m->d_acc, s);
     if (rc) return rc;
     SCONE_CUDA(cudaMemcpyAsync(out_host, m->d_acc, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    int overflow = 0;
-    if (m->d_overflow) SCONE_CUDA(cudaMemcpyAsync(&overflow, m->d_overflow, sizeof(int), cudaMemcpyDeviceToHost, s));
-    SCONE_CUDA(cudaStreamSynchronize(s));
-    if (overflow) {
-        cudaMemset(m->d_overflow, 0, sizeof(int));
-        m->cone_clean = false;
-        scone_set_error("scone_model: a micro-batch exceeded a row-list capacity; the accuracy is incomplete — use a smaller micro-batch or "
-                        "scone_model_set_pipeline(m, 2 / 0)");
-        return 4;
-    }
-    return 0;
+    return report_overflow(m, s, "scone_model_accuracy_host");
 }
 
 // ---- evaluation without the log-probs leaving the device (scone_trajectory_model.py:42-56, 59-71, 73-108) --------------------
@@ -948,8 +955,7 @@ extern "C" int scone_model_eval_host(scone_model* m, int32_t B, const int32_t* p
     m->eval_B = 0;
     if (B == 0) return 0;
     cudaStream_t s = as_stream(st);
-    const int64_t nnz = ptr[B];
-    int rc = ensure_staging(m, B, nnz);
+    int rc = stage_host_inputs(m, B, ptr, last, n_nbrs, tgt, mask, edge, val, true, s);
     if (rc) return rc;
     if (!m->d_choice || m->cap_choice < B) {
         cudaFree(m->d_choice); cudaFree(m->d_rand);
@@ -959,15 +965,6 @@ extern "C" int scone_model_eval_host(scone_model* m, int32_t B, const int32_t* p
         m->cap_choice = m->cap_B;
     }
     if (!m->d_evalf) SCONE_CUDA(cudaMalloc((void**)&m->d_evalf, 4 * sizeof(float)));
-    SCONE_CUDA(cudaMemcpyAsync(m->d_ptr, ptr, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    if (nnz) {
-        SCONE_CUDA(cudaMemcpyAsync(m->d_edge, edge, nnz * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-        SCONE_CUDA(cudaMemcpyAsync(m->d_val, val, nnz * sizeof(float), cudaMemcpyHostToDevice, s));
-    }
-    SCONE_CUDA(cudaMemcpyAsync(m->d_last, last, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    if (n_nbrs) SCONE_CUDA(cudaMemcpyAsync(m->d_nn, n_nbrs, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    if (tgt) SCONE_CUDA(cudaMemcpyAsync(m->d_tgt, tgt, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    if (mask) SCONE_CUDA(cudaMemcpyAsync(m->d_mask, mask, B * sizeof(float), cudaMemcpyHostToDevice, s));
     rc = scone_model_forward_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, m->d_logp_all, st);
     if (rc) return rc;
     const int D = m->cx->D;
@@ -983,16 +980,8 @@ extern "C" int scone_model_eval_host(scone_model* m, int32_t B, const int32_t* p
         if (scone_nll_launch(B, D, m->d_logp_all, m->d_tgt, m->d_mask, m->d_evalf, s)) return 1;
         SCONE_CUDA(cudaMemcpyAsync(nll_out, m->d_evalf, 2 * sizeof(float), cudaMemcpyDeviceToHost, s));
     }
-    int overflow = 0;
-    if (m->d_overflow) SCONE_CUDA(cudaMemcpyAsync(&overflow, m->d_overflow, sizeof(int), cudaMemcpyDeviceToHost, s));
-    SCONE_CUDA(cudaStreamSynchronize(s));
-    if (overflow) {
-        cudaMemset(m->d_overflow, 0, sizeof(int));
-        m->cone_clean = false;
-        scone_set_error("scone_model: a micro-batch exceeded a row-list capacity; the evaluation is incomplete — use a smaller micro-batch or "
-                        "another pipeline");
-        return 4;
-    }
+    rc = report_overflow(m, s, "scone_model_eval_host");
+    if (rc) return rc;
     m->eval_B = B;
     return 0;
 }
@@ -1018,20 +1007,11 @@ extern "C" int scone_model_loss_grad_host(scone_model* m, int32_t B, const int32
                                           void* st) {
     SCONE_REQUIRE(m && ptr && last && tgt && mask && B >= 0, "scone_model_loss_grad_host: bad arguments");
     cudaStream_t s = as_stream(st);
-    const int64_t nnz = B > 0 ? ptr[B] : 0;
-    int rc = ensure_staging(m, B, nnz);
+    const bool overlap = fused_host_overlap_ok(m, B, B > 0 ? ptr[B] : 0);
+    int rc = stage_host_inputs(m, B, ptr, last, nullptr, tgt, mask, edge, val, !overlap, s);
     if (rc) return rc;
-    SCONE_CUDA(cudaMemcpyAsync(m->d_ptr, ptr, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    if (B) {
-        SCONE_CUDA(cudaMemcpyAsync(m->d_last, last, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-        SCONE_CUDA(cudaMemcpyAsync(m->d_tgt, tgt, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-        SCONE_CUDA(cudaMemcpyAsync(m->d_mask, mask, B * sizeof(float), cudaMemcpyHostToDevice, s));
-    }
-    if (fused_host_overlap_ok(m, B, nnz)) return fused_host_overlapped(m, B, ptr, edge, val, nullptr, true, zero_first, s);
-    if (nnz) {
-        SCONE_CUDA(cudaMemcpyAsync(m->d_edge, edge, nnz * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-        SCONE_CUDA(cudaMemcpyAsync(m->d_val, val, nnz * sizeof(float), cudaMemcpyHostToDevice, s));
-    }
+    if (overlap) return fused_host_overlapped(m, B, ptr, edge, val, nullptr, true, zero_first, s);
+    // (B == 0: only ptr was staged; the call still clears the gradient buffer when zero_first is set)
     return scone_model_loss_grad_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, m->d_tgt, m->d_mask, zero_first, st);
 }
 
@@ -1045,18 +1025,7 @@ extern "C" int scone_model_read_grads(scone_model* m, float* out, void* st) {
     SCONE_REQUIRE(m && out, "scone_model_read_grads: NULL argument");
     cudaStream_t s = as_stream(st);
     SCONE_CUDA(cudaMemcpyAsync(out, m->d_grad, (m->n_params + 2) * sizeof(float), cudaMemcpyDeviceToHost, s));
-    int overflow = 0;
-    if (m->d_overflow) SCONE_CUDA(cudaMemcpyAsync(&overflow, m->d_overflow, sizeof(int), cudaMemcpyDeviceToHost, s));
-    SCONE_CUDA(cudaStreamSynchronize(s));
-    if (overflow) {
-        cudaMemset(m->d_overflow, 0, sizeof(int));
-        m->cone_clean = false;
-        scone_set_error("scone_model: a micro-batch exceeded a row-list capacity (%d rows per compact tensor, %d rows of the backward's A "
-                        "buffer, 2048 cone edges per trajectory and layer); the gradients are incomplete — use a smaller micro-batch or "
-                        "scone_model_set_pipeline(m, 2 / 0)", m->row_cap, m->a_cap);
-        return 4;
-    }
-    return 0;
+    return report_overflow(m, s, "scone_model_read_grads");
 }
 
 // ---- planned sets (pipeline 4): plan a dataset once, run only the compute kernel on rows of it every step ----------------------
@@ -1073,17 +1042,9 @@ extern "C" int scone_model_plan_host(scone_model* m, int32_t B, const int32_t* p
                                      void* st) {
     SCONE_REQUIRE(m && B >= 0 && (B == 0 || (ptr && last)), "scone_model_plan_host: bad arguments");
     SCONE_REQUIRE(m->fused != nullptr, "scone_model_plan_host: planned sets need the fused pipeline (uniform width 16 / 32, <= 3 layers)");
-    cudaStream_t s = as_stream(st);
-    const int64_t nnz = B > 0 ? ptr[B] : 0;
     // the plan reads its inputs only while it is built: the staging buffers of the *_host entry points serve
-    int rc = ensure_staging(m, B, nnz);
+    int rc = stage_host_inputs(m, B, ptr, last, nullptr, nullptr, nullptr, edge, val, true, as_stream(st));
     if (rc) return rc;
-    SCONE_CUDA(cudaMemcpyAsync(m->d_ptr, ptr, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    if (nnz) {
-        SCONE_CUDA(cudaMemcpyAsync(m->d_edge, edge, nnz * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-        SCONE_CUDA(cudaMemcpyAsync(m->d_val, val, nnz * sizeof(float), cudaMemcpyHostToDevice, s));
-    }
-    if (B) SCONE_CUDA(cudaMemcpyAsync(m->d_last, last, B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     rc = scone_model_plan_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, st);
     if (rc) return rc;
     return scone_model_check_overflow(m, st);
@@ -1135,19 +1096,7 @@ extern "C" int scone_model_forward_planned_host(scone_model* m, int32_t n, const
 
 extern "C" int scone_model_check_overflow(scone_model* m, void* st) {
     SCONE_REQUIRE(m != nullptr, "scone_model_check_overflow: NULL model");
-    int overflow = 0;
-    cudaStream_t s = as_stream(st);
-    if (m->d_overflow) SCONE_CUDA(cudaMemcpyAsync(&overflow, m->d_overflow, sizeof(int), cudaMemcpyDeviceToHost, s));
-    SCONE_CUDA(cudaStreamSynchronize(s));
-    if (overflow) {
-        cudaMemset(m->d_overflow, 0, sizeof(int));
-        m->cone_clean = false;
-        scone_set_error("scone_model: a micro-batch exceeded a row-list capacity (%d rows per compact tensor, %d rows of the backward's A "
-                        "buffer, 2048 cone edges per trajectory and layer); results since the last check are incomplete and Adam steps were "
-                        "skipped — use a smaller micro-batch or another pipeline", m->row_cap, m->a_cap);
-        return 4;
-    }
-    return 0;
+    return report_overflow(m, as_stream(st), "scone_model_check_overflow");
 }
 
 extern "C" int scone_model_set_weights_keep_state(scone_model* m, const float* w, void* st) {
