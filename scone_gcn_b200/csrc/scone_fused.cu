@@ -1342,17 +1342,24 @@ int scone_fused_plan_finish(const scone_complex* cx, FusedState* f, int B, const
     return scone_table_plan_launch(f, plan_args(cx, f, 0, traj_ptr, flow_edge, flow_val, last_nodes, overflow), B, cx->num_sms, st, 1);
 }
 
-int scone_fused_compute(const scone_complex* cx, FusedState* f, int act, int b, const float* W, const int64_t* w_off, float* logprobs,
-                        const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st) {
-    if (b <= 0) return 0;
+// Arguments of the compute kernels over b trajectories planned into hdr / arena (rows: see TrajArgs)
+static TrajArgs traj_args(const scone_complex* cx, const FusedState* f, const int* hdr, const uint32_t* arena, const int32_t* rows, int b,
+                          const float* W, const int64_t* w_off, float* logprobs, const int32_t* target_idx, const float* mask, bool count_rows) {
     TrajArgs t;
-    t.hdr = f->d_hdr; t.arena = f->d_arena; t.rows = nullptr; t.W = W;
+    t.hdr = hdr; t.arena = arena; t.rows = rows; t.W = W;
     for (int i = 0; i <= 3 * kFusedMaxL; ++i) t.w_off[i] = i <= 3 * f->L ? (int)w_off[i] : 0;
     t.L = f->L; t.b = b; t.D = cx->D; t.n_params = (int)f->n_params;
     t.logprobs = logprobs; t.target_idx = target_idx; t.mask = mask;
     t.partial = f->d_partial; t.scratch = f->d_scratch; t.scratch_stride = f->scratch_stride;
     t.cap_rows = f->cap_rows; t.big_rows = f->big_rows;
     t.rows_done = count_rows ? f->d_rows_done : nullptr;
+    return t;
+}
+
+int scone_fused_compute(const scone_complex* cx, FusedState* f, int act, int b, const float* W, const int64_t* w_off, float* logprobs,
+                        const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st) {
+    if (b <= 0) return 0;
+    TrajArgs t = traj_args(cx, f, f->d_hdr, f->d_arena, nullptr, b, W, w_off, logprobs, target_idx, mask, count_rows);
     return run_traj(f, act, t, grad, st);
 }
 
@@ -1386,13 +1393,9 @@ int scone_fused_plan_set(const scone_complex* cx, FusedState* f, int B, const in
     }
     f->set_n = 0;
     SCONE_CUDA(cudaMemsetAsync(f->d_set_bump, 0, 2 * sizeof(unsigned long long), st));
-    PlanArgs p{};
-    p.flow_edge = flow_edge; p.flow_val = flow_val;
-    p.rank = cx->d_rank; p.nbrhoods = cx->d_nbrhoods; p.inc_ptr = cx->d_inc_ptr; p.inc_ent = cx->d_inc_ent;
-    p.mptr = cx->d_mptr; p.ment = cx->d_ment; p.cone_ptr = f->d_cone_ptr; p.cone_ent = f->d_cone_ent;
-    p.N = cx->N; p.D = cx->D; p.E = cx->E; p.L = f->L;
-    p.arena = f->d_set_arena; p.bump = f->d_set_bump; p.arena_words = f->set_arena_words; p.overflow = overflow;
-    p.n_retry = reinterpret_cast<int*>(f->d_set_bump + 1); p.retry = f->d_retry;
+    PlanArgs p = plan_args(cx, f, 0, traj_ptr, flow_edge, flow_val, last_nodes, overflow);
+    p.arena = f->d_set_arena; p.bump = f->d_set_bump; p.arena_words = f->set_arena_words;     // the set's own arena; hdr: per chunk
+    p.n_retry = reinterpret_cast<int*>(f->d_set_bump + 1);
     ScopedProf prof(SCONE_K_CONE, st);
     for (int off = 0; off < B; off += f->chunk) {
         const int b = std::min(f->chunk, B - off);
@@ -1411,14 +1414,7 @@ int scone_fused_run_planned(const scone_complex* cx, FusedState* f, int act, int
     if (n <= 0) return 0;
     SCONE_REQUIRE(f->set_n > 0, "scone_fused_run_planned: no planned set (call scone_model_plan_* first)");
     SCONE_REQUIRE(rows_dev != nullptr || n <= f->set_n, "scone_fused_run_planned: %d trajectories requested, the planned set holds %d", n, f->set_n);
-    TrajArgs t;
-    t.hdr = f->d_set_hdr; t.arena = f->d_set_arena; t.rows = rows_dev; t.W = W;
-    for (int i = 0; i <= 3 * kFusedMaxL; ++i) t.w_off[i] = i <= 3 * f->L ? (int)w_off[i] : 0;
-    t.L = f->L; t.b = n; t.D = cx->D; t.n_params = (int)f->n_params;
-    t.logprobs = logprobs; t.target_idx = target_idx; t.mask = mask;
-    t.partial = f->d_partial; t.scratch = f->d_scratch; t.scratch_stride = f->scratch_stride;
-    t.cap_rows = f->cap_rows; t.big_rows = f->big_rows;
-    t.rows_done = count_rows ? f->d_rows_done : nullptr;
+    TrajArgs t = traj_args(cx, f, f->d_set_hdr, f->d_set_arena, rows_dev, n, W, w_off, logprobs, target_idx, mask, count_rows);
     return run_traj(f, act, t, grad, st);
 }
 

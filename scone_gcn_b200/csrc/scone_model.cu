@@ -70,6 +70,9 @@ struct scone_model {
     int32_t eval_B = 0;                        // trajectories whose log-probs scone_model_eval_host left in d_logp_all
 };
 
+// The pipeline a model-level call runs: dense zero-fill needs the dense tensors of the unit kernels, whatever pipeline is set.
+static int active_pipeline(const scone_model* m) { return m->zero_fill ? 0 : m->pipeline; }
+
 namespace {
 
 int ensure_staging(scone_model* m, int64_t B, int64_t nnz) {
@@ -187,6 +190,51 @@ int forward_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edg
     return 0;
 }
 
+// backward over one micro-batch whose readout has written G_L: G_L -> G_{L-1} .. G_1, weight gradients accumulated into d_grad
+int backward_mb(scone_model* m, int32_t b, void* st) {
+    const int L = m->L;
+    int wl = -1, tt = 0;
+    for (int l = L - 1; l >= 0; --l) {
+        const int cout = m->hidden[l], cin = l > 0 ? m->hidden[l - 1] : 1;
+        const float* Hin = l > 0 ? m->d_H[l - 1] : m->d_X;
+        if (l > 0 && wait_fill(m, L + (l - 1), as_stream(st))) return 1;
+        SconeLaunchHints h;                  // the previous layer's output worklist; layer L - 1 compacts from the bitmap of G_L
+        h.in_wl = wl;
+        h.in_tt = tt;
+        h.skip_fill = l > 0;                 // G_{l-1}: filled on the side stream (or nobody does); layer 0 writes no G_{l-1}
+        if (l == L - 1) h.in_bm = m->d_bmG;
+        int rc = scone_layer_backward_hinted(m->cx, m->act, b, cin, cout, m->d_G[l], Hin, m->d_w + m->w_off[3 * l], m->d_w + m->w_off[3 * l + 1],
+                                             m->d_w + m->w_off[3 * l + 2], l > 0 ? m->d_G[l - 1] : nullptr, m->d_grad + m->w_off[3 * l], 1,
+                                             m->d_ws, m->d_occG[l], l > 0 ? m->d_occH[l - 1] : nullptr, l > 0 ? m->d_occG[l - 1] : nullptr,
+                                             m->d_occS, st, &h);
+        if (rc) return rc;
+        wl = h.out_wl;
+        tt = h.out_tt;
+    }
+    return 0;
+}
+
+// pipeline 0 over one micro-batch [off, off+b) (ptr / last / tgt / mask: at off); grad = false: log-probs only
+int unit_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last, float* logprobs,
+            const int32_t* tgt, const float* mask, bool grad, cudaStream_t s) {
+    const int L = m->L, CL = m->hidden[L - 1];
+    const float* wout = m->d_w + m->w_off[3 * L];
+    m->x_clean = false;
+    int rc = start_fills(m, b, grad, s);
+    if (!rc) rc = forward_mb(m, b, ptr, edge, val, s);
+    if (rc) return rc;
+    if (!grad)
+        return scone_readout_ws(m->cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, nullptr, nullptr, 0.f, nullptr, nullptr, nullptr,
+                                nullptr, 0, nullptr, m->d_occH[L - 1], nullptr, s, nullptr);
+    if (wait_fill(m, L + (L - 1), s)) return 1;
+    SconeLaunchHints h;                      // G_L: filled on the side stream (or nobody does); its flags also go to the bitmap d_bmG
+    h.skip_fill = true;
+    h.out_bm = m->d_bmG;
+    rc = scone_readout_ws(m->cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, tgt, mask, 1.f, m->d_G[L - 1], m->d_grad + m->w_off[3 * L],
+                          m->d_grad + m->n_params, m->d_grad + m->n_params + 1, 1, m->d_ws, m->d_occH[L - 1], m->d_occG[L - 1], s, &h);
+    return rc ? rc : backward_mb(m, b, s);
+}
+
 // ---- buffers of the active pipeline, allocated on first use ----------------------------------------------------------
 int dev_alloc(void** p, size_t bytes, const char* what) {
     if (*p) return 0;
@@ -207,7 +255,7 @@ int ensure_buffers(scone_model* m) {
     const scone_complex* cx = m->cx;
     const size_t E = cx->E, mb = m->mb;
     const int L = m->L;
-    const int pl = m->zero_fill ? 0 : m->pipeline;
+    const int pl = active_pipeline(m);
     if (!m->d_overflow) {
         SCONE_ALLOC(m->d_overflow, 256, "counters");
         SCONE_CUDA(cudaMemset(m->d_overflow, 0, 256));
@@ -398,6 +446,16 @@ int rows_backward_mb(scone_model* m, int32_t b, cudaStream_t s) {
                                       m->d_grad + m->w_off[0], 1, (float*)m->d_ws, compact ? m->row_cap : 0, s);
 }
 
+// pipelines 1 / 2 over one micro-batch (arguments as unit_mb)
+int rows_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last, float* logprobs,
+            const int32_t* tgt, const float* mask, bool grad, cudaStream_t s) {
+    int rc = rows_forward_mb(m, b, ptr, edge, val, s);
+    if (!rc) rc = rows_readout(m, b, last, logprobs, grad, tgt, mask, s);
+    if (!rc && grad) rc = rows_backward_mb(m, b, s);
+    if (!rc) rc = rows_clear_x(m, b, ptr, edge, val, s);
+    return rc;
+}
+
 // ---- cone-pruned row-list pipeline (3) -----------------------------------------------------------------------------
 // The log-probs of trajectory t read H_L only at the edges incident to the neighbours of its last node; H_{L-1} is needed one
 // hop around those rows, and so on: the receptive cone (geometry only: d_bmC[l], built from last_nodes).  Inside the cone only
@@ -503,6 +561,18 @@ int cone_backward_mb(scone_model* m, int32_t b, cudaStream_t s) {
     ScopedProf prof(SCONE_K_LAYER0_BWD, s);
     return scone_rows_layer0_backward(cx, b, m->hidden[0], m->d_X, m->d_cG[0], m->d_rowsC[0], cone_n(m, 0), m->d_grad + m->w_off[0], 1,
                                       (float*)m->d_ws, m->row_cap, s);
+}
+
+// pipeline 3 over one micro-batch (arguments as unit_mb)
+int cone_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last, float* logprobs,
+            const int32_t* tgt, const float* mask, bool grad, cudaStream_t s) {
+    int rc = cone_build_mb(m, b, ptr, edge, val, last, s);
+    if (!rc) rc = cone_forward_mb(m, b, s);
+    if (!rc) rc = cone_readout(m, b, last, logprobs, grad, tgt, mask, s);
+    if (!rc && grad) rc = cone_backward_mb(m, b, s);
+    if (!rc) rc = rows_clear_x(m, b, ptr, edge, val, s);
+    if (!rc) rc = cone_clear_mb(m, b, s);
+    return rc;
 }
 
 }  // namespace
@@ -677,7 +747,7 @@ extern "C" int scone_model_set_pipeline(scone_model* m, int32_t which) {
     }
     return 0;
 }
-extern "C" int scone_model_get_pipeline(const scone_model* m) { return m ? (m->zero_fill ? 0 : m->pipeline) : -1; }
+extern "C" int scone_model_get_pipeline(const scone_model* m) { return m ? active_pipeline(m) : -1; }
 extern "C" float* scone_model_weights_dev(scone_model* m) { return m ? m->d_w : nullptr; }
 extern "C" float* scone_model_grads_dev(scone_model* m) { return m ? m->d_grad : nullptr; }
 
@@ -737,8 +807,7 @@ static int fused_call(scone_model* m, int32_t B, const int32_t* ptr, const int32
 // are copied in four parts on a copy stream and every part is planned as soon as it has landed — the copy of part k + 1 runs under the
 // plan kernels of part k; one compute launch over the whole batch at the end.  ptr / last / tgt / mask: already enqueued on s.
 static bool fused_host_overlap_ok(const scone_model* m, int32_t B, int64_t nnz) {
-    const bool rows = m->pipeline >= 1 && !m->zero_fill;
-    return rows && m->pipeline == 4 && m->fused && B >= 512 && B <= m->fused->chunk && B <= m->mb && nnz >= (1 << 13);
+    return active_pipeline(m) == 4 && m->fused && B >= 512 && B <= m->fused->chunk && B <= m->mb && nnz >= (1 << 13);
 }
 
 static int fused_host_overlapped(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, float* logprobs_dev,
@@ -796,107 +865,35 @@ static int fused_host_overlapped(scone_model* m, int32_t B, const int32_t* ptr, 
     return finish_call(m, rc, (void*)s);
 }
 
-extern "C" int scone_model_forward_dev(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
-                                       const int32_t* last, float* logprobs, void* user_st) {
-    SCONE_REQUIRE(m && ptr && last && logprobs && B >= 0, "scone_model_forward_dev: bad arguments");
+// Forward (grad = false: log-probs to logprobs [B][D]) or loss + gradient (grad = true: into d_grad, cleared first if zero_first)
+static int run_batch(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last,
+                     float* logprobs, const int32_t* tgt, const float* mask, bool grad, int32_t zero_first, void* user_st) {
     if (fork_to_compute(m, user_st)) return 1;
-    void* st = (void*)m->compute;
-    const scone_complex* cx = m->cx;
-    const bool rows = m->pipeline >= 1 && !m->zero_fill;
-    if (rows && m->pipeline == 4) return finish_call(m, fused_call(m, B, ptr, edge, val, last, logprobs, nullptr, nullptr, false, as_stream(st)), user_st);
+    cudaStream_t s = m->compute;
+    if (grad && zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * sizeof(float), s));
+    const int pl = active_pipeline(m);
+    if (pl == 4) return finish_call(m, fused_call(m, B, ptr, edge, val, last, logprobs, tgt, mask, grad, s), user_st);
+    auto step = pl == 3 ? cone_mb : pl >= 1 ? rows_mb : unit_mb;
     int rc = 0;
     for (int32_t off = 0; off < B && !rc; off += m->mb) {
         const int32_t b = B - off < m->mb ? B - off : m->mb;
-        if (rows && m->pipeline == 3) {
-            rc = cone_build_mb(m, b, ptr + off, edge, val, last + off, as_stream(st));
-            if (!rc) rc = cone_forward_mb(m, b, as_stream(st));
-            if (!rc) rc = cone_readout(m, b, last + off, logprobs + (size_t)off * cx->D, false, nullptr, nullptr, as_stream(st));
-            if (!rc) rc = rows_clear_x(m, b, ptr + off, edge, val, as_stream(st));
-            if (!rc) rc = cone_clear_mb(m, b, as_stream(st));
-            continue;
-        }
-        if (rows) {
-            rc = rows_forward_mb(m, b, ptr + off, edge, val, as_stream(st));
-            if (!rc) rc = rows_readout(m, b, last + off, logprobs + (size_t)off * cx->D, false, nullptr, nullptr, as_stream(st));
-            if (!rc) rc = rows_clear_x(m, b, ptr + off, edge, val, as_stream(st));
-            continue;
-        }
-        m->x_clean = false;
-        rc = start_fills(m, b, false, as_stream(st));
-        if (!rc) rc = forward_mb(m, b, ptr + off, edge, val, st);
-        if (!rc)
-            rc = scone_readout_ws(cx, m->act, b, m->hidden[m->L - 1], m->d_H[m->L - 1], m->d_w + m->w_off[3 * m->L], last + off,
-                                  logprobs + (size_t)off * cx->D, nullptr, nullptr, 0.f, nullptr, nullptr, nullptr, nullptr, 0,
-                                  nullptr, m->d_occH[m->L - 1], nullptr, st, nullptr);
+        rc = step(m, b, ptr + off, edge, val, last + off, grad ? m->d_logp : logprobs + (size_t)off * m->cx->D, grad ? tgt + off : nullptr,
+                  grad ? mask + off : nullptr, grad, s);
     }
     return finish_call(m, rc, user_st);
+}
+
+extern "C" int scone_model_forward_dev(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
+                                       const int32_t* last, float* logprobs, void* user_st) {
+    SCONE_REQUIRE(m && ptr && last && logprobs && B >= 0, "scone_model_forward_dev: bad arguments");
+    return run_batch(m, B, ptr, edge, val, last, logprobs, nullptr, nullptr, false, 0, user_st);
 }
 
 extern "C" int scone_model_loss_grad_dev(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
                                          const int32_t* last, const int32_t* tgt, const float* mask, int32_t zero_first,
                                          void* user_st) {
     SCONE_REQUIRE(m && ptr && last && tgt && mask && B >= 0, "scone_model_loss_grad_dev: bad arguments");
-    if (fork_to_compute(m, user_st)) return 1;
-    void* st = (void*)m->compute;
-    const scone_complex* cx = m->cx;
-    const int L = m->L;
-    cudaStream_t s = as_stream(st);
-    if (zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * sizeof(float), s));
-    const bool rows = m->pipeline >= 1 && !m->zero_fill;
-    if (rows && m->pipeline == 4) return finish_call(m, fused_call(m, B, ptr, edge, val, last, nullptr, tgt, mask, true, s), user_st);
-    int rc = 0;
-    for (int32_t off = 0; off < B && !rc; off += m->mb) {
-        const int32_t b = B - off < m->mb ? B - off : m->mb;
-        if (rows && m->pipeline == 3) {
-            rc = cone_build_mb(m, b, ptr + off, edge, val, last + off, s);
-            if (!rc) rc = cone_forward_mb(m, b, s);
-            if (!rc) rc = cone_readout(m, b, last + off, m->d_logp, true, tgt + off, mask + off, s);
-            if (!rc) rc = cone_backward_mb(m, b, s);
-            if (!rc) rc = rows_clear_x(m, b, ptr + off, edge, val, s);
-            if (!rc) rc = cone_clear_mb(m, b, s);
-            continue;
-        }
-        if (rows) {
-            rc = rows_forward_mb(m, b, ptr + off, edge, val, s);
-            if (!rc) rc = rows_readout(m, b, last + off, m->d_logp, true, tgt + off, mask + off, s);
-            if (!rc) rc = rows_backward_mb(m, b, s);
-            if (!rc) rc = rows_clear_x(m, b, ptr + off, edge, val, s);
-            continue;
-        }
-        m->x_clean = false;
-        rc = start_fills(m, b, true, s);
-        if (!rc) rc = forward_mb(m, b, ptr + off, edge, val, st);
-        const int CL = m->hidden[L - 1];
-        if (!rc && wait_fill(m, L + (L - 1), s)) rc = 1;
-        if (rc) break;
-        SconeLaunchHints rh;                 // G_L: filled on the side stream (or nobody does); its flags also go to the bitmap d_bmG
-        rh.skip_fill = true;
-        rh.out_bm = m->d_bmG;
-        rc = scone_readout_ws(cx, m->act, b, CL, m->d_H[L - 1], m->d_w + m->w_off[3 * L], last + off, m->d_logp, tgt + off,
-                              mask + off, 1.f, m->d_G[L - 1], m->d_grad + m->w_off[3 * L], m->d_grad + m->n_params,
-                              m->d_grad + m->n_params + 1, 1, m->d_ws, m->d_occH[L - 1], m->d_occG[L - 1], st, &rh);
-        int wl = -1, tt = 0;
-        for (int l = L - 1; l >= 0 && !rc; --l) {
-            const int cout = m->hidden[l], cin = l > 0 ? m->hidden[l - 1] : 1;
-            const float* Hin = l > 0 ? m->d_H[l - 1] : m->d_X;
-            if (l > 0 && wait_fill(m, L + (l - 1), s)) {
-                rc = 1;
-                break;
-            }
-            SconeLaunchHints h;              // the previous layer's output worklist; layer L - 1 compacts from the bitmap of G_L
-            h.in_wl = wl;
-            h.in_tt = tt;
-            h.skip_fill = l > 0;             // G_{l-1}: filled on the side stream (or nobody does); layer 0 writes no G_{l-1}
-            if (l == L - 1) h.in_bm = m->d_bmG;
-            rc = scone_layer_backward_hinted(cx, m->act, b, cin, cout, m->d_G[l], Hin, m->d_w + m->w_off[3 * l],
-                                             m->d_w + m->w_off[3 * l + 1], m->d_w + m->w_off[3 * l + 2], l > 0 ? m->d_G[l - 1] : nullptr,
-                                             m->d_grad + m->w_off[3 * l], 1, m->d_ws, m->d_occG[l], l > 0 ? m->d_occH[l - 1] : nullptr,
-                                             l > 0 ? m->d_occG[l - 1] : nullptr, m->d_occS, st, &h);
-            wl = h.out_wl;
-            tt = h.out_tt;
-        }
-    }
-    return finish_call(m, rc, user_st);
+    return run_batch(m, B, ptr, edge, val, last, nullptr, tgt, mask, true, zero_first, user_st);
 }
 
 extern "C" int scone_model_forward_host(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
