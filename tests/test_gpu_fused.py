@@ -20,7 +20,7 @@ def cpu_live_rows(cx, n_layers, flows_row, last):
     for k in range(2):
         rowptr, col, val = cx.shift_csr(k)
         pats.append(sp.csr_matrix((np.ones(len(col)), col, rowptr), shape=(E, E)))
-    pat = ((pats[0] + pats[1] + sp.identity(E, format='csr')) > 0).astype(np.int8).tocsr()
+    pat = ((pats[0] + pats[1] + sp.identity(E, format='csr')) > 0).astype(np.int32).tocsr()
     nb = cx.nbrhoods[last]
     nb = nb[nb >= 0]
     en = cx._edge_nodes
@@ -30,10 +30,10 @@ def cpu_live_rows(cx, n_layers, flows_row, last):
     cones = [None] * (n_layers + 1)
     cones[n_layers] = top
     for l in range(n_layers - 1, 0, -1):
-        cones[l] = (pat @ cones[l + 1].astype(np.int8)) > 0
-    live = [None, cones[1] & ((pat @ (flows_row != 0).astype(np.int8)) > 0)]
+        cones[l] = (pat @ cones[l + 1].astype(np.int32)) > 0
+    live = [None, cones[1] & ((pat @ (flows_row != 0).astype(np.int32)) > 0)]
     for l in range(2, n_layers + 1):
-        live.append(cones[l] & ((pat @ live[l - 1].astype(np.int8)) > 0))
+        live.append(cones[l] & ((pat @ live[l - 1].astype(np.int32)) > 0))
     return live
 
 
