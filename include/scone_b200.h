@@ -144,12 +144,9 @@ int scone_model_create(const scone_complex* cx, int32_t n_layers, const int32_t*
                        scone_model** out);
 int scone_model_destroy(scone_model* m);
 int64_t scone_model_num_params(const scone_model* m);
-/* The model-level calls keep their activation / gradient tensors private, so by default (0) unflagged rows are never written
- * and traffic follows the support of the trajectories; 1 = bulk zero-fill every tensor once per micro-batch (complete dense
- * [E][b][C] arrays, the dense-streaming formulation).  Results are bit-identical either way. */
-int scone_model_set_zero_fill(scone_model* m, int32_t on);
-int scone_model_get_zero_fill(const scone_model* m);
-/* Model-level pipeline (same results within fp32 rounding; buffers of a pipeline are allocated on first use):
+/* Model-level pipeline (same results within fp32 rounding; buffers of a pipeline are allocated on first use).  The model-level calls
+ * keep their activation / gradient tensors private: rows outside the support of the trajectories are never written, so traffic
+ * follows that support.
  *   3 (default when every hidden width is 16 or 32) = pipeline 2's kernels restricted to the READOUT CONE: the log-probs of a
  *     trajectory read H_L only at the edges incident to the neighbours of its last node (trajectory_experiments.py:151,298-303),
  *     H_{L-1} one hop around those, and so on; the cone of layer l is both the rows of H_l the forward must produce and the rows
@@ -165,7 +162,7 @@ int scone_model_get_zero_fill(const scone_model* m);
  *     the trajectories, so micro_batch can be thousands (E * micro_batch < 2^31).  A compact tensor holds at most 32 M rows and
  *     the backward's A buffer 6 M rows per micro-batch; beyond that scone_model_read_grads reports an error.
  *   1 = the same row-list kernels over dense [E][micro_batch][C] tensors.
- *   0 = unit kernels over byte flags and dense tensors (every width; fp32 SIMT).  zero_fill = 1 always uses 0. */
+ *   0 = unit kernels over byte flags and dense tensors (every width; fp32 SIMT). */
 /*   4 (default when all hidden widths are equal, 16 or 32, with at most 3 layers, and the cones of the complex fit the shared-memory
  *     tables) = TRAJECTORY-FUSED kernels (csrc/scone_fused.cu): one plan kernel (cone & support -> per-trajectory live rows in ascending
  *     edge order + gather programs; weight-independent integer work) and one compute kernel that keeps all activations and
@@ -325,12 +322,8 @@ int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32_t* traj_pt
 int scone_bunch_read_grads(scone_bunch* m, float* out_host, void* stream);
 int scone_bunch_adam_step(scone_bunch* m, int32_t step, float lr, float weight_decay, void* stream);
 
-/* KERNEL-LEVEL calls: flagged kernels write only the rows that can be non-zero.  With zero-fill ON (default) every output tensor is first
- * bulk-zeroed, so it is a complete dense [E][b][C] array (the dense-streaming contract: each output byte written).
- * With zero-fill OFF unflagged rows are left unwritten and every consumer must honour the flags (all kernels of this
- * library do): traffic then scales with the support of the trajectories instead of E.  Results are identical. */
-int scone_set_zero_fill(int32_t on);
-int scone_get_zero_fill(void);
+/* KERNEL-LEVEL calls: every output of a public kernel-level call is a complete dense [E][b][C] array.  The flagged kernels compute
+ * only the rows that can be non-zero and bulk-zero the output tensor first. */
 
 /* Dense (no occupancy flags) fused layer kernels: 3 (default, see below) = tcgen05 / TMEM; 1 = slab kernels for widths 16 / 32 (merged-row gather straight
  * into mma.sync fragments, 3xTF32 tensor-core product, fp32-grade accuracy), a warp owning 16 trajectories of one edge;
@@ -344,15 +337,11 @@ int scone_set_dense_kernel(int32_t which);
  * operands in shared memory, accumulated in TMEM and folded into fp32 sums every 32 slabs (deterministic; Gprev may alias Hin).
  * scone_umma_status synchronises the stream and returns 3 if a launch reported an mbarrier time-out. */
 int scone_umma_status(void* stream);
-/* Tile order of the tcgen05 forward kernel: tiles (16 edges x 16 trajectories) are dealt to the CTAs in chunks of `tiles` consecutive
- * tiles, round-robin; 0 = one contiguous range per CTA.  Also read from SCONE_DENSE_CHUNK when the first dense layer runs. */
-int scone_set_dense_chunk(int32_t tiles);
 int scone_get_dense_kernel(void);
 
 /* Optional per-kernel-family device timing (CUDA events recorded on the launching stream around each launch);
  * off by default.  kind: 0 fused conv layer fwd, 1 fused conv layer bwd (+ its partial reduce), 2 first layer fwd,
- * 3 first layer bwd, 4 readout (+reduce), 5 flows->dense, 6 dense zero-fill of output tensors (on the model's side
- * stream in the model-level calls).  Used by bench.py for the roofline figures. */
+ * 3 first layer bwd, 4 readout (+reduce), 5 flows->dense, 6 dense zero-fill of output tensors.  Used by bench.py for the roofline figures. */
 int scone_profile_enable(int32_t on);
 int scone_profile_reset(void);
 int scone_profile_read(int32_t kind, int64_t* launches, double* total_ms);

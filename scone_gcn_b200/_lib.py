@@ -44,10 +44,7 @@ SIGNATURES = {
     'scone_layer_backward': (C.c_int, [_vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     'scone_readout_workspace': (_i64, [_i32, _i32]),
     'scone_readout': (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp]),
-    'scone_set_zero_fill': (C.c_int, [_i32]),
-    'scone_get_zero_fill': (C.c_int, []),
     'scone_set_dense_kernel': (C.c_int, [_i32]),
-    'scone_set_dense_chunk': (C.c_int, [_i32]),
     'scone_get_dense_kernel': (C.c_int, []),
     'scone_umma_status': (C.c_int, [_vp]),
     'scone_csr_create': (C.c_int, [_i32, _i32, _vp, _vp, _vp, C.POINTER(_vp)]),
@@ -65,8 +62,6 @@ SIGNATURES = {
     'scone_model_create': (C.c_int, [_vp, _i32, _vp, _i32, C.POINTER(_vp)]),
     'scone_model_destroy': (C.c_int, [_vp]),
     'scone_model_num_params': (_i64, [_vp]),
-    'scone_model_set_zero_fill': (C.c_int, [_vp, _i32]),
-    'scone_model_get_zero_fill': (C.c_int, [_vp]),
     'scone_model_set_pipeline': (C.c_int, [_vp, _i32]),
     'scone_model_get_pipeline': (C.c_int, [_vp]),
     'scone_model_set_weights': (C.c_int, [_vp, _vp]),

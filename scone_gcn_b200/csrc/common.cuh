@@ -36,7 +36,6 @@ extern std::atomic<long long> g_scone_launches;
 enum { SCONE_K_LAYER_FWD = 0, SCONE_K_LAYER_BWD = 1, SCONE_K_LAYER0_FWD = 2, SCONE_K_LAYER0_BWD = 3, SCONE_K_READOUT = 4,
        SCONE_K_OTHER = 5, SCONE_K_FILL = 6, SCONE_K_CONE = 7, SCONE_K_COUNT = 8 };
 extern bool g_scone_prof;
-extern bool g_scone_zero_fill;   // flagged kernels: bulk zero-fill outputs (dense-streaming contract) or leave unflagged rows unwritten
 void scone_prof_begin_impl(int kind, cudaStream_t st);
 void scone_prof_end_impl(int kind, cudaStream_t st);
 // device counter of the (edge, trajectory) rows a unit kernel family produced while profiling is on (NULL when off)
@@ -50,7 +49,7 @@ struct ScopedProf {
 // Hints the model-level code passes to one flagged kernel-level call (the *_hinted functions and scone_readout_ws below; nullptr =
 // none, which is what the public C entry points pass):
 //   in_wl/in_tt   the previous call's output worklist (index in the scratch, unit width) describes occ_in -> no re-compaction
-//   skip_fill     the caller zero-fills the output tensor itself (e.g. on a side stream)
+//   skip_fill     the caller reads only the flagged rows of the output: no zero-fill, unflagged rows stay unwritten
 // out_wl/out_tt are written back by the call (out_wl stays -1 when it built no output worklist).
 //   in_bm         row bitmap of occ_in (bit e*b + t set <=> flag byte set): compaction reads it instead of the E*b flag bytes
 //   out_bm        row bitmap the producer call (scone_flows_to_dense, scone_readout) should set next to the flags it writes

@@ -22,7 +22,6 @@
 // arena is sized for the worst case.  A trajectory whose rows do not fit the shared-memory row store runs in the BIG variant of
 // the same kernel (rows in a per-CTA global scratch).
 #include <algorithm>
-#include <cstdlib>
 #include <cub/device/device_radix_sort.cuh>
 #include "common.cuh"
 #include "fused.cuh"
@@ -1206,7 +1205,7 @@ int scone_fused_create(const scone_complex* cx, int L, int C, int mb, int64_t n_
         return 0;
     }
     {
-        // (tools/sweep_plan_tiers.sh on the 1M-edge bench complex: 1024 slots / 27 KB per CTA beat 2048 / 45 KB although twice as
+        // (measured on the 1M-edge bench complex: 1024 slots / 27 KB per CTA beat 2048 / 45 KB although twice as
         // many trajectories go to the second tier — occupancy is what the first tier lives on; 192 live rows / 3072 entries per
         // layer hold all but the trajectories the compute kernel sends to its big variant anyway)
         table_shape(f->quantile_cone, &f->HS0, &f->hshift0);
@@ -1216,16 +1215,6 @@ int scone_fused_create(const scone_complex* cx, int L, int C, int mb, int64_t n_
         if (!f->two_tiers) {
             f->HS0 = f->HS;
             f->hshift0 = f->hshift;
-        }
-        auto env_int = [](const char* name, int dflt) {    // tuning overrides (profiling experiments)
-            const char* v = getenv(name);
-            return v && *v ? atoi(v) : dflt;
-        };
-        if (f->two_tiers) {
-            const int hs0 = env_int("SCONE_FUSED_HS0", f->HS0);
-            if (hs0 != f->HS0 && hs0 >= 256 && hs0 <= f->HS && (hs0 & (hs0 - 1)) == 0) table_shape((hs0 * 3) / 4 - 1, &f->HS0, &f->hshift0);
-            f->LV0 = std::min(env_int("SCONE_FUSED_LV0", f->LV0), f->LV);
-            f->EC0 = std::min(env_int("SCONE_FUSED_EC0", f->EC0), f->EC);
         }
         f->plan_smem0 = plan_smem_bytes(f->HS0, f->LV0, f->EC0);
     }

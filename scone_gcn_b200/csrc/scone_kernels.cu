@@ -19,7 +19,6 @@
 // Weight gradients are accumulated in registers in a data-independent thread mapping and a fixed row order, written
 // as per-CTA partials and reduced in CTA order: bit-reproducible run to run.
 #include <math_constants.h>
-#include <cstdlib>
 #include "common.cuh"
 
 namespace {
@@ -944,10 +943,8 @@ __global__ void __launch_bounds__(kThreads) layer0_bwd_units_kernel(const float*
     }
 }
 
-// Dense zero-fill of an output tensor (128-bit streaming stores, grid-stride).  In the default (zero-fill ON) mode this is
-// where the HBM time of a step goes: every dense [E][b][C] tensor is written once per micro-batch.
-// One short-lived CTA per 32 KB chunk: SM slots turn over every few microseconds, so the (higher-priority) flag / unit
-// kernels of the main stream are scheduled in between instead of queueing behind a persistent fill.
+// Dense zero-fill of an output tensor of a public flagged kernel-level call (128-bit streaming stores): one short-lived CTA per
+// 32 KB chunk.
 __global__ void __launch_bounds__(kThreads) zero_fill_kernel(float4* __restrict__ p, size_t n16) {
     const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
     const size_t base = (size_t)blockIdx.x * ((size_t)kThreads * 8);
@@ -1270,12 +1267,6 @@ __global__ void adam_kernel(float* __restrict__ W, float* __restrict__ m, float*
     W[i] = W[i] - lr * (mi / c1) / (sqrtf(vi / c2) + eps);
 }
 
-}  // namespace
-
-bool g_scone_zero_fill = true;
-
-namespace {
-
 // =================================================================================================================
 // launchers
 // =================================================================================================================
@@ -1386,7 +1377,7 @@ int prepare_units(const scone_complex* cx, int b, const uint8_t* occ_in, uint8_t
     return compact_units<TT>(cx, b, occ_out, sc.wl[*out], sc.counts, sc.n[*out], st);
 }
 
-bool zero_fill_here(const SconeLaunchHints* h) { return g_scone_zero_fill && !(h && h->skip_fill); }
+bool zero_fill_here(const SconeLaunchHints* h) { return !(h && h->skip_fill); }
 
 template <int CIN, int COUT, int ACT>
 int launch_fwd(const scone_complex* cx, int b, const float* Hin, const float* W0, const float* W1, const float* W2, float* Hout,
@@ -1531,9 +1522,10 @@ int scone_zero_fill(const scone_complex* cx, void* p, size_t bytes, cudaStream_t
     }
     ScopedProf prof(SCONE_K_FILL, st);
     const size_t n16 = bytes / 16;
-    // the (unused) dynamic shared memory caps residency at ~4 fill CTAs per SM, leaving slots for the concurrent kernels
+    // the (unused) 56 KB of dynamic shared memory caps residency at ~4 fill CTAs per SM: the launch shape behind the recorded
+    // zero-fill timings (profile kind 6), kept so that they stay comparable
     static bool configured = false;
-    const int fill_smem = getenv("SCONE_FILL_SMEM") ? atoi(getenv("SCONE_FILL_SMEM")) : 56 * 1024;
+    constexpr int fill_smem = 56 * 1024;
     if (!configured) {
         SCONE_CUDA(cudaFuncSetAttribute(zero_fill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
         configured = true;
@@ -1546,12 +1538,6 @@ int scone_zero_fill(const scone_complex* cx, void* p, size_t bytes, cudaStream_t
 // ---------------------------------------------------------------------------------------------------------------
 // C ABI
 // ---------------------------------------------------------------------------------------------------------------
-extern "C" int scone_set_zero_fill(int32_t on) {
-    g_scone_zero_fill = on != 0;
-    return 0;
-}
-extern "C" int scone_get_zero_fill(void) { return g_scone_zero_fill ? 1 : 0; }
-
 #define SCONE_DISPATCH_WIDTHS(FN, ...)                                              \
     do {                                                                            \
         const int key_ = cin * 1000 + cout;                                         \
@@ -1760,7 +1746,7 @@ int scone_readout_ws(const scone_complex* cx, int32_t act, int32_t b, int32_t C,
     const SconeLaunchHints h = hints ? *hints : SconeLaunchHints{};
     if (GL) {
         SCONE_REQUIRE(target_idx && mask && workspace, "scone_readout: gradient mode needs target_idx, mask, workspace");
-        // without flags the consumer reads every row of GL: it must be dense zeros; with flags only when zero-fill is on
+        // GL is a complete dense array unless the caller reads its flagged rows only (skip_fill)
         const bool flagged = occ_GL != nullptr || h.out_bm != nullptr;
         if ((!flagged || zero_fill_here(&h)) && scone_zero_fill(cx, GL, (size_t)cx->E * b * C * sizeof(float), st)) return 1;
         if (occ_GL) SCONE_CUDA(cudaMemsetAsync(occ_GL, 0, (size_t)cx->E * b, st));

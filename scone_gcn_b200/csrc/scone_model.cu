@@ -24,19 +24,15 @@ struct scone_model {
     std::vector<float*> d_G;                  // dL/dZ of layer l, [E][mb][C_l]
     std::vector<uint8_t*> d_occH;             // occupancy flags of H_1..H_L, [E][mb]
     std::vector<uint8_t*> d_occG;             // occupancy flags of the dL/dZ buffers
-    cudaStream_t side = nullptr;              // zero-fill of the next tensors overlaps the current kernels (lowest priority)
     cudaStream_t compute = nullptr;           // all kernels of a model-level call (highest priority), forked from / joined to the caller's stream
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    cudaEvent_t ev_begin = nullptr;
     cudaStream_t copy = nullptr;              // pipeline 4, *_host entry points: the flow arrays arrive in parts under the plan kernels
     cudaEvent_t ev_copy0 = nullptr, ev_part[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     cudaEvent_t ev_plan_done = nullptr;       // the plan kernels of the last overlapped *_host call have read the flow staging buffers
     long long staging_epoch = 0, plan_done_epoch = -1;      // ensure_staging calls so far / value when ev_plan_done was recorded
-    std::vector<cudaEvent_t> ev_fill;         // [2L]: H_1..H_L, G_{L-1}..G_0
     uint8_t* d_occS = nullptr;                // worklists / counters scratch (scone_occ_scratch_bytes)
     uint8_t* d_occX = nullptr;                // flags of the flows X
     uint32_t *d_bmX = nullptr, *d_bmG = nullptr;   // quad bitmaps of the flags of X and of G_L (compaction reads these)
-    bool zero_fill = false;                   // dense zero-fill of every activation / gradient tensor (scone_model_set_zero_fill)
     // bitmap-native row-list pipeline (scone_rows.cu): row bitmaps per tensor, one row list, compact A rows for the dW GEMM
     // pipeline: 0 unit kernels + byte flags (dense [E][mb][C] tensors), 1 row lists over the dense tensors, 2 row lists over
     // COMPACT tensors (row r of a tensor at index rank(r) of its bitmap = its position in the compacted row list), 3 the same
@@ -69,9 +65,6 @@ struct scone_model {
     int64_t cap_choice = 0;
     int32_t eval_B = 0;                        // trajectories whose log-probs scone_model_eval_host left in d_logp_all
 };
-
-// The pipeline a model-level call runs: dense zero-fill needs the dense tensors of the unit kernels, whatever pipeline is set.
-static int active_pipeline(const scone_model* m) { return m->zero_fill ? 0 : m->pipeline; }
 
 namespace {
 
@@ -135,32 +128,6 @@ int report_overflow(scone_model* m, cudaStream_t s, const char* what) {
     return 4;
 }
 
-// Zero-fill of this micro-batch's dense tensors on the side stream (they are only written, never read, before their
-// consumer kernel runs): the fills overlap the small flag / unit kernels of the main stream.
-int start_fills(scone_model* m, int32_t b, bool with_grads, cudaStream_t s) {
-    if (!m->zero_fill) return 0;
-    const size_t E = m->cx->E;
-    SCONE_CUDA(cudaEventRecord(m->ev_begin, s));              // everything that still reads the old contents is before this
-    SCONE_CUDA(cudaStreamWaitEvent(m->side, m->ev_begin, 0));
-    for (int l = 0; l < m->L; ++l) {
-        if (scone_zero_fill(m->cx, m->d_H[l], E * b * m->hidden[l] * sizeof(float), m->side)) return 1;
-        SCONE_CUDA(cudaEventRecord(m->ev_fill[l], m->side));
-    }
-    if (with_grads)
-        for (int l = m->L - 1; l >= 0; --l) {
-            if (scone_zero_fill(m->cx, m->d_G[l], E * b * m->hidden[l] * sizeof(float), m->side)) return 1;
-            SCONE_CUDA(cudaEventRecord(m->ev_fill[m->L + l], m->side));
-        }
-    return 0;
-}
-// Orders s after the side-stream fill of tensor idx.  The kernel-level call that writes the tensor then gets skip_fill: either the
-// side stream filled it, or nobody does.
-int wait_fill(scone_model* m, int idx, cudaStream_t s) {
-    if (!m->zero_fill) return 0;
-    SCONE_CUDA(cudaStreamWaitEvent(s, m->ev_fill[idx], 0));
-    return 0;
-}
-
 // forward over one micro-batch [off, off+b): X -> H_1 .. H_L (kept) ; returns 0 on success
 int forward_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, void* st) {
     const scone_complex* cx = m->cx;
@@ -172,7 +139,6 @@ int forward_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edg
     int cin = 1, wl = -1, tt = 0;
     for (int l = 0; l < m->L; ++l) {
         const int cout = m->hidden[l];
-        if (wait_fill(m, l, as_stream(st))) return 1;
         SconeLaunchHints h;                  // the previous layer's output worklist; layer 0 compacts from the bitmap of X
         h.in_wl = wl;
         h.in_tt = tt;
@@ -197,11 +163,10 @@ int backward_mb(scone_model* m, int32_t b, void* st) {
     for (int l = L - 1; l >= 0; --l) {
         const int cout = m->hidden[l], cin = l > 0 ? m->hidden[l - 1] : 1;
         const float* Hin = l > 0 ? m->d_H[l - 1] : m->d_X;
-        if (l > 0 && wait_fill(m, L + (l - 1), as_stream(st))) return 1;
         SconeLaunchHints h;                  // the previous layer's output worklist; layer L - 1 compacts from the bitmap of G_L
         h.in_wl = wl;
         h.in_tt = tt;
-        h.skip_fill = l > 0;                 // G_{l-1}: filled on the side stream (or nobody does); layer 0 writes no G_{l-1}
+        h.skip_fill = l > 0;                 // layer 0 writes no G_{l-1}
         if (l == L - 1) h.in_bm = m->d_bmG;
         int rc = scone_layer_backward_hinted(m->cx, m->act, b, cin, cout, m->d_G[l], Hin, m->d_w + m->w_off[3 * l], m->d_w + m->w_off[3 * l + 1],
                                              m->d_w + m->w_off[3 * l + 2], l > 0 ? m->d_G[l - 1] : nullptr, m->d_grad + m->w_off[3 * l], 1,
@@ -220,14 +185,12 @@ int unit_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, 
     const int L = m->L, CL = m->hidden[L - 1];
     const float* wout = m->d_w + m->w_off[3 * L];
     m->x_clean = false;
-    int rc = start_fills(m, b, grad, s);
-    if (!rc) rc = forward_mb(m, b, ptr, edge, val, s);
+    int rc = forward_mb(m, b, ptr, edge, val, s);
     if (rc) return rc;
     if (!grad)
         return scone_readout_ws(m->cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, nullptr, nullptr, 0.f, nullptr, nullptr, nullptr,
                                 nullptr, 0, nullptr, m->d_occH[L - 1], nullptr, s, nullptr);
-    if (wait_fill(m, L + (L - 1), s)) return 1;
-    SconeLaunchHints h;                      // G_L: filled on the side stream (or nobody does); its flags also go to the bitmap d_bmG
+    SconeLaunchHints h;                      // G_L's flags also go to the bitmap d_bmG
     h.skip_fill = true;
     h.out_bm = m->d_bmG;
     rc = scone_readout_ws(m->cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, tgt, mask, 1.f, m->d_G[L - 1], m->d_grad + m->w_off[3 * L],
@@ -255,7 +218,7 @@ int ensure_buffers(scone_model* m) {
     const scone_complex* cx = m->cx;
     const size_t E = cx->E, mb = m->mb;
     const int L = m->L;
-    const int pl = active_pipeline(m);
+    const int pl = m->pipeline;
     if (!m->d_overflow) {
         SCONE_ALLOC(m->d_overflow, 256, "counters");
         SCONE_CUDA(cudaMemset(m->d_overflow, 0, 256));
@@ -662,14 +625,10 @@ extern "C" int scone_model_create(const scone_complex* cx, int32_t n_layers, con
     alloc((void**)&m->d_logp, mb * (size_t)(cx->D > 0 ? cx->D : 1) * sizeof(float));
     if (!rc) {
         int prio_lo = 0, prio_hi = 0;
-        cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);      // lowest priority: compute CTAs are scheduled first
-        cudaStreamCreateWithPriority(&m->side, cudaStreamNonBlocking, prio_lo);
+        cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
         cudaStreamCreateWithPriority(&m->compute, cudaStreamNonBlocking, prio_hi);
         cudaEventCreateWithFlags(&m->ev_fork, cudaEventDisableTiming);
         cudaEventCreateWithFlags(&m->ev_join, cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&m->ev_begin, cudaEventDisableTiming);
-        m->ev_fill.assign(2 * n_layers, nullptr);
-        for (auto& e : m->ev_fill) cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
         cudaMemset(m->d_w, 0, off * sizeof(float));
         cudaMemset(m->d_m, 0, off * sizeof(float));
         cudaMemset(m->d_v, 0, off * sizeof(float));
@@ -703,16 +662,13 @@ extern "C" int scone_model_destroy(scone_model* m) {
     for (float* p : m->d_G) cudaFree(p);
     cudaFree(m->d_ws); cudaFree(m->d_logp);
     scone_fused_destroy(m->fused);
-    if (m->side) cudaStreamDestroy(m->side);
     if (m->compute) cudaStreamDestroy(m->compute);
     if (m->ev_fork) cudaEventDestroy(m->ev_fork);
     if (m->ev_join) cudaEventDestroy(m->ev_join);
-    if (m->ev_begin) cudaEventDestroy(m->ev_begin);
     if (m->copy) cudaStreamDestroy(m->copy);
     if (m->ev_copy0) cudaEventDestroy(m->ev_copy0);
     if (m->ev_plan_done) cudaEventDestroy(m->ev_plan_done);
     for (auto e : m->ev_part) if (e) cudaEventDestroy(e);
-    for (auto e : m->ev_fill) if (e) cudaEventDestroy(e);
     cudaFree(m->d_ptr); cudaFree(m->d_edge); cudaFree(m->d_last); cudaFree(m->d_tgt); cudaFree(m->d_val);
     cudaFree(m->d_mask); cudaFree(m->d_logp_all); cudaFree(m->d_nn); cudaFree(m->d_acc);
     cudaFree(m->d_choice); cudaFree(m->d_rand); cudaFree(m->d_evalf);
@@ -721,13 +677,6 @@ extern "C" int scone_model_destroy(scone_model* m) {
 }
 
 extern "C" int64_t scone_model_num_params(const scone_model* m) { return m ? m->n_params : -1; }
-extern "C" int scone_model_set_zero_fill(scone_model* m, int32_t on) {
-    SCONE_REQUIRE(m != nullptr, "scone_model_set_zero_fill: NULL model");
-    SCONE_REQUIRE(!on || (size_t)m->cx->E * m->mb < ((size_t)1 << 31), "scone_model_set_zero_fill: E * micro_batch >= 2^31 runs on pipeline 3 only");
-    m->zero_fill = on != 0;
-    return ensure_buffers(m);
-}
-extern "C" int scone_model_get_zero_fill(const scone_model* m) { return m && m->zero_fill ? 1 : 0; }
 extern "C" int scone_model_set_pipeline(scone_model* m, int32_t which) {
     SCONE_REQUIRE(m != nullptr && which >= 0 && which <= 4,
                   "scone_model_set_pipeline: 0 (unit kernels, byte flags), 1 (row lists, dense tensors), 2 (row lists, compact tensors), "
@@ -747,7 +696,7 @@ extern "C" int scone_model_set_pipeline(scone_model* m, int32_t which) {
     }
     return 0;
 }
-extern "C" int scone_model_get_pipeline(const scone_model* m) { return m ? active_pipeline(m) : -1; }
+extern "C" int scone_model_get_pipeline(const scone_model* m) { return m ? m->pipeline : -1; }
 extern "C" float* scone_model_weights_dev(scone_model* m) { return m ? m->d_w : nullptr; }
 extern "C" float* scone_model_grads_dev(scone_model* m) { return m ? m->d_grad : nullptr; }
 
@@ -765,8 +714,8 @@ extern "C" int scone_model_get_weights(const scone_model* m, float* w) {
     return 0;
 }
 
-// The caller's stream is forked into the model's high-priority compute stream (and joined back): block scheduling
-// then prefers the flag / unit kernels over the low-priority zero-fill CTAs, so the two really overlap.
+// The caller's stream is forked into the model's highest-priority compute stream (and joined back): block scheduling then
+// prefers the library's kernels over work that other streams of the process have queued.
 static int fork_to_compute(scone_model* m, void* user_st) {
     SCONE_CUDA(cudaEventRecord(m->ev_fork, as_stream(user_st)));
     SCONE_CUDA(cudaStreamWaitEvent(m->compute, m->ev_fork, 0));
@@ -807,7 +756,7 @@ static int fused_call(scone_model* m, int32_t B, const int32_t* ptr, const int32
 // are copied in four parts on a copy stream and every part is planned as soon as it has landed — the copy of part k + 1 runs under the
 // plan kernels of part k; one compute launch over the whole batch at the end.  ptr / last / tgt / mask: already enqueued on s.
 static bool fused_host_overlap_ok(const scone_model* m, int32_t B, int64_t nnz) {
-    return active_pipeline(m) == 4 && m->fused && B >= 512 && B <= m->fused->chunk && B <= m->mb && nnz >= (1 << 13);
+    return m->pipeline == 4 && m->fused && B >= 512 && B <= m->fused->chunk && B <= m->mb && nnz >= (1 << 13);
 }
 
 static int fused_host_overlapped(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, float* logprobs_dev,
@@ -871,7 +820,7 @@ static int run_batch(scone_model* m, int32_t B, const int32_t* ptr, const int32_
     if (fork_to_compute(m, user_st)) return 1;
     cudaStream_t s = m->compute;
     if (grad && zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * sizeof(float), s));
-    const int pl = active_pipeline(m);
+    const int pl = m->pipeline;
     if (pl == 4) return finish_call(m, fused_call(m, B, ptr, edge, val, last, logprobs, tgt, mask, grad, s), user_st);
     auto step = pl == 3 ? cone_mb : pl >= 1 ? rows_mb : unit_mb;
     int rc = 0;

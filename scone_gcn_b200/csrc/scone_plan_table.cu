@@ -764,21 +764,16 @@ int scone_table_build(const scone_complex* cx, FusedState* f, int L, bool* ok) {
     if (want_rows) {
         f->tb_entries = te;
         f->tb_bytes = bytes;
-        auto env_int = [](const char* name, int dflt) {    // tuning overrides (profiling experiments)
-            const char* v = getenv(name);
-            return v && *v ? atoi(v) : dflt;
-        };
         // first tier: tables for the cones of ~99 % of the nodes and the live rows of all but the heaviest trajectories
-        f->tbM0 = std::min(f->tbM, (env_int("SCONE_TABLE_M0", f->quantile_cone) + 63) & ~63);
-        f->tbLV0 = std::min(f->tbLV, (env_int("SCONE_TABLE_LV0", 192) + 63) & ~63);
+        f->tbM0 = std::min(f->tbM, (f->quantile_cone + 63) & ~63);
+        f->tbLV0 = std::min(f->tbLV, 192);
         f->tb_two_tiers = f->tbM0 < f->tbM || f->tbLV0 < f->tbLV;
         f->tb_smem0 = table_plan_smem(f->tbM0, f->tbLV0);
         // middle tier: the cones of ~99.9 % of the nodes, 512 live rows per layer — a fraction of the last tier's shared memory
-        f->tbM1 = std::min(f->tbM, (env_int("SCONE_TABLE_M1", std::max(quantile999, 2 * f->tbM0)) + 63) & ~63);
-        f->tbLV1 = std::min(f->tbLV, (env_int("SCONE_TABLE_LV1", 512) + 63) & ~63);
+        f->tbM1 = std::min(f->tbM, (std::max(quantile999, 2 * f->tbM0) + 63) & ~63);
+        f->tbLV1 = std::min(f->tbLV, 512);
         f->tb_smem1 = table_plan_smem(f->tbM1, f->tbLV1);
         f->tb_mid_tier = f->tb_two_tiers && (f->tbM1 > f->tbM0 || f->tbLV1 > f->tbLV0) && 2 * f->tb_smem1 <= f->tb_smem;
-        SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
         SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
         SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
         SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<kTier1Threads>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
@@ -804,10 +799,7 @@ int scone_table_plan_launch(const FusedState* f, PlanArgs p, int b, int num_sms,
     p.retry = f->tb_two_tiers ? list0 : nullptr;
     p.n_retry = cnt0;
     if (phase != 1) {
-        static const int t0 = [] { const char* v = getenv("SCONE_TABLE_T0"); return v && *v ? atoi(v) : 128; }();
-        if (t0 == 64) table_plan_kernel<64><<<b, 64, f->tb_smem0, st>>>(p);
-        else if (t0 == 256) table_plan_kernel<256><<<b, 256, f->tb_smem0, st>>>(p);
-        else table_plan_kernel<128><<<b, 128, f->tb_smem0, st>>>(p);
+        table_plan_kernel<128><<<b, 128, f->tb_smem0, st>>>(p);
         SCONE_LAUNCHED();
     }
     if (!f->tb_two_tiers || phase == 0) return 0;

@@ -118,8 +118,8 @@ int dispatch_fwd_act(const scone_complex* cx, int act, int ts, int b, const floa
 // candidate rows.  rows[] holds the ids e*b + t of the rows of Hout that can be non-zero (ascending: the output's row
 // bitmap compacted by compact_bitmap_kernel); a warp takes 16 consecutive list entries.  Lane group q (the LPR = C/4 lanes
 // that cover one row) walks the merged operator row of ITS row; a neighbour row is loaded only if its flag byte in occ_in
-// (or, in the bitmap pipeline, its bit in bm_in) is set (unflagged rows are exact zeros and — with zero-fill off — may never
-// have been written).  All 16 rows' k-th
+// (or, in the bitmap pipeline, its bit in bm_in) is set (unflagged rows are exact zeros and, in the model-level
+// pipelines, may never have been written).  All 16 rows' k-th
 // neighbours are in flight together.  Each row's result is independent of the other rows in its slab and uses the same
 // summation order and mma sequence as the dense slab kernel: bit-identical to it.
 // =================================================================================================================

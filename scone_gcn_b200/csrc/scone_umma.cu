@@ -17,8 +17,6 @@
 // private barriers: while one group's tile is in the tensor core the other group gathers.  Weights are read once per 128 rows
 // (mma.sync: once per 16 rows) and the tensor instruction stream is one thread's, not every warp's.
 // Every wait is bounded: a protocol error sets *err and the kernel runs on (wrong results, reported by the host) instead of hanging.
-#include <cstdlib>
-#include <cstring>
 #include "common.cuh"
 
 namespace {
@@ -29,6 +27,10 @@ constexpr int kGatherWarps = 16, kGroupWarps = 8, kUmmaThreads = kGatherWarps * 
 // (no dedicated MMA warp: a 17th warp would put 5 warps on one SM sub-partition and cap every thread at 96 registers)
 constexpr int kC = 32;
 constexpr int kGatherDepth = 4;            // neighbour rows in flight per warp: the gather is bound by load latency at 17 warps per SM
+// Forward tile order: chunks of kTileChunk consecutive tiles dealt round-robin to the CTAs.  Inside a chunk the neighbour rows of
+// consecutive edges are L1 hits; with small chunks all CTAs sweep the same region of the tensor and an L1 miss is an L2 hit instead
+// of a DRAM read.  Measured on the 1M-edge complex: 9.34 ms at 8, 9.62 ms with one contiguous range per CTA, 10.86 ms at 1.
+constexpr int kTileChunk = 8;
 constexpr uint32_t kTmemCols = 512;
 constexpr uint32_t kColsAhi = 0, kColsAlo = 96, kColsD = 192, kColsGroup = 224;
 // f32 accumulate, tf32 x tf32, A / B K-major, N = 32, M = 128 (UMMA instruction descriptor, cute/arch/mma_sm100_desc.hpp)
@@ -102,7 +104,7 @@ template <int ACT>
 __global__ void __launch_bounds__(kUmmaThreads, 1) layer_fwd_umma_kernel(const float* __restrict__ Hin, float* __restrict__ Hout,
                                                                         const float* __restrict__ W0, const float* __restrict__ W1,
                                                                         const float* __restrict__ W2, const int32_t* __restrict__ mptr,
-                                                                        const int2* __restrict__ ment, int E, int b, int chunk, int* __restrict__ err) {
+                                                                        const int2* __restrict__ ment, int E, int b, int* __restrict__ err) {
     constexpr int TS = 16;
     using G = SlabGeom<kC, TS>;
     constexpr int NT = kC / 8;
@@ -142,11 +144,6 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) layer_fwd_umma_kernel(const f
     const int n_ts = (b + TS - 1) / TS;
     const int tiles_per_ts = (E + kGatherWarps - 1) / kGatherWarps;      // a CTA tile = 16 consecutive edges x one slab of 16 trajectories
     const long long n_tiles = (long long)n_ts * tiles_per_ts;
-    // Tile sequence of this CTA: chunks of `cl` consecutive tiles dealt round-robin to the CTAs (chunk = 0: one chunk per CTA, i.e.
-    // contiguous ranges).  Inside a chunk the neighbour rows of consecutive edges are L1 hits; with small chunks all CTAs sweep
-    // the same region of the tensor and an L1 miss is an L2 hit instead of a DRAM read.
-    const long long per = (n_tiles + gridDim.x - 1) / gridDim.x;
-    const long long cl = chunk > 0 ? (long long)chunk : per;
 
     {
         // ---- gather warps ----
@@ -159,7 +156,7 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) layer_fwd_umma_kernel(const f
         int pe0 = 0, pt0 = 0;                              // slab whose product is in flight
         bool pending = false, plive = false;
         for (long long k = 0;; ++k) {
-            const long long tile = ((k / cl) * gridDim.x + blockIdx.x) * cl + k % cl;
+            const long long tile = ((k / kTileChunk) * gridDim.x + blockIdx.x) * kTileChunk + k % kTileChunk;
             const bool have = tile < n_tiles;
             int e0 = 0, t0 = 0;
             bool live = false;
@@ -255,17 +252,6 @@ __global__ void __launch_bounds__(kUmmaThreads, 1) layer_fwd_umma_kernel(const f
 
 int* g_umma_err = nullptr;
 
-int g_dense_chunk = -1;
-int scone_dense_chunk() {                 // tiles per chunk of the forward kernel's tile sequence (0 = contiguous ranges)
-    int& chunk = g_dense_chunk;
-    if (chunk < 0) {
-        const char* e = getenv("SCONE_DENSE_CHUNK");
-        chunk = e ? atoi(e) : 8;                      // measured: 9.34 ms at 8, 9.62 contiguous, 10.86 at 1 (tools/sweep_dense_chunk.py)
-        if (chunk < 0) chunk = 0;
-    }
-    return chunk;
-}
-
 // =================================================================================================================
 // Backward of the same layer (32 -> 32, dense [E][b][32] tensors):
 //
@@ -286,6 +272,8 @@ int scone_dense_chunk() {                 // tiles per chunk of the forward kern
 // Buffer strides are padded (core-matrix pitch 144 B, k-chunk pitch = 8 words mod 32) so that the fragment-layout stores of a
 // warp hit 32 different banks.
 // =================================================================================================================
+constexpr int kBwdWarps = 12;              // warps per CTA: their operand buffers (BwdBuf) fill the shared memory
+constexpr int kBwdGatherDepth = 4;         // neighbour rows in flight per warp (measured faster than 6 or 8)
 constexpr int kFlushTiles = 32;            // slabs per warp between two flushes of the TMEM accumulators
 constexpr int kDW = 3 * kC * kC;
 
@@ -293,7 +281,6 @@ constexpr int kDW = 3 * kC * kC;
 // fragment value a lane keeps for k-step s, half h): the four lanes of a quad write four consecutive rows of ONE core matrix, so
 // with the k-chunk pitch at 16 banks mod 32 every fragment store of a warp hits 32 different banks at the canonical 128-byte
 // core-matrix pitch (16.6 KB per warp: 12 warps + 24 KB of weight fragments fill the 227 KB of shared memory)
-template <int NW>
 struct BwdBuf {
     static constexpr uint32_t SBO_A = 128u;                         // bytes between core matrices adjacent in M (8 accumulator rows)
     static constexpr uint32_t LBO_A = 1600u;                        // ... adjacent in K (row / 4): 12 core matrices of M + 64 B (16 banks)
@@ -336,15 +323,15 @@ __device__ __forceinline__ float umma_dact(float h) {               // derivativ
     return h > 0.f ? 1.f : 0.f;
 }
 
-template <int ACT, bool WG, int NW, int DEPTH>
-__global__ void __launch_bounds__(NW * 32, 1) layer_bwd_umma_kernel(const float* __restrict__ Gd, const float* Hin, float* Gprev,
-                                                                       const float* __restrict__ W0, const float* __restrict__ W1,
-                                                                       const float* __restrict__ W2, float* __restrict__ ws,
-                                                                       const int32_t* __restrict__ mptr, const int2* __restrict__ ment,
-                                                                       int E, int b, int interleave, int* __restrict__ err) {
-    constexpr int TS = 16;
+template <int ACT, bool WG>
+__global__ void __launch_bounds__(kBwdWarps * 32, 1) layer_bwd_umma_kernel(const float* __restrict__ Gd, const float* Hin, float* Gprev,
+                                                                           const float* __restrict__ W0, const float* __restrict__ W1,
+                                                                           const float* __restrict__ W2, float* __restrict__ ws,
+                                                                           const int32_t* __restrict__ mptr, const int2* __restrict__ ment,
+                                                                           int E, int b, int* __restrict__ err) {
+    constexpr int TS = 16, NW = kBwdWarps;
     using G = SlabGeom<kC, TS>;
-    using L = BwdBuf<NW>;
+    using L = BwdBuf;
     constexpr int NT = kC / 8;
     extern __shared__ __align__(128) unsigned char bw_smem[];
     __shared__ __align__(8) uint64_t s_bar[NW];
@@ -386,14 +373,11 @@ __global__ void __launch_bounds__(NW * 32, 1) layer_bwd_umma_kernel(const float*
     const int n_ts = b / TS;
     const int tiles_per_ts = (E + NW - 1) / NW;                          // a CTA tile = NW consecutive edges x one slab of 16 trajectories
     const long long n_tiles = (long long)n_ts * tiles_per_ts;
-    // Tile -> CTA.  Interleaved (default): CTA i takes tiles i, i + grid, ...: at any time the CTAs work on ~grid x NW consecutive edges
+    // Tile -> CTA, static and interleaved: CTA i takes tiles i, i + grid, ...: at any time the CTAs work on ~grid x NW consecutive edges
     // of one trajectory slab, every neighbour row comes from DRAM once and is an L2 hit for its other ~13 uses (the operand buffers
-    // leave ~16 KB of L1: the forward kernels' contiguous ranges, which live on L1 reuse, gave L1 14 % / L2 54 % hits and 1.97 x the
-    // compulsory DRAM reads here).  Static either way.
-    const long long per = (n_tiles + gridDim.x - 1) / gridDim.x;
-    const long long lo = interleave ? (long long)blockIdx.x : (long long)blockIdx.x * per;
-    const long long hi = interleave ? n_tiles : (lo + per < n_tiles ? lo + per : n_tiles);
-    const long long step = interleave ? (long long)gridDim.x : 1;
+    // leave ~16 KB of L1: contiguous tile ranges per CTA, which live on L1 reuse, gave L1 14 % / L2 54 % hits and 1.97 x the
+    // compulsory DRAM reads here).
+    const long long lo = blockIdx.x, hi = n_tiles, step = gridDim.x;
     // this warp's share of the flushes: TMEM lane quarter q = warp & 3 (term q of the stacked gradient) of the accumulators
     // j = warp >> 2, + nq, ... (nq = warps of this quarter); its running fp32 sums live in ws[cta][warp >> 2][term q][ci][co = lane]
     const int fq = warp & 3, fidx = warp >> 2, fnq = (NW - fq + 3) / 4;
@@ -417,7 +401,7 @@ __global__ void __launch_bounds__(NW * 32, 1) layer_bwd_umma_kernel(const float*
             for (int nt = 0; nt < NT; ++nt) hv[r][nt] = *reinterpret_cast<const float2*>(src + nt * 8);
         }
         u64 acc[3][G::NL][2];
-        slab_gather<kC, TS, DEPTH>(Gd, rowbytes, mptr, ment, E, b, e0, t0, acc);
+        slab_gather<kC, TS, kBwdGatherDepth>(Gd, rowbytes, mptr, ment, E, b, e0, t0, acc);
         if (pending) {                                                   // the MMAs of the previous slab have read the buffers
             mbar_wait(&s_bar[warp], phase, err);
             phase ^= 1u;
@@ -543,45 +527,22 @@ __global__ void __launch_bounds__(256) umma_reduce_partials_kernel(const float* 
     }
 }
 
-template <int ACT, bool WG, int NW, int DEPTH>
+template <int ACT, bool WG>
 int launch_bwd_umma(const scone_complex* cx, int b, const float* G, const float* Hin, const float* W0, const float* W1, const float* W2,
                     float* Gprev, float* ws, int* grid_out, cudaStream_t st) {
-    const size_t smem = (size_t)kBwdBfBytes + (size_t)NW * BwdBuf<NW>::WARP_BYTES;
-    auto kern = layer_bwd_umma_kernel<ACT, WG, NW, DEPTH>;
+    const size_t smem = (size_t)kBwdBfBytes + (size_t)kBwdWarps * BwdBuf::WARP_BYTES;
+    auto kern = layer_bwd_umma_kernel<ACT, WG>;
     static bool configured = false;
     if (!configured) {
         SCONE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured = true;
     }
-    const long long n_tiles = (long long)(b / 16) * ((cx->E + NW - 1) / NW);
+    const long long n_tiles = (long long)(b / 16) * ((cx->E + kBwdWarps - 1) / kBwdWarps);
     const int grid = (int)(n_tiles < cx->num_sms ? n_tiles : cx->num_sms);
     *grid_out = grid;
-    static int interleave = -1;
-    if (interleave < 0) {
-        const char* e = getenv("SCONE_UMMA_BWD_INTERLEAVE");             // 0: contiguous tile ranges per CTA (experiments)
-        interleave = (e && e[0] == '0') ? 0 : 1;
-    }
-    kern<<<grid, NW * 32, smem, st>>>(G, Hin, Gprev, W0, W1, W2, ws, cx->d_mptr, cx->d_ment, cx->E, b, interleave, g_umma_err);
+    kern<<<grid, kBwdWarps * 32, smem, st>>>(G, Hin, Gprev, W0, W1, W2, ws, cx->d_mptr, cx->d_ment, cx->E, b, g_umma_err);
     SCONE_LAUNCHED();
     return 0;
-}
-
-template <int ACT, bool WG>
-int dispatch_bwd_umma_cfg(const scone_complex* cx, int b, const float* G, const float* Hin, const float* W0, const float* W1,
-                          const float* W2, float* Gprev, float* ws, int* grid_out, cudaStream_t st) {
-    static int cfg = -1;
-    if (cfg < 0) {
-        const char* e = getenv("SCONE_UMMA_BWD_CFG");                    // "<warps>x<gather depth>" (experiments)
-        cfg = e ? atoi(e) * 100 + (strchr(e, 'x') ? atoi(strchr(e, 'x') + 1) : 4) : 1204;
-    }
-#define SCONE_BWD_CFG(NW_, D_) \
-    if (cfg == NW_ * 100 + D_) return launch_bwd_umma<ACT, WG, NW_, D_>(cx, b, G, Hin, W0, W1, W2, Gprev, ws, grid_out, st);
-    SCONE_BWD_CFG(10, 4)
-    SCONE_BWD_CFG(12, 4)
-    SCONE_BWD_CFG(12, 6)
-#undef SCONE_BWD_CFG
-    scone_set_error("SCONE_UMMA_BWD_CFG: unknown configuration %d", cfg);
-    return 2;
 }
 
 }  // namespace
@@ -601,16 +562,15 @@ int scone_umma_forward(const scone_complex* cx, int act, int b, const float* Hin
     const int n_ts = (b + 15) / 16;
     const long long n_tiles = (long long)n_ts * ((cx->E + kGatherWarps - 1) / kGatherWarps);
     const int grid = (int)(n_tiles < cx->num_sms ? n_tiles : cx->num_sms);
-    const int chunk = scone_dense_chunk();
     switch (act) {
         case SCONE_ACT_TANH:
-            layer_fwd_umma_kernel<SCONE_ACT_TANH><<<grid, kUmmaThreads, 0, st>>>(Hin, Hout, W0, W1, W2, cx->d_mptr, cx->d_ment, cx->E, b, chunk, g_umma_err);
+            layer_fwd_umma_kernel<SCONE_ACT_TANH><<<grid, kUmmaThreads, 0, st>>>(Hin, Hout, W0, W1, W2, cx->d_mptr, cx->d_ment, cx->E, b, g_umma_err);
             break;
         case SCONE_ACT_LEAKY_RELU:
-            layer_fwd_umma_kernel<SCONE_ACT_LEAKY_RELU><<<grid, kUmmaThreads, 0, st>>>(Hin, Hout, W0, W1, W2, cx->d_mptr, cx->d_ment, cx->E, b, chunk, g_umma_err);
+            layer_fwd_umma_kernel<SCONE_ACT_LEAKY_RELU><<<grid, kUmmaThreads, 0, st>>>(Hin, Hout, W0, W1, W2, cx->d_mptr, cx->d_ment, cx->E, b, g_umma_err);
             break;
         case SCONE_ACT_RELU:
-            layer_fwd_umma_kernel<SCONE_ACT_RELU><<<grid, kUmmaThreads, 0, st>>>(Hin, Hout, W0, W1, W2, cx->d_mptr, cx->d_ment, cx->E, b, chunk, g_umma_err);
+            layer_fwd_umma_kernel<SCONE_ACT_RELU><<<grid, kUmmaThreads, 0, st>>>(Hin, Hout, W0, W1, W2, cx->d_mptr, cx->d_ment, cx->E, b, g_umma_err);
             break;
         default:
             scone_set_error("unknown activation %d", act);
@@ -631,8 +591,8 @@ int scone_umma_backward(const scone_complex* cx, int act, int b, const float* G,
     int rc = 2, grid = 0;
 #define SCONE_UMMA_BWD(A)                                                                                                      \
     case A:                                                                                                                    \
-        rc = Gprev ? dispatch_bwd_umma_cfg<A, true>(cx, b, G, Hin, W0, W1, W2, Gprev, ws, &grid, st)                            \
-                   : dispatch_bwd_umma_cfg<A, false>(cx, b, G, Hin, W0, W1, W2, Gprev, ws, &grid, st);                          \
+        rc = Gprev ? launch_bwd_umma<A, true>(cx, b, G, Hin, W0, W1, W2, Gprev, ws, &grid, st)                                  \
+                   : launch_bwd_umma<A, false>(cx, b, G, Hin, W0, W1, W2, Gprev, ws, &grid, st);                                \
         break;
     switch (act) {
         SCONE_UMMA_BWD(SCONE_ACT_TANH)
@@ -646,12 +606,6 @@ int scone_umma_backward(const scone_complex* cx, int act, int b, const float* G,
     if (rc) return rc;
     umma_reduce_partials_kernel<<<(kDW + 31) / 32, 256, 0, st>>>(ws, 3 * grid, kDW, dW, accumulate);
     SCONE_LAUNCHED();
-    return 0;
-}
-
-extern "C" int scone_set_dense_chunk(int32_t tiles) {
-    SCONE_REQUIRE(tiles >= 0, "scone_set_dense_chunk: tiles per chunk must be >= 0 (0 = contiguous tile ranges per CTA)");
-    g_dense_chunk = tiles;
     return 0;
 }
 

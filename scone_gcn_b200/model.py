@@ -9,7 +9,7 @@ from . import _lib
 
 
 class SconeModel:
-    def __init__(self, cx, hidden, micro_batch=64, zero_fill=False):
+    def __init__(self, cx, hidden, micro_batch=64):
         self.cx = cx
         self.hidden = [int(h) for h in hidden]
         self.micro_batch = int(micro_batch)
@@ -19,8 +19,6 @@ class SconeModel:
         _lib.check(L.scone_model_create(cx.handle, len(self.hidden), _lib.ptr(harr), self.micro_batch, C.byref(h)),
                    'scone_model_create')
         self.handle = h
-        if zero_fill:
-            self.set_zero_fill(True)
         self.n_params = L.scone_model_num_params(h)
         self.planned = 0
         self.shapes = []
@@ -29,11 +27,6 @@ class SconeModel:
             self.shapes += [(cin, c)] * 3
             cin = c
         self.shapes.append((cin, 1))
-
-    def set_zero_fill(self, on):
-        """Dense zero-fill of every activation / gradient tensor once per micro-batch (default off: rows outside the
-        trajectories' support are never written; results are bit-identical)."""
-        _lib.check(_lib.lib().scone_model_set_zero_fill(self.handle, int(bool(on))), 'scone_model_set_zero_fill')
 
     @property
     def pipeline(self):

@@ -143,28 +143,3 @@ def test_umma_backward_many_slabs_per_warp_and_in_place():
     finally:
         L.scone_set_dense_kernel(_lib.DEFAULT_DENSE_KERNEL)
     assert np.array_equal(Hc.cpu().numpy(), Gp3) and np.array_equal(dW.cpu().numpy(), dW3)
-
-
-def test_umma_forward_does_not_depend_on_the_tile_order():
-    """scone_set_dense_chunk: tiles dealt to the CTAs in chunks of 1 / 8 / 64 or as contiguous ranges (0) — every row is computed by
-    one warp from the same inputs in the same order, so the output bits cannot depend on it."""
-    import scone_gcn_b200 as sg
-    from scone_gcn_b200 import _lib
-    from scone_gcn_b200 import synthetic_data_gen as sdg
-    sp = sdg.generate_sparse_dataset(3000, 8, seed=5, n_waypoints=8)
-    cx = sg.SimplicialComplex.from_simplices(int(sp.n_nodes), sp.edges, sp.faces, 'scone')
-    dev = torch.device('cuda')
-    g = torch.Generator(device='cpu').manual_seed(9)
-    b = 48
-    H = torch.randn(cx.E, b, 32, generator=g).to(dev)
-    W = [(torch.randn(32, 32, generator=g) * 0.2).to(dev) for _ in range(3)]
-    L = _lib.lib()
-    outs = []
-    try:
-        for chunk in (0, 1, 8, 64):
-            _lib.check(L.scone_set_dense_chunk(chunk))
-            outs.append(_run(cx, 0, b, H, W, 3))
-    finally:
-        L.scone_set_dense_chunk(8)
-    for o in outs[1:]:
-        assert np.array_equal(outs[0], o)

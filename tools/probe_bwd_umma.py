@@ -1,6 +1,6 @@
 """Dense backward probe: tcgen05 backward kernel (scone_set_dense_kernel(3)) against the fp32 SIMT tile kernel (0) on the same
 dense random tensors — max differences of Gprev and dW (and of dW_0 against float64), run-to-run bit-exactness, timing.
-SCONE_UMMA_BWD_CFG=<warps>x<gather depth> (10x4, 12x4, 12x6) picks the kernel variant.  Usage: python tools/probe_bwd_umma.py [n_nodes] [b]"""
+Usage: python tools/probe_bwd_umma.py [n_nodes] [b]"""
 import os
 import sys
 
@@ -21,7 +21,7 @@ E = cx.E
 dev = torch.device('cuda')
 st = torch.cuda.current_stream().cuda_stream
 PEAK = 6554.2
-print('complex: N=%d E=%d b=%d cfg=%s' % (n, E, b, os.environ.get('SCONE_UMMA_BWD_CFG', '10x4')), flush=True)
+print('complex: N=%d E=%d b=%d' % (n, E, b), flush=True)
 g = torch.Generator(device='cpu').manual_seed(1)
 H = torch.tanh(torch.randn(E, b, C, device=dev))
 G = torch.randn(E, b, C, device=dev)
