@@ -198,6 +198,22 @@ int scone_model_loss_grad_dev(scone_model* m, int32_t B, const int32_t* traj_ptr
 int scone_model_loss_grad_host(scone_model* m, int32_t B, const int32_t* traj_ptr, const int32_t* flow_edge,
                                const float* flow_val, const int32_t* last_nodes,
                                const int32_t* target_idx, const float* mask, int32_t zero_first, void* stream);
+/* Vector-Jacobian product of the log-probs (what jax.grad derives for ANY function of vmap(model)'s output, e.g. the reference's
+ * -sum(preds * y) / sum(mask) with a non-one-hot y, scone_trajectory_model.py:42-56,307).  cot [B][D] = upstream gradient
+ * dL/dlogprob[t][j]; accumulates into the same [grads | nll_sum | count] buffer as loss_grad (so scone_model_adam_step, the
+ * data-parallel step and an all-reduce of the buffer apply unchanged):
+ *   grads += sum_t sum_j cot[t][j] * d logprob[t][j] / dW ;  nll_sum += sum_t sum_j cot[t][j] * logprob[t][j] ;  count += count_add
+ * The readout's seed is dlogit_j = cot_j - p_j * sum_k cot_k with k over ALL D slots: a padded slot's log-prob depends on every real
+ * logit, while no gradient reaches its own constant logit.  Every sum is taken in a fixed order (deterministic).  With
+ * cot = -mask * onehot(target) and count_add = sum(mask), masks in {0, 1}, the buffer is bit for bit the one loss_grad leaves.
+ * The forward is recomputed inside the same pass (nothing from an earlier forward call is reused).  Same pipelines, micro-batching,
+ * copy overlap (*_host) and capacity-overflow flag as loss_grad.  cot == NULL with B > 0 is rejected (error code 2, nothing launched);
+ * B = 0 only clears the buffer (zero_first) and adds count_add. */
+int scone_model_vjp_dev(scone_model* m, int32_t B, const int32_t* traj_ptr_dev, const int32_t* flow_edge_dev, const float* flow_val_dev,
+                        const int32_t* last_nodes_dev, const float* cot_dev /* [B][D] */, float count_add, int32_t zero_first,
+                        void* stream);
+int scone_model_vjp_host(scone_model* m, int32_t B, const int32_t* traj_ptr, const int32_t* flow_edge, const float* flow_val,
+                         const int32_t* last_nodes, const float* cot /* [B][D] */, float count_add, int32_t zero_first, void* stream);
 /* Next-node accuracy on the device (scone_trajectory_model.py:59-71): for every trajectory with mask != 0 the prediction is
  * argmax_j of (j < n_nbrs[t] ? logprobs[t][j] : -100) over ALL D slots — the first maximum wins, a NaN wins over numbers, as
  * NumPy / JAX argmax — compared with target_idx[t].  out[0] = correct predictions, out[1] = masked trajectories (integers:
@@ -267,6 +283,11 @@ int scone_model_loss_grad_planned_host(scone_model* m, int32_t n, const int32_t*
 int scone_model_loss_grad_planned_dev(scone_model* m, int32_t n, const int32_t* rows_dev, const int32_t* target_idx_dev, const float* mask_dev,
                                       int32_t zero_first, void* stream);
 int scone_model_forward_planned_host(scone_model* m, int32_t n, const int32_t* rows, float* logprobs_out /* [n][D] */, void* stream);
+/* scone_model_vjp_* over rows of the planned set; cot [n][D] indexed by batch position. */
+int scone_model_vjp_planned_dev(scone_model* m, int32_t n, const int32_t* rows_dev, const float* cot_dev, float count_add, int32_t zero_first,
+                                void* stream);
+int scone_model_vjp_planned_host(scone_model* m, int32_t n, const int32_t* rows, const float* cot, float count_add, int32_t zero_first,
+                                 void* stream);
 /* Capacity overflow (pipelines 2 / 3 only; pipeline 4 and the dense pipelines cannot overflow): a micro-batch whose row lists exceed
  * their capacity sets a device flag.  While the flag is set scone_model_adam_step leaves the weights and the Adam state untouched (the
  * gradients are truncated).  The flag is REPORTED (error code 4) and cleared by scone_model_read_grads, scone_model_forward_host,
@@ -319,6 +340,10 @@ int scone_bunch_forward_host(scone_bunch* m, int32_t B, const int32_t* traj_ptr,
 int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32_t* traj_ptr, const int32_t* flow_edge, const float* flow_val,
                                const int32_t* last_nodes, const int32_t* target_idx, const float* mask, int32_t zero_first,
                                void* stream);
+/* VJP of the log-probs (scone_model_vjp_host's contract): the seed of slot j goes to the node slot j reads, a padded slot's to node
+ * N - 1 (negative indexing, as the forward reads it).  last_nodes checked as above; cot == NULL with B > 0: error code 2. */
+int scone_bunch_vjp_host(scone_bunch* m, int32_t B, const int32_t* traj_ptr, const int32_t* flow_edge, const float* flow_val,
+                         const int32_t* last_nodes, const float* cot /* [B][D] */, float count_add, int32_t zero_first, void* stream);
 int scone_bunch_read_grads(scone_bunch* m, float* out_host, void* stream);
 int scone_bunch_adam_step(scone_bunch* m, int32_t step, float lr, float weight_decay, void* stream);
 

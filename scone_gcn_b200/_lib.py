@@ -57,6 +57,7 @@ SIGNATURES = {
     'scone_bunch_get_weights': (C.c_int, [_vp, _vp]),
     'scone_bunch_forward_host': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     'scone_bunch_loss_grad_host': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp]),
+    'scone_bunch_vjp_host': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _i32, _vp]),
     'scone_bunch_read_grads': (C.c_int, [_vp, _vp, _vp]),
     'scone_bunch_adam_step': (C.c_int, [_vp, _i32, _f32, _f32, _vp]),
     'scone_model_create': (C.c_int, [_vp, _i32, _vp, _i32, C.POINTER(_vp)]),
@@ -72,6 +73,10 @@ SIGNATURES = {
     'scone_model_forward_dev': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     'scone_model_loss_grad_dev': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp]),
     'scone_model_loss_grad_host': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp]),
+    'scone_model_vjp_dev': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _i32, _vp]),
+    'scone_model_vjp_host': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _i32, _vp]),
+    'scone_model_vjp_planned_dev': (C.c_int, [_vp, _i32, _vp, _vp, _f32, _i32, _vp]),
+    'scone_model_vjp_planned_host': (C.c_int, [_vp, _i32, _vp, _vp, _f32, _i32, _vp]),
     'scone_accuracy_dev': (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     'scone_model_accuracy_host': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     'scone_model_read_grads': (C.c_int, [_vp, _vp, _vp]),

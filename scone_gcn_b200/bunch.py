@@ -105,6 +105,16 @@ class BunchModel:
                    'scone_bunch_loss_grad_host')
         return self.read_grads(stream) if read else None
 
+    def vjp(self, traj_ptr, flow_edge, flow_val, last_nodes, cot, count_add, zero_first=True, stream=None, read=True):
+        """VJP of the log-probs (SconeModel.vjp's contract); a padded slot's cotangent reaches node N - 1, the node it reads."""
+        B = len(last_nodes)
+        a = [np.ascontiguousarray(traj_ptr, np.int32), np.ascontiguousarray(flow_edge, np.int32),
+             np.ascontiguousarray(flow_val, np.float32), np.ascontiguousarray(last_nodes, np.int32),
+             np.ascontiguousarray(cot, np.float32).reshape(B, self.D)]
+        _lib.check(_lib.lib().scone_bunch_vjp_host(self.handle, B, *[_lib.ptr(x) for x in a], float(count_add), int(zero_first), stream),
+                   'scone_bunch_vjp_host')
+        return self.read_grads(stream) if read else None
+
     def read_grads(self, stream=None):
         buf = np.zeros(self.n_params + 2, np.float32)
         _lib.check(_lib.lib().scone_bunch_read_grads(self.handle, _lib.ptr(buf), stream), 'scone_bunch_read_grads')

@@ -121,7 +121,8 @@ int scone_layer_backward_hinted(const scone_complex* cx, int32_t act, int32_t b,
 int scone_readout_ws(const scone_complex* cx, int32_t act, int32_t b, int32_t C, const float* HL, const float* wout,
                      const int32_t* last_nodes, float* logprobs, const int32_t* target_idx, const float* mask,
                      float scale, float* GL, float* dwout, float* nll_sum, float* count, int32_t accumulate,
-                     void* workspace, const uint8_t* occ_HL, uint8_t* occ_GL, void* stream, const SconeLaunchHints* hints);
+                     void* workspace, const uint8_t* occ_HL, uint8_t* occ_GL, void* stream, const SconeLaunchHints* hints,
+                     const float* cot = nullptr);   // cot [b][D]: cotangent seed instead of target_idx / mask (readout_kernel)
 // data-parallel exchange fused with Adam (scone_dp.cu)
 struct scone_dp;
 int scone_dp_allreduce_adam(scone_dp* d, float* W, float* m, float* v, float* grad, int64_t n_params, const int* overflow_dev,
@@ -175,12 +176,13 @@ int scone_rows_readout_backward(const scone_complex* cx, int act, int b, int C, 
                                 const int32_t* last_nodes, const float* logprobs, const int32_t* target_idx, const float* mask,
                                 float scale, float* GL, const int* n_dev, int g_cap, int* overflow_dev, float* dwout, float* nll_sum,
                                 float* count, int accumulate, float* ws, const uint32_t* bmH, const uint32_t* prefH, const uint32_t* bmG,
-                                const uint32_t* prefG, cudaStream_t st);
+                                const uint32_t* prefG, cudaStream_t st, const float* cot = nullptr);
 int scone_accuracy_launch(int B, int D, const float* logprobs, const int32_t* n_nbrs, const int32_t* target_idx, const float* mask,
                           int32_t* out, cudaStream_t st);
 int scone_predict_launch(int B, int D, const float* logprobs, const int32_t* n_nbrs, int32_t* choice, cudaStream_t st);
 int scone_two_target_launch(int B, int D, const float* logprobs, const int32_t* n_nbrs, const int32_t* true_idx, const int32_t* rand_idx,
                             const float* mask, int32_t* out, cudaStream_t st);
 int scone_nll_launch(int B, int D, const float* logprobs, const int32_t* target_idx, const float* mask, float* out, cudaStream_t st);
+int scone_add_scalar_launch(float* dst, float v, cudaStream_t st);      // *dst += v on the stream (the count of a VJP call)
 int scone_adam_launch(float* W, float* m, float* v, const float* gradbuf, int64_t n, int32_t step, float lr,
                       float wd, void* stream, const int* overflow_dev = nullptr);

@@ -151,7 +151,8 @@ int scone_fused_create(const scone_complex* cx, int L, int C, int mb, int64_t n_
 void scone_fused_destroy(FusedState* f);
 int scone_fused_run(const scone_complex* cx, FusedState* f, int act, int b, const int32_t* traj_ptr, const int32_t* flow_edge,
                     const float* flow_val, const int32_t* last_nodes, const float* W, const int64_t* w_off, float* logprobs,
-                    const int32_t* target_idx, const float* mask, float* grad, int* overflow, bool count_rows, cudaStream_t st);
+                    const int32_t* target_idx, const float* mask, float* grad, int* overflow, bool count_rows, cudaStream_t st,
+                    const float* cot = nullptr);   // cot [b][D] (with grad): cotangent seed instead of target_idx / mask
 int scone_fused_begin(FusedState* f, cudaStream_t st);
 int scone_fused_plan_part(const scone_complex* cx, FusedState* f, int off, int b, const int32_t* traj_ptr, const int32_t* flow_edge,
                           const float* flow_val, const int32_t* last_nodes, int* overflow, cudaStream_t st,
@@ -159,10 +160,12 @@ int scone_fused_plan_part(const scone_complex* cx, FusedState* f, int off, int b
 int scone_fused_plan_finish(const scone_complex* cx, FusedState* f, int B, const int32_t* traj_ptr, const int32_t* flow_edge,
                             const float* flow_val, const int32_t* last_nodes, int* overflow, cudaStream_t st);
 int scone_fused_compute(const scone_complex* cx, FusedState* f, int act, int b, const float* W, const int64_t* w_off, float* logprobs,
-                        const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st);
+                        const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st,
+                        const float* cot = nullptr);
 int scone_fused_plan_set(const scone_complex* cx, FusedState* f, int B, const int32_t* traj_ptr, const int32_t* flow_edge,
                          const float* flow_val, const int32_t* last_nodes, int* overflow, cudaStream_t st);
 int scone_fused_run_planned(const scone_complex* cx, FusedState* f, int act, int n, const int32_t* rows_dev, const float* W, const int64_t* w_off,
-                            float* logprobs, const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st);
+                            float* logprobs, const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st,
+                            const float* cot = nullptr);
 int scone_fused_last_retries(FusedState* f);
 int scone_fused_read(FusedState* f, int t, int* hdr_out, unsigned off, int words, uint32_t* arena_out);

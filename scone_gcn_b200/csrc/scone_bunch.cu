@@ -306,11 +306,13 @@ __global__ void relu_bwd_kernel(const float* __restrict__ dX, const float* __res
     if (i < n) G[i] = h[i] > 0.f ? dX[i] : 0.f;
 }
 
-// readout: one thread per trajectory
+// readout: one thread per trajectory.  COT (cotangent seed, scone_bunch_vjp_host): dlogit_j = cot_j - p_j * sum_k cot_k over all D
+// slots, added to the node slot j reads (a padded slot reads node N - 1); partial = {sum_j cot_j * logp_j, 0}; tgt / mask unused.
+template <bool COT>
 __global__ void bunch_readout_kernel(const float* __restrict__ VL /* [N][b] */, const int32_t* __restrict__ nbrhoods,
                                      const int32_t* __restrict__ last_nodes, float* __restrict__ logprobs, const int32_t* __restrict__ tgt,
                                      const float* __restrict__ mask, float* __restrict__ dVL /* [N][b], pre-zeroed or NULL */,
-                                     float* __restrict__ partial /* [b][2] */, int N, int D, int b) {
+                                     float* __restrict__ partial /* [b][2] */, int N, int D, int b, const float* __restrict__ cot /* [b][D] */) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= b) return;
     const int last = last_nodes[t];
@@ -333,6 +335,21 @@ __global__ void bunch_readout_kernel(const float* __restrict__ VL /* [N][b] */, 
         logprobs[(size_t)t * D + j] = VL[(size_t)idx * b + t] - lse;
     }
     if (dVL == nullptr) return;
+    if (COT) {
+        const float* c = cot + (size_t)t * D;
+        float cs = 0.f, el = 0.f;
+        for (int j = 0; j < D; ++j) cs += c[j];
+        for (int j = 0; j < D; ++j) {
+            int idx = nbrhoods[(size_t)last * D + j];
+            if (idx < 0) idx += N;
+            const float lp = VL[(size_t)idx * b + t] - lse;
+            dVL[(size_t)idx * b + t] += c[j] - expf(lp) * cs;                          // same thread: sequential
+            el = fmaf(c[j], lp, el);
+        }
+        partial[2 * t] = el;
+        partial[2 * t + 1] = 0.f;
+        return;
+    }
     const float mk = mask[t];
     const int y = tgt[t];
     for (int j = 0; j < D; ++j) {
@@ -422,7 +439,7 @@ struct scone_bunch {
     float *d_logp = nullptr, *d_partial = nullptr;
     float* d_outer = nullptr;                 // [tiles][blocks][64] partial weight-gradient tiles
     int32_t *d_ptr = nullptr, *d_edge = nullptr, *d_last = nullptr, *d_tgt = nullptr;
-    float *d_val = nullptr, *d_mask = nullptr, *d_logp_all = nullptr;
+    float *d_val = nullptr, *d_mask = nullptr, *d_logp_all = nullptr, *d_cot = nullptr;
     int64_t cap_B = 0, cap_nnz = 0;
 };
 
@@ -435,7 +452,7 @@ extern "C" int scone_bunch_destroy(scone_bunch* m) {
     }
     cudaFree(m->d_U); cudaFree(m->d_dU); cudaFree(m->d_logp); cudaFree(m->d_partial); cudaFree(m->d_outer);
     cudaFree(m->d_ptr); cudaFree(m->d_edge); cudaFree(m->d_last); cudaFree(m->d_tgt); cudaFree(m->d_val); cudaFree(m->d_mask);
-    cudaFree(m->d_logp_all);
+    cudaFree(m->d_logp_all); cudaFree(m->d_cot);
     delete m;
     return 0;
 }
@@ -523,11 +540,12 @@ __global__ void flows_to_edges_kernel(const int32_t* __restrict__ ptr, const int
 
 int ensure_staging(scone_bunch* m, int64_t B, int64_t nnz) {
     if (B > m->cap_B) {
-        cudaFree(m->d_ptr); cudaFree(m->d_last); cudaFree(m->d_tgt); cudaFree(m->d_mask); cudaFree(m->d_logp_all);
+        cudaFree(m->d_ptr); cudaFree(m->d_last); cudaFree(m->d_tgt); cudaFree(m->d_mask); cudaFree(m->d_logp_all); cudaFree(m->d_cot);
         const int64_t cap = B + B / 4 + 16;
         SCONE_CUDA(cudaMalloc((void**)&m->d_ptr, (cap + 1) * 4)); SCONE_CUDA(cudaMalloc((void**)&m->d_last, cap * 4));
         SCONE_CUDA(cudaMalloc((void**)&m->d_tgt, cap * 4)); SCONE_CUDA(cudaMalloc((void**)&m->d_mask, cap * 4));
         SCONE_CUDA(cudaMalloc((void**)&m->d_logp_all, cap * (size_t)m->D * 4));
+        SCONE_CUDA(cudaMalloc((void**)&m->d_cot, cap * (size_t)m->D * 4));
         m->cap_B = cap;
     }
     if (nnz > m->cap_nnz) {
@@ -633,8 +651,8 @@ extern "C" int scone_bunch_forward_host(scone_bunch* m, int32_t B, const int32_t
     for (int32_t off = 0; off < B; off += m->mb) {
         const int b = B - off < m->mb ? B - off : m->mb;
         if (bunch_forward_mb(m, b, m->d_ptr + off, m->d_edge, m->d_val, st)) return 1;
-        bunch_readout_kernel<<<nblk(b), kBT, 0, st>>>(m->act[0][m->L], m->d_nbr, m->d_last + off, m->d_logp_all + (size_t)off * m->D, nullptr,
-                                                     nullptr, nullptr, nullptr, m->n[0], m->D, b);
+        bunch_readout_kernel<false><<<nblk(b), kBT, 0, st>>>(m->act[0][m->L], m->d_nbr, m->d_last + off, m->d_logp_all + (size_t)off * m->D,
+                                                            nullptr, nullptr, nullptr, nullptr, m->n[0], m->D, b, nullptr);
         SCONE_LAUNCHED();
     }
     SCONE_CUDA(cudaMemcpyAsync(logprobs_out, m->d_logp_all, (size_t)B * m->D * 4, cudaMemcpyDeviceToHost, st));
@@ -642,12 +660,11 @@ extern "C" int scone_bunch_forward_host(scone_bunch* m, int32_t B, const int32_t
     return 0;
 }
 
-extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
-                                          const int32_t* last, const int32_t* tgt, const float* mask, int32_t zero_first, void* stream) {
-    SCONE_REQUIRE(m && ptr && last && tgt && mask && B >= 0, "scone_bunch_loss_grad_host: bad arguments");
-    if (check_readout_indices("scone_bunch_loss_grad_host", m, B, last, tgt)) return 2;
-    cudaStream_t st = as_stream(stream);
+// loss + gradient (tgt / mask) or VJP (cot [B][D], count_add) over B trajectories from HOST buffers
+static int bunch_grad_host(scone_bunch* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last,
+                           const int32_t* tgt, const float* mask, const float* cot, float count_add, int32_t zero_first, cudaStream_t st) {
     if (zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * 4, st));
+    if (cot && count_add != 0.f && scone_add_scalar_launch(m->d_grad + m->n_params + 1, count_add, st)) return 1;
     if (B == 0) return 0;                                     // nothing to add: the buffer is cleared (zero_first) or left as it is
     const int64_t nnz = ptr[B];
     if (ensure_staging(m, B, nnz)) return 1;
@@ -657,8 +674,12 @@ extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32
         SCONE_CUDA(cudaMemcpyAsync(m->d_val, val, nnz * 4, cudaMemcpyHostToDevice, st));
     }
     SCONE_CUDA(cudaMemcpyAsync(m->d_last, last, B * 4, cudaMemcpyHostToDevice, st));
-    SCONE_CUDA(cudaMemcpyAsync(m->d_tgt, tgt, B * 4, cudaMemcpyHostToDevice, st));
-    SCONE_CUDA(cudaMemcpyAsync(m->d_mask, mask, B * 4, cudaMemcpyHostToDevice, st));
+    if (cot) {
+        SCONE_CUDA(cudaMemcpyAsync(m->d_cot, cot, (size_t)B * m->D * 4, cudaMemcpyHostToDevice, st));
+    } else {
+        SCONE_CUDA(cudaMemcpyAsync(m->d_tgt, tgt, B * 4, cudaMemcpyHostToDevice, st));
+        SCONE_CUDA(cudaMemcpyAsync(m->d_mask, mask, B * 4, cudaMemcpyHostToDevice, st));
+    }
     const int L = m->L;
     for (int32_t off = 0; off < B; off += m->mb) {
         const int b = B - off < m->mb ? B - off : m->mb;
@@ -666,8 +687,12 @@ extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32
         // dL/d(output of the last layer): only the node level is read by the readout
         int cur = 0;
         for (int lv = 0; lv < 3; ++lv) SCONE_CUDA(cudaMemsetAsync(m->d_dX[lv], 0, (size_t)m->n[lv] * b * m->width[L] * 4, st));
-        bunch_readout_kernel<<<nblk(b), kBT, 0, st>>>(m->act[0][L], m->d_nbr, m->d_last + off, m->d_logp, m->d_tgt + off, m->d_mask + off,
-                                                     m->d_dX[0], m->d_partial, m->n[0], m->D, b);
+        if (cot)
+            bunch_readout_kernel<true><<<nblk(b), kBT, 0, st>>>(m->act[0][L], m->d_nbr, m->d_last + off, m->d_logp, nullptr, nullptr, m->d_dX[0],
+                                                               m->d_partial, m->n[0], m->D, b, m->d_cot + (size_t)off * m->D);
+        else
+            bunch_readout_kernel<false><<<nblk(b), kBT, 0, st>>>(m->act[0][L], m->d_nbr, m->d_last + off, m->d_logp, m->d_tgt + off,
+                                                                m->d_mask + off, m->d_dX[0], m->d_partial, m->n[0], m->D, b, nullptr);
         SCONE_LAUNCHED();
         bunch_readout_reduce_kernel<<<1, 32, 0, st>>>(m->d_partial, b, m->d_grad + m->n_params, m->d_grad + m->n_params + 1);
         SCONE_LAUNCHED();
@@ -747,6 +772,21 @@ extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32
         }
     }
     return 0;
+}
+
+extern "C" int scone_bunch_loss_grad_host(scone_bunch* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
+                                          const int32_t* last, const int32_t* tgt, const float* mask, int32_t zero_first, void* stream) {
+    SCONE_REQUIRE(m && ptr && last && tgt && mask && B >= 0, "scone_bunch_loss_grad_host: bad arguments");
+    if (check_readout_indices("scone_bunch_loss_grad_host", m, B, last, tgt)) return 2;
+    return bunch_grad_host(m, B, ptr, edge, val, last, tgt, mask, nullptr, 0.f, zero_first, as_stream(stream));
+}
+
+extern "C" int scone_bunch_vjp_host(scone_bunch* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last,
+                                    const float* cot, float count_add, int32_t zero_first, void* stream) {
+    SCONE_REQUIRE(m && ptr && last && B >= 0, "scone_bunch_vjp_host: bad arguments");
+    SCONE_REQUIRE(cot || B == 0, "scone_bunch_vjp_host: cot is NULL");
+    if (check_readout_indices("scone_bunch_vjp_host", m, B, last, nullptr)) return 2;
+    return bunch_grad_host(m, B, ptr, edge, val, last, nullptr, nullptr, cot, count_add, zero_first, as_stream(stream));
 }
 
 extern "C" int scone_bunch_read_grads(scone_bunch* m, float* out, void* stream) {

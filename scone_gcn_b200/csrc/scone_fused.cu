@@ -464,6 +464,7 @@ struct TrajArgs {
     int cap_rows;                          // rows of the shared-memory row store (small variant)
     int big_rows;                          // rows of the per-CTA global row store
     unsigned long long* rows_done;         // optional device counters: [0] forward rows, [1] backward rows produced
+    const float* cot;                      // [b][D] cotangent seed of the COT variant (target_idx / mask unused), else NULL
 };
 
 template <int C>
@@ -652,7 +653,9 @@ __device__ __forceinline__ void fu_dw(float (&acc)[FuGeom<C>::TPW][4], const flo
     }
 }
 
-template <int C, int ACT, bool GRAD, bool BIG>
+// COT (with GRAD; scone_model_vjp_*): the readout's dlogit seed is dl_j = cot_j - p_j * sum_k cot_k over ALL D slots (padded slots
+// included: quirk Q1), the NLL slot takes sum_j cot_j * logp_j and the count slot 0.  Everything after the seed is shared.
+template <int C, int ACT, bool GRAD, bool BIG, bool COT = false>
 __global__ void __launch_bounds__(kTrajThreads, 2) fused_traj_kernel(const TrajArgs a) {
     using G = FuGeom<C>;
     extern __shared__ __align__(16) unsigned char sm[];
@@ -855,17 +858,31 @@ __global__ void __launch_bounds__(kTrajThreads, 2) fused_traj_kernel(const TrajA
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) se += __shfl_xor_sync(0xffffffffu, se, o);
             const float lse = mx + logf(se);
-            const float mk = GRAD ? a.mask[t] : 0.f;
-            const int y = GRAD ? a.target_idx[t] : -1;
+            const float mk = GRAD && !COT ? a.mask[t] : 0.f;
+            const int y = GRAD && !COT ? a.target_idx[t] : -1;
+            float cs = 0.f;                                // COT: sum_k cot_k (lane-strided, fixed butterfly); dl holds the row meanwhile
+            if (COT) {
+                for (int j = lane; j < D; j += 32) {
+                    const float c = a.cot[(size_t)t * D + j];
+                    dl[j] = c;
+                    cs += c;
+                }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) cs += __shfl_xor_sync(0xffffffffu, cs, o);
+            }
             for (int j = lane; j < D; j += 32) {
                 const float lp = lg[j] - lse;
                 if (a.logprobs != nullptr) a.logprobs[(size_t)t * D + j] = lp;
-                if (GRAD) {
+                if (COT) {
+                    const float c = dl[j];
+                    dl[j] = c - expf(lp) * cs;
+                    acc_nll = fmaf(c, lp, acc_nll);        // (summed over lanes at the end)
+                } else if (GRAD) {
                     dl[j] = mk * (expf(lp) - (j == y ? 1.f : 0.f));
                     if (j == y) acc_nll += -mk * lp;       // (lane y % 32 of warp 0 owns the term; summed over lanes at the end)
                 }
             }
-            if (GRAD && lane == 0) acc_cnt += mk;
+            if (GRAD && !COT && lane == 0) acc_cnt += mk;
         }
         if (!GRAD) {
             cp_async_wait_all();
@@ -1053,31 +1070,31 @@ size_t traj_smem_bytes(int D, int cap_rows) {
     return fl * sizeof(float);
 }
 
-template <int C, int ACT, bool GRAD>
+template <int C, int ACT, bool GRAD, bool COT>
 int launch_traj(const TrajArgs& base, int grid_small, int grid_big, size_t smem_small, size_t smem_big, cudaStream_t st) {
     static bool configured = false;
     if (!configured) {
-        SCONE_CUDA(cudaFuncSetAttribute(fused_traj_kernel<C, ACT, GRAD, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 1024));
-        SCONE_CUDA(cudaFuncSetAttribute(fused_traj_kernel<C, ACT, GRAD, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 1024));
+        SCONE_CUDA(cudaFuncSetAttribute(fused_traj_kernel<C, ACT, GRAD, false, COT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 1024));
+        SCONE_CUDA(cudaFuncSetAttribute(fused_traj_kernel<C, ACT, GRAD, true, COT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 1024));
         configured = true;
     }
     TrajArgs a = base;
-    fused_traj_kernel<C, ACT, GRAD, false><<<grid_small, kTrajThreads, smem_small, st>>>(a);
+    fused_traj_kernel<C, ACT, GRAD, false, COT><<<grid_small, kTrajThreads, smem_small, st>>>(a);
     SCONE_LAUNCHED();
     if (grid_big > 0) {
         if (GRAD) a.partial = base.partial + (size_t)grid_small * (base.n_params + 2);
-        fused_traj_kernel<C, ACT, GRAD, true><<<grid_big, kTrajThreads, smem_big, st>>>(a);
+        fused_traj_kernel<C, ACT, GRAD, true, COT><<<grid_big, kTrajThreads, smem_big, st>>>(a);
         SCONE_LAUNCHED();
     }
     return 0;
 }
 
-template <int C, bool GRAD>
+template <int C, bool GRAD, bool COT = false>
 int dispatch_traj(int act, const TrajArgs& a, int gs, int gb, size_t ss, size_t sb, cudaStream_t st) {
     switch (act) {
-        case SCONE_ACT_TANH: return launch_traj<C, SCONE_ACT_TANH, GRAD>(a, gs, gb, ss, sb, st);
-        case SCONE_ACT_LEAKY_RELU: return launch_traj<C, SCONE_ACT_LEAKY_RELU, GRAD>(a, gs, gb, ss, sb, st);
-        case SCONE_ACT_RELU: return launch_traj<C, SCONE_ACT_RELU, GRAD>(a, gs, gb, ss, sb, st);
+        case SCONE_ACT_TANH: return launch_traj<C, SCONE_ACT_TANH, GRAD, COT>(a, gs, gb, ss, sb, st);
+        case SCONE_ACT_LEAKY_RELU: return launch_traj<C, SCONE_ACT_LEAKY_RELU, GRAD, COT>(a, gs, gb, ss, sb, st);
+        case SCONE_ACT_RELU: return launch_traj<C, SCONE_ACT_RELU, GRAD, COT>(a, gs, gb, ss, sb, st);
     }
     scone_set_error("unknown activation %d", act);
     return 2;
@@ -1115,12 +1132,14 @@ int run_traj(FusedState* f, int act, TrajArgs& t, float* grad, cudaStream_t st) 
     t.okeys = k_out;
     t.order = v_out;
     int rc;
+    const int gs = f->grid_small, gb = f->grid_big;
+    const size_t ss = f->traj_smem_small, sb = f->traj_smem_big;
     if (f->C == 32)
-        rc = want_grad ? dispatch_traj<32, true>(act, t, f->grid_small, f->grid_big, f->traj_smem_small, f->traj_smem_big, st)
-                       : dispatch_traj<32, false>(act, t, f->grid_small, f->grid_big, f->traj_smem_small, f->traj_smem_big, st);
+        rc = !want_grad ? dispatch_traj<32, false>(act, t, gs, gb, ss, sb, st)
+                        : (t.cot ? dispatch_traj<32, true, true>(act, t, gs, gb, ss, sb, st) : dispatch_traj<32, true>(act, t, gs, gb, ss, sb, st));
     else
-        rc = want_grad ? dispatch_traj<16, true>(act, t, f->grid_small, f->grid_big, f->traj_smem_small, f->traj_smem_big, st)
-                       : dispatch_traj<16, false>(act, t, f->grid_small, f->grid_big, f->traj_smem_small, f->traj_smem_big, st);
+        rc = !want_grad ? dispatch_traj<16, false>(act, t, gs, gb, ss, sb, st)
+                        : (t.cot ? dispatch_traj<16, true, true>(act, t, gs, gb, ss, sb, st) : dispatch_traj<16, true>(act, t, gs, gb, ss, sb, st));
     if (rc) return rc;
     if (want_grad) {
         const int np = (int)f->n_params + 2;
@@ -1333,12 +1352,13 @@ int scone_fused_plan_finish(const scone_complex* cx, FusedState* f, int B, const
 
 // Arguments of the compute kernels over b trajectories planned into hdr / arena (rows: see TrajArgs)
 static TrajArgs traj_args(const scone_complex* cx, const FusedState* f, const int* hdr, const uint32_t* arena, const int32_t* rows, int b,
-                          const float* W, const int64_t* w_off, float* logprobs, const int32_t* target_idx, const float* mask, bool count_rows) {
+                          const float* W, const int64_t* w_off, float* logprobs, const int32_t* target_idx, const float* mask, const float* cot,
+                          bool count_rows) {
     TrajArgs t;
     t.hdr = hdr; t.arena = arena; t.rows = rows; t.W = W;
     for (int i = 0; i <= 3 * kFusedMaxL; ++i) t.w_off[i] = i <= 3 * f->L ? (int)w_off[i] : 0;
     t.L = f->L; t.b = b; t.D = cx->D; t.n_params = (int)f->n_params;
-    t.logprobs = logprobs; t.target_idx = target_idx; t.mask = mask;
+    t.logprobs = logprobs; t.target_idx = target_idx; t.mask = mask; t.cot = cot;
     t.partial = f->d_partial; t.scratch = f->d_scratch; t.scratch_stride = f->scratch_stride;
     t.cap_rows = f->cap_rows; t.big_rows = f->big_rows;
     t.rows_done = count_rows ? f->d_rows_done : nullptr;
@@ -1346,20 +1366,21 @@ static TrajArgs traj_args(const scone_complex* cx, const FusedState* f, const in
 }
 
 int scone_fused_compute(const scone_complex* cx, FusedState* f, int act, int b, const float* W, const int64_t* w_off, float* logprobs,
-                        const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st) {
+                        const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st, const float* cot) {
     if (b <= 0) return 0;
-    TrajArgs t = traj_args(cx, f, f->d_hdr, f->d_arena, nullptr, b, W, w_off, logprobs, target_idx, mask, count_rows);
+    TrajArgs t = traj_args(cx, f, f->d_hdr, f->d_arena, nullptr, b, W, w_off, logprobs, target_idx, mask, cot, count_rows);
     return run_traj(f, act, t, grad, st);
 }
 
 int scone_fused_run(const scone_complex* cx, FusedState* f, int act, int b, const int32_t* traj_ptr, const int32_t* flow_edge,
                     const float* flow_val, const int32_t* last_nodes, const float* W, const int64_t* w_off, float* logprobs,
-                    const int32_t* target_idx, const float* mask, float* grad, int* overflow, bool count_rows, cudaStream_t st) {
+                    const int32_t* target_idx, const float* mask, float* grad, int* overflow, bool count_rows, cudaStream_t st,
+                    const float* cot) {
     if (b <= 0) return 0;
     SCONE_REQUIRE(b <= f->chunk, "scone_fused_run: chunk of %d trajectories exceeds the planned %d", b, f->chunk);
     int rc = scone_fused_begin(f, st);
     if (!rc) rc = scone_fused_plan_part(cx, f, 0, b, traj_ptr, flow_edge, flow_val, last_nodes, overflow, st);
-    if (!rc) rc = scone_fused_compute(cx, f, act, b, W, w_off, logprobs, target_idx, mask, grad, count_rows, st);
+    if (!rc) rc = scone_fused_compute(cx, f, act, b, W, w_off, logprobs, target_idx, mask, grad, count_rows, st, cot);
     return rc;
 }
 
@@ -1399,11 +1420,12 @@ int scone_fused_plan_set(const scone_complex* cx, FusedState* f, int B, const in
 
 // Compute kernel over n trajectories of the planned set (rows_dev[t] = index into the set; NULL = the first n of the set).
 int scone_fused_run_planned(const scone_complex* cx, FusedState* f, int act, int n, const int32_t* rows_dev, const float* W, const int64_t* w_off,
-                            float* logprobs, const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st) {
+                            float* logprobs, const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st,
+                            const float* cot) {
     if (n <= 0) return 0;
     SCONE_REQUIRE(f->set_n > 0, "scone_fused_run_planned: no planned set (call scone_model_plan_* first)");
     SCONE_REQUIRE(rows_dev != nullptr || n <= f->set_n, "scone_fused_run_planned: %d trajectories requested, the planned set holds %d", n, f->set_n);
-    TrajArgs t = traj_args(cx, f, f->d_set_hdr, f->d_set_arena, rows_dev, n, W, w_off, logprobs, target_idx, mask, count_rows);
+    TrajArgs t = traj_args(cx, f, f->d_set_hdr, f->d_set_arena, rows_dev, n, W, w_off, logprobs, target_idx, mask, cot, count_rows);
     return run_traj(f, act, t, grad, st);
 }
 

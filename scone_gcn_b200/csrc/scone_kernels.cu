@@ -1119,7 +1119,10 @@ constexpr int kReadoutMaxD = SCONE_MAX_DEGREE, kReadoutMaxCper = 4;   // D <= 12
 // One CTA (4 warps) per trajectory; warp w owns the neighbour slots j = w, w + 4, ...  A row of GL receives at most two
 // contributions (an edge has two end nodes), added with atomicAdd onto a zeroed row: a + b == b + a, so the result does not
 // depend on the order (deterministic without serialising the warps).
+// COT (cotangent seed, scone_model_vjp_*): dlogit_j = cot_j - p_j * sum_k cot_k over ALL D slots (a padded slot's log-prob depends on
+// every real logit), the NLL slot of the partials takes sum_j cot_j * logprob_j and the count slot 0; target_idx / mask are not read.
 constexpr int kReadoutWarps = 4;
+template <bool COT>
 __global__ void __launch_bounds__(32 * kReadoutWarps) readout_kernel(const float* __restrict__ HL, const float* __restrict__ wout,
                                                      const int32_t* __restrict__ last_nodes, const int32_t* __restrict__ nbrhoods,
                                                      const int32_t* __restrict__ inc_ptr, const int2* __restrict__ inc_ent,
@@ -1128,12 +1131,14 @@ __global__ void __launch_bounds__(32 * kReadoutWarps) readout_kernel(const float
                                                      float* __restrict__ partial /* [b][C+2] */, const uint8_t* __restrict__ occ_HL,
                                                      uint8_t* __restrict__ occ_GL, uint32_t* __restrict__ bm_GL, int act, int N, int D,
                                                      int b, int C, const uint32_t* __restrict__ bm_HL, uint32_t* __restrict__ bm_cand,
-                                                     const int32_t* __restrict__ mptr, const int2* __restrict__ ment) {
+                                                     const int32_t* __restrict__ mptr, const int2* __restrict__ ment,
+                                                     const float* __restrict__ cot /* [b][D], COT */) {
     // bm_HL != NULL: the row bitmap of H_L replaces the flag bytes; bm_cand != NULL: every row of G_L this trajectory touches
     // also marks the candidate rows one hop further (its merged operator row) for the first backward layer
     __shared__ float logit[kReadoutMaxD];
     __shared__ float s_dw[kReadoutWarps][32 * kReadoutMaxCper];
     __shared__ float s_lse;
+    __shared__ float s_cot[COT ? kReadoutMaxD : 1], s_csum, s_ell;
     const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
     const int t = blockIdx.x;
     const int last = last_nodes[t];
@@ -1174,6 +1179,21 @@ __global__ void __launch_bounds__(32 * kReadoutWarps) readout_kernel(const float
         const float lse_ = mx + logf(se);
         for (int j = lane; j < D; j += 32) logprobs[(size_t)t * D + j] = logit[j] - lse_;
         if (lane == 0) s_lse = lse_;
+        if (COT && GL != nullptr) {                        // the cotangent row, its sum and sum_j cot_j * logprob_j (fixed order)
+            float cs = 0.f, el = 0.f;
+            for (int j = lane; j < D; j += 32) {
+                const float c = cot[(size_t)t * D + j];
+                s_cot[j] = c;
+                cs += c;
+                el = fmaf(c, logit[j] - lse_, el);
+            }
+            cs = warp_sum(cs);
+            el = warp_sum(el);
+            if (lane == 0) {
+                s_csum = cs;
+                s_ell = el;
+            }
+        }
     }
     if (GL == nullptr) return;
     // gradient: the rows of GL this trajectory touches are zeroed and flagged first ...
@@ -1198,13 +1218,13 @@ __global__ void __launch_bounds__(32 * kReadoutWarps) readout_kernel(const float
     }
     __syncthreads();                                       // ... (also publishes s_lse) then accumulated
     const float lse = s_lse;
-    const float mk = mask[t];
-    const int y = target_idx[t];
+    const float mk = COT ? 0.f : mask[t];
+    const int y = COT ? -1 : target_idx[t];
     float dwl[kReadoutMaxCper] = {0.f, 0.f, 0.f, 0.f};
     for (int j = warp; j < D; j += kReadoutWarps) {
         const int nbr = last_ok ? nbrhoods[(size_t)last * D + j] : -1;
         if (nbr < 0) continue;
-        const float dl = mk * scale * (expf(logit[j] - lse) - (j == y ? 1.f : 0.f));
+        const float dl = COT ? s_cot[j] - expf(logit[j] - lse) * s_csum : mk * scale * (expf(logit[j] - lse) - (j == y ? 1.f : 0.f));
         for (int p = inc_ptr[nbr]; p < inc_ptr[nbr + 1]; ++p) {
             const int2 es = inc_ent[p];
             const size_t base = ((size_t)es.x * b + t) * C;
@@ -1233,7 +1253,7 @@ __global__ void __launch_bounds__(32 * kReadoutWarps) readout_kernel(const float
                 pt[lane + 32 * q] = sacc;
             }
         if (lane == 0) {
-            pt[C] = (y >= 0 && y < D) ? -mk * (logit[y] - lse) : 0.f;
+            pt[C] = COT ? s_ell : ((y >= 0 && y < D) ? -mk * (logit[y] - lse) : 0.f);
             pt[C + 1] = mk;
         }
     }
@@ -1736,7 +1756,7 @@ int64_t scone_readout_workspace_bytes(int32_t b, int32_t C) { return (int64_t)b 
 int scone_readout_ws(const scone_complex* cx, int32_t act, int32_t b, int32_t C, const float* HL, const float* wout,
                      const int32_t* last_nodes, float* logprobs, const int32_t* target_idx, const float* mask, float scale,
                      float* GL, float* dwout, float* nll_sum, float* count, int32_t accumulate, void* workspace,
-                     const uint8_t* occ_HL, uint8_t* occ_GL, void* stream, const SconeLaunchHints* hints) {
+                     const uint8_t* occ_HL, uint8_t* occ_GL, void* stream, const SconeLaunchHints* hints, const float* cot) {
     SCONE_REQUIRE(cx && HL && wout && last_nodes && logprobs, "scone_readout: NULL argument");
     SCONE_REQUIRE(!cx->host_only, "scone_readout: index-only complex has no device arrays");
     SCONE_REQUIRE(C >= 1 && C <= 32 * kReadoutMaxCper, "scone_readout: C must be in [1,%d]", 32 * kReadoutMaxCper);
@@ -1745,7 +1765,7 @@ int scone_readout_ws(const scone_complex* cx, int32_t act, int32_t b, int32_t C,
     ScopedProf prof(SCONE_K_READOUT, st);
     const SconeLaunchHints h = hints ? *hints : SconeLaunchHints{};
     if (GL) {
-        SCONE_REQUIRE(target_idx && mask && workspace, "scone_readout: gradient mode needs target_idx, mask, workspace");
+        SCONE_REQUIRE((cot || (target_idx && mask)) && workspace, "scone_readout: gradient mode needs target_idx, mask, workspace");
         // GL is a complete dense array unless the caller reads its flagged rows only (skip_fill)
         const bool flagged = occ_GL != nullptr || h.out_bm != nullptr;
         if ((!flagged || zero_fill_here(&h)) && scone_zero_fill(cx, GL, (size_t)cx->E * b * C * sizeof(float), st)) return 1;
@@ -1756,9 +1776,14 @@ int scone_readout_ws(const scone_complex* cx, int32_t act, int32_t b, int32_t C,
     uint32_t* bm = (GL && (occ_GL || bm_HL)) ? h.out_bm : nullptr;
     if (bm) SCONE_CUDA(cudaMemsetAsync(bm, 0, scone_bitmap_words(cx->E, b) * 4, st));
     if (bm_cand) SCONE_CUDA(cudaMemsetAsync(bm_cand, 0, scone_bitmap_words(cx->E, b) * 4, st));
-    readout_kernel<<<b, 32 * kReadoutWarps, 0, st>>>(HL, wout, last_nodes, cx->d_nbrhoods, cx->d_inc_ptr, cx->d_inc_ent, logprobs,
-                                              target_idx, mask, scale, GL, (float*)workspace, occ_HL, GL ? occ_GL : nullptr, bm, act,
-                                              cx->N, cx->D, b, C, bm_HL, bm_cand, cx->d_mptr, cx->d_ment);
+    if (GL && cot)
+        readout_kernel<true><<<b, 32 * kReadoutWarps, 0, st>>>(HL, wout, last_nodes, cx->d_nbrhoods, cx->d_inc_ptr, cx->d_inc_ent, logprobs,
+                                                         nullptr, nullptr, scale, GL, (float*)workspace, occ_HL, occ_GL, bm, act, cx->N,
+                                                         cx->D, b, C, bm_HL, bm_cand, cx->d_mptr, cx->d_ment, cot);
+    else
+        readout_kernel<false><<<b, 32 * kReadoutWarps, 0, st>>>(HL, wout, last_nodes, cx->d_nbrhoods, cx->d_inc_ptr, cx->d_inc_ent, logprobs,
+                                                          target_idx, mask, scale, GL, (float*)workspace, occ_HL, GL ? occ_GL : nullptr, bm,
+                                                          act, cx->N, cx->D, b, C, bm_HL, bm_cand, cx->d_mptr, cx->d_ment, nullptr);
     SCONE_LAUNCHED();
     if (GL) {
         readout_reduce_kernel<<<1, ((C + 2 + 31) / 32) * 32, 0, st>>>((const float*)workspace, b, C, dwout, nll_sum, count, accumulate);
@@ -1775,6 +1800,14 @@ extern "C" int scone_readout(const scone_complex* cx, int32_t act, int32_t b, in
                              const uint8_t* occ_HL, uint8_t* occ_GL, void* stream) {
     return scone_readout_ws(cx, act, b, C, HL, wout, last_nodes, logprobs, target_idx, mask, scale, GL, dwout, nll_sum, count,
                             accumulate, workspace, occ_HL, occ_GL, stream, nullptr);
+}
+
+__global__ void add_scalar_kernel(float* __restrict__ dst, float v) { *dst += v; }
+
+int scone_add_scalar_launch(float* dst, float v, cudaStream_t st) {
+    add_scalar_kernel<<<1, 1, 0, st>>>(dst, v);
+    SCONE_LAUNCHED();
+    return 0;
 }
 
 int scone_adam_launch(float* W, float* m, float* v, const float* gradbuf, int64_t n, int32_t step, float lr, float wd, void* stream,

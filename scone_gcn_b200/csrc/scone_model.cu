@@ -59,7 +59,8 @@ struct scone_model {
     // staging for the *_host entry points
     int32_t *d_ptr = nullptr, *d_edge = nullptr, *d_last = nullptr, *d_tgt = nullptr, *d_nn = nullptr, *d_acc = nullptr;
     float *d_val = nullptr, *d_mask = nullptr, *d_logp_all = nullptr;
-    int64_t cap_B = 0, cap_nnz = 0;
+    float* d_cot = nullptr;                   // [cap_B][D] cotangents of the *_vjp_*_host entry points (allocated on first use)
+    int64_t cap_B = 0, cap_nnz = 0, cap_cot = 0;
     int32_t *d_choice = nullptr, *d_rand = nullptr;   // evaluation: predictions, random other targets
     float* d_evalf = nullptr;
     int64_t cap_choice = 0;
@@ -90,6 +91,21 @@ int ensure_staging(scone_model* m, int64_t B, int64_t nnz) {
         SCONE_CUDA(cudaMalloc((void**)&m->d_val, cap * sizeof(float)));
         m->cap_nnz = cap;
     }
+    return 0;
+}
+
+// Copies the [B][D] cotangents of a *_vjp_*_host entry point to the device staging buffer on s.
+int stage_cot(scone_model* m, int32_t B, const float* cot, cudaStream_t s) {
+    const size_t n = (size_t)B * m->cx->D;
+    if ((int64_t)n > m->cap_cot) {
+        cudaFree(m->d_cot);
+        m->d_cot = nullptr;
+        m->cap_cot = 0;
+        const size_t cap = n + n / 4 + 16;
+        SCONE_CUDA(cudaMalloc((void**)&m->d_cot, cap * sizeof(float)));
+        m->cap_cot = (int64_t)cap;
+    }
+    if (n) SCONE_CUDA(cudaMemcpyAsync(m->d_cot, cot, n * sizeof(float), cudaMemcpyHostToDevice, s));
     return 0;
 }
 
@@ -179,9 +195,10 @@ int backward_mb(scone_model* m, int32_t b, void* st) {
     return 0;
 }
 
-// pipeline 0 over one micro-batch [off, off+b) (ptr / last / tgt / mask: at off); grad = false: log-probs only
+// pipeline 0 over one micro-batch [off, off+b) (ptr / last / tgt / mask / cot: at off); grad = false: log-probs only; cot != NULL:
+// the gradient is seeded with the cotangent rows instead of tgt / mask
 int unit_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last, float* logprobs,
-            const int32_t* tgt, const float* mask, bool grad, cudaStream_t s) {
+            const int32_t* tgt, const float* mask, const float* cot, bool grad, cudaStream_t s) {
     const int L = m->L, CL = m->hidden[L - 1];
     const float* wout = m->d_w + m->w_off[3 * L];
     m->x_clean = false;
@@ -194,7 +211,7 @@ int unit_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, 
     h.skip_fill = true;
     h.out_bm = m->d_bmG;
     rc = scone_readout_ws(m->cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, tgt, mask, 1.f, m->d_G[L - 1], m->d_grad + m->w_off[3 * L],
-                          m->d_grad + m->n_params, m->d_grad + m->n_params + 1, 1, m->d_ws, m->d_occH[L - 1], m->d_occG[L - 1], s, &h);
+                          m->d_grad + m->n_params, m->d_grad + m->n_params + 1, 1, m->d_ws, m->d_occH[L - 1], m->d_occG[L - 1], s, &h, cot);
     return rc ? rc : backward_mb(m, b, s);
 }
 
@@ -341,7 +358,7 @@ int rows_clear_x(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* e
 
 // readout on the row-list pipelines; grad = false: log-probs only
 int rows_readout(scone_model* m, int32_t b, const int32_t* last, float* logprobs, bool grad, const int32_t* tgt, const float* mask,
-                 cudaStream_t s) {
+                 const float* cot, cudaStream_t s) {
     const scone_complex* cx = m->cx;
     const int L = m->L, CL = m->hidden[L - 1];
     const float* wout = m->d_w + m->w_off[3 * L];
@@ -355,7 +372,7 @@ int rows_readout(scone_model* m, int32_t b, const int32_t* last, float* logprobs
             h.cand_bm = L >= 2 ? m->d_bmGr[L - 2] : nullptr;
             return scone_readout_ws(cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, tgt, mask, 1.f, m->d_G[L - 1],
                                     m->d_grad + m->w_off[3 * L], m->d_grad + m->n_params, m->d_grad + m->n_params + 1, 1, m->d_ws, nullptr,
-                                    nullptr, s, &h);
+                                    nullptr, s, &h, cot);
         }
         return scone_readout_ws(cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, nullptr, nullptr, 0.f, nullptr, nullptr, nullptr,
                                 nullptr, 0, nullptr, nullptr, nullptr, s, &h);
@@ -376,7 +393,7 @@ int rows_readout(scone_model* m, int32_t b, const int32_t* last, float* logprobs
     return scone_rows_readout_backward(cx, m->act, b, CL, m->d_cH[L - 1], wout, last, logprobs, tgt, mask, 1.f, m->d_cG[L - 1], m->d_nrows,
                                        m->row_cap, m->d_overflow, m->d_grad + m->w_off[3 * L], m->d_grad + m->n_params,
                                        m->d_grad + m->n_params + 1, 1, (float*)m->d_ws, m->d_bmH[L - 1], m->d_prefH[L - 1], bmG,
-                                       m->d_prefG[L - 1], s);
+                                       m->d_prefG[L - 1], s, cot);
 }
 
 int rows_backward_mb(scone_model* m, int32_t b, cudaStream_t s) {
@@ -411,9 +428,9 @@ int rows_backward_mb(scone_model* m, int32_t b, cudaStream_t s) {
 
 // pipelines 1 / 2 over one micro-batch (arguments as unit_mb)
 int rows_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last, float* logprobs,
-            const int32_t* tgt, const float* mask, bool grad, cudaStream_t s) {
+            const int32_t* tgt, const float* mask, const float* cot, bool grad, cudaStream_t s) {
     int rc = rows_forward_mb(m, b, ptr, edge, val, s);
-    if (!rc) rc = rows_readout(m, b, last, logprobs, grad, tgt, mask, s);
+    if (!rc) rc = rows_readout(m, b, last, logprobs, grad, tgt, mask, cot, s);
     if (!rc && grad) rc = rows_backward_mb(m, b, s);
     if (!rc) rc = rows_clear_x(m, b, ptr, edge, val, s);
     return rc;
@@ -493,7 +510,7 @@ int cone_forward_mb(scone_model* m, int32_t b, cudaStream_t s) {
 }
 
 int cone_readout(scone_model* m, int32_t b, const int32_t* last, float* logprobs, bool grad, const int32_t* tgt, const float* mask,
-                 cudaStream_t s) {
+                 const float* cot, cudaStream_t s) {
     const scone_complex* cx = m->cx;
     const int L = m->L, CL = m->hidden[L - 1];
     const float* wout = m->d_w + m->w_off[3 * L];
@@ -504,7 +521,7 @@ int cone_readout(scone_model* m, int32_t b, const int32_t* last, float* logprobs
     return scone_rows_readout_backward(cx, m->act, b, CL, m->d_cH[L - 1], wout, last, logprobs, tgt, mask, 1.f, m->d_cG[L - 1],
                                        cone_n(m, L - 1), m->row_cap, m->d_overflow, m->d_grad + m->w_off[3 * L], m->d_grad + m->n_params,
                                        m->d_grad + m->n_params + 1, 1, (float*)m->d_ws, m->d_bmGr[L - 1], m->d_prefG[L - 1],
-                                       m->d_bmGr[L - 1], m->d_prefG[L - 1], s);
+                                       m->d_bmGr[L - 1], m->d_prefG[L - 1], s, cot);
 }
 
 int cone_backward_mb(scone_model* m, int32_t b, cudaStream_t s) {
@@ -528,10 +545,10 @@ int cone_backward_mb(scone_model* m, int32_t b, cudaStream_t s) {
 
 // pipeline 3 over one micro-batch (arguments as unit_mb)
 int cone_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last, float* logprobs,
-            const int32_t* tgt, const float* mask, bool grad, cudaStream_t s) {
+            const int32_t* tgt, const float* mask, const float* cot, bool grad, cudaStream_t s) {
     int rc = cone_build_mb(m, b, ptr, edge, val, last, s);
     if (!rc) rc = cone_forward_mb(m, b, s);
-    if (!rc) rc = cone_readout(m, b, last, logprobs, grad, tgt, mask, s);
+    if (!rc) rc = cone_readout(m, b, last, logprobs, grad, tgt, mask, cot, s);
     if (!rc && grad) rc = cone_backward_mb(m, b, s);
     if (!rc) rc = rows_clear_x(m, b, ptr, edge, val, s);
     if (!rc) rc = cone_clear_mb(m, b, s);
@@ -670,7 +687,7 @@ extern "C" int scone_model_destroy(scone_model* m) {
     if (m->ev_plan_done) cudaEventDestroy(m->ev_plan_done);
     for (auto e : m->ev_part) if (e) cudaEventDestroy(e);
     cudaFree(m->d_ptr); cudaFree(m->d_edge); cudaFree(m->d_last); cudaFree(m->d_tgt); cudaFree(m->d_val);
-    cudaFree(m->d_mask); cudaFree(m->d_logp_all); cudaFree(m->d_nn); cudaFree(m->d_acc);
+    cudaFree(m->d_mask); cudaFree(m->d_logp_all); cudaFree(m->d_nn); cudaFree(m->d_acc); cudaFree(m->d_cot);
     cudaFree(m->d_choice); cudaFree(m->d_rand); cudaFree(m->d_evalf);
     delete m;
     return 0;
@@ -740,13 +757,14 @@ static int finish_call(scone_model* m, int rc, void* user_st) {
 
 // pipeline 4: the micro-batch is walked in chunks the program arena was sized for (scone_fused_create)
 static int fused_call(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last,
-                      float* logprobs, const int32_t* tgt, const float* mask, bool grad, cudaStream_t s) {
+                      float* logprobs, const int32_t* tgt, const float* mask, const float* cot, bool grad, cudaStream_t s) {
     const int step = m->fused->chunk < m->mb ? m->fused->chunk : m->mb;
     for (int32_t off = 0; off < B; off += step) {
         const int32_t b = B - off < step ? B - off : step;
         int rc = scone_fused_run(m->cx, m->fused, m->act, b, ptr + off, edge, val, last + off, m->d_w, m->w_off.data(),
-                                 logprobs ? logprobs + (size_t)off * m->cx->D : nullptr, grad ? tgt + off : nullptr,
-                                 grad ? mask + off : nullptr, grad ? m->d_grad : nullptr, m->d_overflow, g_scone_prof, s);
+                                 logprobs ? logprobs + (size_t)off * m->cx->D : nullptr, grad && !cot ? tgt + off : nullptr,
+                                 grad && !cot ? mask + off : nullptr, grad ? m->d_grad : nullptr, m->d_overflow, g_scone_prof, s,
+                                 grad && cot ? cot + (size_t)off * m->cx->D : nullptr);
         if (rc) return rc;
     }
     return 0;
@@ -759,8 +777,9 @@ static bool fused_host_overlap_ok(const scone_model* m, int32_t B, int64_t nnz) 
     return m->pipeline == 4 && m->fused && B >= 512 && B <= m->fused->chunk && B <= m->mb && nnz >= (1 << 13);
 }
 
+// cot_dev != NULL (grad): the VJP seeded with these staged cotangents; count_add is added to the count slot.
 static int fused_host_overlapped(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, float* logprobs_dev,
-                                 bool grad, int32_t zero_first, cudaStream_t s) {
+                                 bool grad, int32_t zero_first, cudaStream_t s, const float* cot_dev = nullptr, float count_add = 0.f) {
     // parts of >= 4096 trajectories, at most 4: a part's first plan tier runs as soon as its flows have landed; the later tiers (a few
     // heavy trajectories, each launch as long as its slowest one) run once over all parts.  Small batches are planned in one piece
     // (their copy is short, and steps enqueued back to back copy under the previous compute)
@@ -795,6 +814,7 @@ static int fused_host_overlapped(scone_model* m, int32_t B, const int32_t* ptr, 
     if (fork_to_compute(m, (void*)s)) return 1;
     cudaStream_t c = m->compute;
     if (grad && zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * sizeof(float), c));
+    if (grad && cot_dev && count_add != 0.f && scone_add_scalar_launch(m->d_grad + m->n_params + 1, count_add, c)) return finish_call(m, 1, (void*)s);
     int rc = scone_fused_begin(m->fused, c);
     for (int k = 0; k < kParts && !rc; ++k) {
         SCONE_CUDA(cudaStreamWaitEvent(c, m->ev_part[k], 0));
@@ -809,25 +829,30 @@ static int fused_host_overlapped(scone_model* m, int32_t B, const int32_t* ptr, 
         m->plan_done_epoch = -1;
     }
     if (!rc)
-        rc = scone_fused_compute(m->cx, m->fused, m->act, B, m->d_w, m->w_off.data(), logprobs_dev, grad ? m->d_tgt : nullptr,
-                                 grad ? m->d_mask : nullptr, grad ? m->d_grad : nullptr, g_scone_prof, c);
+        rc = scone_fused_compute(m->cx, m->fused, m->act, B, m->d_w, m->w_off.data(), logprobs_dev, grad && !cot_dev ? m->d_tgt : nullptr,
+                                 grad && !cot_dev ? m->d_mask : nullptr, grad ? m->d_grad : nullptr, g_scone_prof, c, grad ? cot_dev : nullptr);
     return finish_call(m, rc, (void*)s);
 }
 
-// Forward (grad = false: log-probs to logprobs [B][D]) or loss + gradient (grad = true: into d_grad, cleared first if zero_first)
+// Forward (grad = false: log-probs to logprobs [B][D]) or loss + gradient (grad = true: into d_grad, cleared first if zero_first).
+// cot != NULL (grad): the VJP — the gradient is seeded with the cotangent rows [B][D] instead of tgt / mask, and count_add is added to
+// the count slot.
 static int run_batch(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last,
-                     float* logprobs, const int32_t* tgt, const float* mask, bool grad, int32_t zero_first, void* user_st) {
+                     float* logprobs, const int32_t* tgt, const float* mask, bool grad, int32_t zero_first, void* user_st,
+                     const float* cot = nullptr, float count_add = 0.f) {
     if (fork_to_compute(m, user_st)) return 1;
     cudaStream_t s = m->compute;
     if (grad && zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * sizeof(float), s));
+    if (grad && cot && count_add != 0.f && scone_add_scalar_launch(m->d_grad + m->n_params + 1, count_add, s)) return finish_call(m, 1, user_st);
     const int pl = m->pipeline;
-    if (pl == 4) return finish_call(m, fused_call(m, B, ptr, edge, val, last, logprobs, tgt, mask, grad, s), user_st);
+    if (pl == 4) return finish_call(m, fused_call(m, B, ptr, edge, val, last, logprobs, tgt, mask, cot, grad, s), user_st);
     auto step = pl == 3 ? cone_mb : pl >= 1 ? rows_mb : unit_mb;
     int rc = 0;
     for (int32_t off = 0; off < B && !rc; off += m->mb) {
         const int32_t b = B - off < m->mb ? B - off : m->mb;
-        rc = step(m, b, ptr + off, edge, val, last + off, grad ? m->d_logp : logprobs + (size_t)off * m->cx->D, grad ? tgt + off : nullptr,
-                  grad ? mask + off : nullptr, grad, s);
+        rc = step(m, b, ptr + off, edge, val, last + off, grad ? m->d_logp : logprobs + (size_t)off * m->cx->D,
+                  grad && !cot ? tgt + off : nullptr, grad && !cot ? mask + off : nullptr, grad && cot ? cot + (size_t)off * m->cx->D : nullptr,
+                  grad, s);
     }
     return finish_call(m, rc, user_st);
 }
@@ -961,6 +986,26 @@ extern "C" int scone_model_loss_grad_host(scone_model* m, int32_t B, const int32
     return scone_model_loss_grad_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, m->d_tgt, m->d_mask, zero_first, st);
 }
 
+extern "C" int scone_model_vjp_dev(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last,
+                                   const float* cot, float count_add, int32_t zero_first, void* user_st) {
+    SCONE_REQUIRE(m && ptr && last && B >= 0, "scone_model_vjp_dev: bad arguments");
+    SCONE_REQUIRE(cot || B == 0, "scone_model_vjp_dev: cot is NULL");
+    return run_batch(m, B, ptr, edge, val, last, nullptr, nullptr, nullptr, true, zero_first, user_st, cot, count_add);
+}
+
+extern "C" int scone_model_vjp_host(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last,
+                                    const float* cot, float count_add, int32_t zero_first, void* st) {
+    SCONE_REQUIRE(m && ptr && last && B >= 0, "scone_model_vjp_host: bad arguments");
+    SCONE_REQUIRE(cot || B == 0, "scone_model_vjp_host: cot is NULL");
+    cudaStream_t s = as_stream(st);
+    const bool overlap = fused_host_overlap_ok(m, B, B > 0 ? ptr[B] : 0);
+    int rc = stage_host_inputs(m, B, ptr, last, nullptr, nullptr, nullptr, edge, val, !overlap, s);
+    if (!rc) rc = stage_cot(m, B, cot, s);
+    if (rc) return rc;
+    if (overlap) return fused_host_overlapped(m, B, ptr, edge, val, nullptr, true, zero_first, s, m->d_cot, count_add);
+    return scone_model_vjp_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, B > 0 ? m->d_cot : nullptr, count_add, zero_first, st);
+}
+
 extern "C" int scone_model_read_grads_async(scone_model* m, float* out_pinned, void* st) {
     SCONE_REQUIRE(m && out_pinned, "scone_model_read_grads_async: NULL argument");
     SCONE_CUDA(cudaMemcpyAsync(out_pinned, m->d_grad, (m->n_params + 2) * sizeof(float), cudaMemcpyDeviceToHost, as_stream(st)));
@@ -1020,6 +1065,34 @@ extern "C" int scone_model_loss_grad_planned_host(scone_model* m, int32_t n, con
         SCONE_CUDA(cudaMemcpyAsync(m->d_mask, mask, n * sizeof(float), cudaMemcpyHostToDevice, s));
     }
     return scone_model_loss_grad_planned_dev(m, n, rows ? m->d_nn : nullptr, m->d_tgt, m->d_mask, zero_first, st);
+}
+
+extern "C" int scone_model_vjp_planned_dev(scone_model* m, int32_t n, const int32_t* rows_dev, const float* cot_dev, float count_add,
+                                           int32_t zero_first, void* user_st) {
+    SCONE_REQUIRE(m && n >= 0, "scone_model_vjp_planned_dev: bad arguments");
+    SCONE_REQUIRE(cot_dev || n == 0, "scone_model_vjp_planned_dev: cot is NULL");
+    SCONE_REQUIRE(m->fused != nullptr, "scone_model_vjp_planned_dev: no fused pipeline");
+    if (fork_to_compute(m, user_st)) return 1;
+    cudaStream_t s = m->compute;
+    if (zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * sizeof(float), s));
+    int rc = count_add != 0.f ? scone_add_scalar_launch(m->d_grad + m->n_params + 1, count_add, s) : 0;
+    if (!rc)
+        rc = scone_fused_run_planned(m->cx, m->fused, m->act, n, rows_dev, m->d_w, m->w_off.data(), nullptr, nullptr, nullptr, m->d_grad,
+                                     g_scone_prof, s, cot_dev);
+    return finish_call(m, rc, user_st);
+}
+
+extern "C" int scone_model_vjp_planned_host(scone_model* m, int32_t n, const int32_t* rows, const float* cot, float count_add,
+                                            int32_t zero_first, void* st) {
+    SCONE_REQUIRE(m && n >= 0, "scone_model_vjp_planned_host: bad arguments");
+    SCONE_REQUIRE(cot || n == 0, "scone_model_vjp_planned_host: cot is NULL");
+    SCONE_REQUIRE(m->fused != nullptr, "scone_model_vjp_planned_host: no fused pipeline");
+    cudaStream_t s = as_stream(st);
+    int rc = ensure_staging(m, n, 0);
+    if (!rc) rc = stage_cot(m, n, cot, s);
+    if (rc) return rc;
+    if (n && rows) SCONE_CUDA(cudaMemcpyAsync(m->d_nn, rows, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    return scone_model_vjp_planned_dev(m, n, rows ? m->d_nn : nullptr, n ? m->d_cot : nullptr, count_add, zero_first, st);
 }
 
 extern "C" int scone_model_forward_planned_host(scone_model* m, int32_t n, const int32_t* rows, float* logprobs_out, void* st) {

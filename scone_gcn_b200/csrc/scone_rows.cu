@@ -780,7 +780,8 @@ __global__ void __launch_bounds__(256) rows_reduce_kernel(const float* __restric
 //                             of the rows of G_L this trajectory touches and the candidate bits one hop further
 //   rows_readout_bwd_kernel   dl_j = mask * scale * (exp(logp_j) - [j == y]); adds s(e, nbr_j) * dl_j * w * act'(h) onto row rank(e, t)
 //                             of the zeroed compact G_L (at most two contributions per row: a + b == b + a, deterministic), the
-//                             w_out gradient partials, the NLL term and the mask count.
+//                             w_out gradient partials, the NLL term and the mask count.  COT (cotangent seed, scone_model_vjp_*):
+//                             dl_j = cot_j - p_j * sum_k cot_k over ALL D slots, NLL term sum_j cot_j * logp_j, count 0
 // One CTA (4 warps) per trajectory, warps split the neighbour slots (same arithmetic as readout_kernel).
 // ---------------------------------------------------------------------------------------------------------------
 
@@ -915,6 +916,7 @@ __global__ void __launch_bounds__(256) rows_zero_kernel(float4* __restrict__ T, 
         T[i] = make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
+template <bool COT>
 __global__ void __launch_bounds__(32 * kRoWarps) rows_readout_bwd_kernel(const float* __restrict__ HL, const float* __restrict__ wout,
                                                                         const int32_t* __restrict__ last_nodes, const int32_t* __restrict__ nbrhoods,
                                                                         const int32_t* __restrict__ inc_ptr, const int2* __restrict__ inc_ent,
@@ -922,8 +924,10 @@ __global__ void __launch_bounds__(32 * kRoWarps) rows_readout_bwd_kernel(const f
                                                                         const float* __restrict__ mask, float scale, float* __restrict__ GL,
                                                                         float* __restrict__ partial /* [b][C+2] */, const uint32_t* __restrict__ bmH,
                                                                         const uint32_t* __restrict__ prefH, const uint32_t* __restrict__ bmG,
-                                                                        const uint32_t* __restrict__ prefG, int g_cap, int act, int N, int D, int E, int C) {
+                                                                        const uint32_t* __restrict__ prefG, int g_cap, int act, int N, int D, int E, int C,
+                                                                        const float* __restrict__ cot /* [b][D], COT */) {
     __shared__ float s_dw[kRoWarps][32 * kRoMaxCper];
+    __shared__ float s_cot[COT ? kRoMaxD : 1], s_csum, s_ell;
     __shared__ RoPairs pairs;
     __shared__ RoItem items[kRoItems];
     const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
@@ -948,16 +952,35 @@ __global__ void __launch_bounds__(32 * kRoWarps) rows_readout_bwd_kernel(const f
         return it;
     };
     for (int i = threadIdx.x; i < total && i < kRoItems; i += blockDim.x) items[i] = resolve(i, pairs.slot_of(i));
+    if (COT && warp == 0) {                                // the cotangent row, its sum and sum_j cot_j * logp_j (fixed order)
+        float cs = 0.f, el = 0.f;
+        for (int j = lane; j < D; j += 32) {
+            const float c = cot[(size_t)t * D + j];
+            s_cot[j] = c;
+            cs += c;
+            el = fmaf(c, logprobs[(size_t)t * D + j], el);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            cs += __shfl_xor_sync(0xffffffffu, cs, o);
+            el += __shfl_xor_sync(0xffffffffu, el, o);
+        }
+        if (lane == 0) {
+            s_csum = cs;
+            s_ell = el;
+        }
+    }
     __syncthreads();
     float w[kRoMaxCper];
 #pragma unroll
     for (int q = 0; q < kRoMaxCper; ++q) w[q] = (lane + 32 * q < C) ? wout[lane + 32 * q] : 0.f;
-    const float mk = mask[t];
-    const int y = target_idx[t];
+    const float mk = COT ? 0.f : mask[t];
+    const int y = COT ? -1 : target_idx[t];
     float dwl[kRoMaxCper] = {0.f, 0.f, 0.f, 0.f};
     for (int j = warp; j < D; j += kRoWarps) {
         if (pairs.s_ptr[j] < 0) continue;
-        const float dl = mk * scale * (expf(logprobs[(size_t)t * D + j]) - (j == y ? 1.f : 0.f));
+        const float dl = COT ? s_cot[j] - expf(logprobs[(size_t)t * D + j]) * s_csum
+                             : mk * scale * (expf(logprobs[(size_t)t * D + j]) - (j == y ? 1.f : 0.f));
         const int i1 = pairs.s_off[j + 1];
         for (int i0 = pairs.s_off[j]; i0 < i1; i0 += 4) {
             RoItem it[4];
@@ -1000,7 +1023,7 @@ __global__ void __launch_bounds__(32 * kRoWarps) rows_readout_bwd_kernel(const f
                 pt[lane + 32 * q] = sacc;
             }
         if (lane == 0) {
-            pt[C] = (y >= 0 && y < D) ? -mk * logprobs[(size_t)t * D + y] : 0.f;
+            pt[C] = COT ? s_ell : ((y >= 0 && y < D) ? -mk * logprobs[(size_t)t * D + y] : 0.f);
             pt[C + 1] = mk;
         }
     }
@@ -1407,11 +1430,17 @@ int scone_rows_readout_backward(const scone_complex* cx, int act, int b, int C, 
                                 const int32_t* last_nodes, const float* logprobs, const int32_t* target_idx, const float* mask,
                                 float scale, float* GL, const int* n_dev, int g_cap, int* overflow_dev, float* dwout, float* nll_sum,
                                 float* count, int accumulate, float* ws, const uint32_t* bmH, const uint32_t* prefH, const uint32_t* bmG,
-                                const uint32_t* prefG, cudaStream_t st) {
+                                const uint32_t* prefG, cudaStream_t st, const float* cot) {
     rows_zero_kernel<<<cx->num_sms * 4, 256, 0, st>>>(reinterpret_cast<float4*>(GL), n_dev, g_cap, C / 4, overflow_dev);
     SCONE_LAUNCHED();
-    rows_readout_bwd_kernel<<<b, 32 * kRoWarps, 0, st>>>(HL, wout, last_nodes, cx->d_nbrhoods, cx->d_inc_ptr, cx->d_inc_ent, logprobs, target_idx,
-                                                        mask, scale, GL, ws, bmH, prefH, bmG, prefG, g_cap, act, cx->N, cx->D, cx->E, C);
+    if (cot)
+        rows_readout_bwd_kernel<true><<<b, 32 * kRoWarps, 0, st>>>(HL, wout, last_nodes, cx->d_nbrhoods, cx->d_inc_ptr, cx->d_inc_ent, logprobs,
+                                                                  nullptr, nullptr, scale, GL, ws, bmH, prefH, bmG, prefG, g_cap, act, cx->N,
+                                                                  cx->D, cx->E, C, cot);
+    else
+        rows_readout_bwd_kernel<false><<<b, 32 * kRoWarps, 0, st>>>(HL, wout, last_nodes, cx->d_nbrhoods, cx->d_inc_ptr, cx->d_inc_ent, logprobs,
+                                                                   target_idx, mask, scale, GL, ws, bmH, prefH, bmG, prefG, g_cap, act, cx->N,
+                                                                   cx->D, cx->E, C, nullptr);
     SCONE_LAUNCHED();
     rows_readout_reduce_kernel<<<(C + 2 + 7) / 8, 256, 0, st>>>(ws, b, C, dwout, nll_sum, count, accumulate);
     SCONE_LAUNCHED();

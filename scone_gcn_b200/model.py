@@ -113,6 +113,17 @@ class SconeModel:
                    'scone_model_loss_grad_host')
         return self.read_grads(stream) if read else None
 
+    def vjp(self, traj_ptr, flow_edge, flow_val, last_nodes, cot, count_add, zero_first=True, stream=None, read=True):
+        """VJP of the log-probs from HOST inputs: grads += sum cot * dlogprob/dW, nll_sum += sum cot * logprob, count += count_add, in the
+        loss_grad buffer [grads | nll_sum | count]; cot [B, D] = dL/dlogprob.  Optionally read it back."""
+        B = len(last_nodes)
+        a = [np.ascontiguousarray(traj_ptr, np.int32), np.ascontiguousarray(flow_edge, np.int32),
+             np.ascontiguousarray(flow_val, np.float32), np.ascontiguousarray(last_nodes, np.int32),
+             np.ascontiguousarray(cot, np.float32).reshape(B, self.cx.D)]
+        _lib.check(_lib.lib().scone_model_vjp_host(self.handle, B, *[_lib.ptr(x) for x in a], float(count_add), int(zero_first), stream),
+                   'scone_model_vjp_host')
+        return self.read_grads(stream) if read else None
+
     def accuracy(self, traj_ptr, flow_edge, flow_val, last_nodes, n_nbrs, target_idx, mask, stream=None):
         """(correct, counted) over the trajectories with mask != 0: forward + argmax on the device
         (scone_trajectory_model.py:59-71; slots >= n_nbrs count as -100, first maximum wins)."""
@@ -145,6 +156,15 @@ class SconeModel:
         t, k = np.ascontiguousarray(target_idx, np.int32), np.ascontiguousarray(mask, np.float32)
         _lib.check(_lib.lib().scone_model_loss_grad_planned_host(self.handle, n, _lib.ptr(r), _lib.ptr(t), _lib.ptr(k), int(zero_first), stream),
                    'scone_model_loss_grad_planned_host')
+        return self.read_grads(stream) if read else None
+
+    def vjp_planned(self, rows, cot, count_add, zero_first=True, stream=None, read=True):
+        """vjp over rows of the planned set (None = its first len(cot) trajectories); cot [n, D] by batch position."""
+        n = len(cot)
+        r = None if rows is None else np.ascontiguousarray(rows, np.int32)
+        c = np.ascontiguousarray(cot, np.float32).reshape(n, self.cx.D)
+        _lib.check(_lib.lib().scone_model_vjp_planned_host(self.handle, n, _lib.ptr(r), _lib.ptr(c), float(count_add), int(zero_first), stream),
+                   'scone_model_vjp_planned_host')
         return self.read_grads(stream) if read else None
 
     def forward_planned(self, rows=None, n=None, stream=None):

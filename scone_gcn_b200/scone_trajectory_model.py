@@ -5,7 +5,8 @@ Same constructor, methods, argument meaning, printed lines and NumPy RNG stream 
 
   reference                                              here
   self.model = vmap(model, in_axes)            :256  ->  batched op over device-resident index arrays
-  grad(self.loss)(weights, inputs, y, mask)    :307  ->  SconeModel.loss_grad (fused fwd+bwd kernels)
+  grad(self.loss)(weights, inputs, y, mask)    :307  ->  SconeModel.loss_grad (fused fwd+bwd kernels); a y that is not
+                                                         one-hot: SconeModel.vjp with cot = -mask * y
   adam(step_size) init/update/get_params       :300  ->  SconeModel.adam_step (device Adam state)
 
 Differences that are deliberate and results-identical:
@@ -302,6 +303,10 @@ class Scone_GCN():
         n_batches = n_train_samples // self.batch_size
         yv = onp.asarray(y)
         target_idx = onp.argmax(yv.reshape(N, -1), axis=1).astype(onp.int32)
+        # a soft target (not one-hot) is trained through the VJP of the log-probs with cot = -mask * y, the gradient of
+        # -sum(preds * y) that jax.grad takes at :307; one-hot targets keep the loss_grad path
+        soft = not self._is_onehot(yv)
+        y_flat = onp.ascontiguousarray(yv.reshape(N, -1), onp.float32) if soft else None
 
         self._net.set_weights([onp.asarray(w) for w in self.weights], reset_adam=True)     # init_fun(self.weights)
         # the batches of every epoch are drawn from the same N trajectories: their plans (receptive cone, live rows, gather
@@ -332,7 +337,13 @@ class Scone_GCN():
             if use_dp:                                     # this rank's contiguous share of the batch (same rows on every rank)
                 keep = dp.shard_rows(onp.arange(len(rows)))
                 rows, m = rows[keep], m[keep]
-            if planned:
+            if soft:
+                cot = -m[:, None] * y_flat[rows]
+                if planned:
+                    self._net.vjp_planned(rows, cot, m.sum(), zero_first=True, read=False)
+                else:
+                    self._net.vjp(*p.select(rows), cot, m.sum(), zero_first=True, read=False)
+            elif planned:
                 self._net.loss_grad_planned(rows, target_idx[rows], m, zero_first=True, read=False)
             else:
                 ptr, fe, fv, last = p.select(rows)
