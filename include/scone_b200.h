@@ -105,7 +105,8 @@ int scone_layer_forward(const scone_complex* cx, int32_t act, int32_t b, int32_t
 /* Backward of the same layer (what jax.grad derives from the lines above, scone_trajectory_model.py:307).
  * G_dev = dL/dZ of this layer ( = dL/dHout * act'(Hout), already multiplied) [E][b][cout].
  * Outputs:  Gprev_dev [E][b][cin] = dL/dZ of the previous layer = (dL/dHin) * act'(Hin)
- *           (pass NULL for the first layer: the reference never differentiates w.r.t. the flows);
+ *           (pass NULL for the first layer: this call has no input gradient there; the model-level
+ *           scone_model_vjp_flows_* return dL/dflow_val);
  *           dW_dev [3][cin][cout] += sum over rows, reduced in a fixed order (deterministic, no atomics).
  * workspace: scone_layer_backward_workspace_bytes(cin, cout) bytes, device. */
 int64_t scone_layer_backward_workspace_bytes(int32_t cin, int32_t cout);
@@ -214,6 +215,23 @@ int scone_model_vjp_dev(scone_model* m, int32_t B, const int32_t* traj_ptr_dev, 
                         void* stream);
 int scone_model_vjp_host(scone_model* m, int32_t B, const int32_t* traj_ptr, const int32_t* flow_edge, const float* flow_val,
                          const int32_t* last_nodes, const float* cot /* [B][D] */, float count_add, int32_t zero_first, void* stream);
+/* scone_model_vjp_* that also returns the gradient with respect to the flow values: the [grads | nll_sum | count] buffer is handled
+ * exactly as there, and for every p in [traj_ptr[0], traj_ptr[B])
+ *   dflow[p] = d(sum_t sum_j cot[t][j] * logprob[t][j]) / d flow_val[p]        (other elements of dflow are not touched)
+ * i.e. one transposed operator hop of the first layer's gradient G_1 without activation, dL/dX = G_1 w0^T + S0 (G_1 w1^T) + S1 (G_1 w2^T),
+ * read at the flow entries.  An entry whose edge id is out of range gets 0 (the forward ignores it); an entry outside the readout cone
+ * T_0 of its trajectory gets exactly 0; duplicate edge ids inside one trajectory are unspecified, as in the forward.  Every sum is
+ * taken in a fixed order (deterministic, no float atomics).  Pipeline 4 plans every flow entry of T_0 into layer-1 liveness whatever
+ * its value (the extra rows hold exact zeros: log-probs and weight gradients are unchanged) and computes dflow inside the compute
+ * kernel; pipelines 0-3 run one more kernel after the first layer's backward.  Same micro-batching and capacity-overflow flag as
+ * scone_model_vjp_* (while the flag is set dflow is invalid too).  cot == NULL or dflow == NULL with B > 0: error code 2, nothing
+ * launched.  _host: host pointers (dflow indexed like flow_val), the plain staged path; synchronises the stream before it returns. */
+int scone_model_vjp_flows_dev(scone_model* m, int32_t B, const int32_t* traj_ptr_dev, const int32_t* flow_edge_dev,
+                              const float* flow_val_dev, const int32_t* last_nodes_dev, const float* cot_dev /* [B][D] */,
+                              float count_add, int32_t zero_first, float* dflow_dev /* indexed like flow_val */, void* stream);
+int scone_model_vjp_flows_host(scone_model* m, int32_t B, const int32_t* traj_ptr, const int32_t* flow_edge, const float* flow_val,
+                               const int32_t* last_nodes, const float* cot /* [B][D] */, float count_add, int32_t zero_first,
+                               float* dflow /* host, indexed like flow_val */, void* stream);
 /* Next-node accuracy on the device (scone_trajectory_model.py:59-71): for every trajectory with mask != 0 the prediction is
  * argmax_j of (j < n_nbrs[t] ? logprobs[t][j] : -100) over ALL D slots — the first maximum wins, a NaN wins over numbers, as
  * NumPy / JAX argmax — compared with target_idx[t].  out[0] = correct predictions, out[1] = masked trajectories (integers:

@@ -75,6 +75,8 @@ SIGNATURES = {
     'scone_model_loss_grad_host': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp]),
     'scone_model_vjp_dev': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _i32, _vp]),
     'scone_model_vjp_host': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _i32, _vp]),
+    'scone_model_vjp_flows_dev': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _i32, _vp, _vp]),
+    'scone_model_vjp_flows_host': (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _i32, _vp, _vp]),
     'scone_model_vjp_planned_dev': (C.c_int, [_vp, _i32, _vp, _vp, _f32, _i32, _vp]),
     'scone_model_vjp_planned_host': (C.c_int, [_vp, _i32, _vp, _vp, _f32, _i32, _vp]),
     'scone_accuracy_dev': (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),

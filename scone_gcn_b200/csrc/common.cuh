@@ -165,6 +165,10 @@ int scone_rows_layer0_forward(const scone_complex* cx, int act, int b, int cout,
                               int* overflow_dev, cudaStream_t st);
 int scone_rows_layer0_backward(const scone_complex* cx, int b, int cout, const float* X, const float* G, const uint32_t* rows,
                                const int* n_dev, float* dW, int accumulate, float* ws, int g_cap, cudaStream_t st);
+// dL/dx at the flow entries from G_1 = G (dense rows with byte flags occ, dense rows with bitmap bm, or compact rows through bm + pref)
+int scone_rows_flow_grad(const scone_complex* cx, int b, const int32_t* traj_ptr, const int32_t* flow_edge, int C, const float* G,
+                         const uint8_t* occ, const uint32_t* bm, const uint32_t* pref, int cap, const float* w0, const float* w1,
+                         const float* w2, float* dflow, cudaStream_t st);
 int scone_rows_backward(const scone_complex* cx, int act, int b, int cin, int cout, const float* G, const float* Hin, float* Gprev,
                         float* Abuf, const float* W0, const float* W1, const float* W2, const uint32_t* rows, const int* n_dev,
                         const uint32_t* bmG, const uint32_t* bmH, int a_cap, int* overflow_dev, float* dW, int accumulate, float* ws,

@@ -52,6 +52,7 @@ struct PlanArgs {
     const int* in_list;
     int* n_retry;              // trajectories this tier gives up on (tables too small): device counter + list; retry == NULL: last tier,
     int* retry;                //   giving up = the overflow flag
+    unsigned* fg_off;          // flow-gradient plan (NULL: none): word offset of trajectory t's layer-0 transposed program (below)
 };
 
 #ifdef __CUDACC__
@@ -88,6 +89,56 @@ __device__ inline int fused_block_scan_excl(int* a, int n, int* s_warp) {
     if (tid == 0) a[n] = total;
     __syncthreads();
     return total;
+}
+
+// Layer-0 transposed program of a flow-gradient plan (both plan kernels; written at PlanArgs::fg_off[t]): row pointers [n_f + 1]
+// (relative to the first entry) then int2 entries {live layer-1 row | own << 31, (c1 << 16) | c0} in column order, the format of the
+// transposed programs of layers 2 / 3.  One row per flow entry of the trajectory in CSR order; an entry outside T_0 or with an edge id
+// out of range has an empty row.  row(i, emit) calls emit(entry) for the entries of flow entry i in column order.  The rows go
+// kFlowChunk at a time: one pass counts (the size of the arena piece), a second scans each chunk and writes it.  Returns the piece's
+// word offset, or ~0u when the arena is exhausted (block-uniform; every thread of the THREADS-thread CTA calls it).
+constexpr int kFlowChunk = 128;
+template <int THREADS, typename Row>
+__device__ unsigned fused_flow_program(const PlanArgs& a, int n_f, int* s_warp, Row row) {
+    static_assert(THREADS >= kFlowChunk, "a thread per row of a chunk");
+    __shared__ int s_c[kFlowChunk + 1];
+    __shared__ unsigned s_off;
+    const int tid = threadIdx.x;
+    auto count = [&](int i) {
+        int c = 0;
+        if (tid < kFlowChunk && i < n_f) row(i, [&](int2) { ++c; });
+        if (tid < kFlowChunk) s_c[tid] = c;
+    };
+    int total = 0;
+    for (int base = 0; base < n_f; base += kFlowChunk) {
+        count(base + tid);
+        total += fused_block_scan_excl<THREADS>(s_c, kFlowChunk, s_warp);
+    }
+    const int ptr_words = (n_f + 2) & ~1;
+    if (tid == 0) {
+        const unsigned long long w = (unsigned long long)ptr_words + 2ull * (unsigned long long)total;
+        const unsigned long long o = atomicAdd(a.bump, w);
+        s_off = o + w > a.arena_words ? ~0u : (unsigned)o;
+    }
+    __syncthreads();
+    const unsigned off = s_off;
+    if (off == ~0u) return off;
+    int* ptr = reinterpret_cast<int*>(a.arena + off);
+    int2* ent = reinterpret_cast<int2*>(a.arena + off + ptr_words);
+    int run = 0;
+    for (int base = 0; base < n_f; base += kFlowChunk) {
+        const int i = base + tid;
+        count(i);
+        const int chunk_total = fused_block_scan_excl<THREADS>(s_c, kFlowChunk, s_warp);
+        if (tid < kFlowChunk && i < n_f) {
+            int k = run + s_c[tid];
+            ptr[i] = k;
+            row(i, [&](int2 en) { ent[k++] = en; });
+        }
+        run += chunk_total;
+    }
+    if (tid == 0) ptr[n_f] = run;
+    return off;
 }
 #endif
 
@@ -134,6 +185,7 @@ struct FusedState {
     size_t sort_tmp_bytes = 0;
     int sort_cap = 0;
     // planned set (scone_fused_plan_set): headers + programs of a whole dataset, kept across calls
+    unsigned* d_fg_off = nullptr;         // [chunk] layer-0 transposed programs of a flow-gradient plan (allocated on first use)
     int* d_set_hdr = nullptr;
     uint32_t* d_set_arena = nullptr;
     unsigned long long* d_set_bump = nullptr;
@@ -152,16 +204,17 @@ void scone_fused_destroy(FusedState* f);
 int scone_fused_run(const scone_complex* cx, FusedState* f, int act, int b, const int32_t* traj_ptr, const int32_t* flow_edge,
                     const float* flow_val, const int32_t* last_nodes, const float* W, const int64_t* w_off, float* logprobs,
                     const int32_t* target_idx, const float* mask, float* grad, int* overflow, bool count_rows, cudaStream_t st,
-                    const float* cot = nullptr);   // cot [b][D] (with grad): cotangent seed instead of target_idx / mask
+                    const float* cot = nullptr,    // cot [b][D] (with grad): cotangent seed instead of target_idx / mask
+                    float* dflow = nullptr);       // (with cot) d(sum cot * logprob) / d flow_val, indexed like flow_val
 int scone_fused_begin(FusedState* f, cudaStream_t st);
 int scone_fused_plan_part(const scone_complex* cx, FusedState* f, int off, int b, const int32_t* traj_ptr, const int32_t* flow_edge,
                           const float* flow_val, const int32_t* last_nodes, int* overflow, cudaStream_t st,
-                          bool defer_tiers = false);
+                          bool defer_tiers = false, bool flow_grad = false);
 int scone_fused_plan_finish(const scone_complex* cx, FusedState* f, int B, const int32_t* traj_ptr, const int32_t* flow_edge,
                             const float* flow_val, const int32_t* last_nodes, int* overflow, cudaStream_t st);
 int scone_fused_compute(const scone_complex* cx, FusedState* f, int act, int b, const float* W, const int64_t* w_off, float* logprobs,
                         const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st,
-                        const float* cot = nullptr);
+                        const float* cot = nullptr, float* dflow = nullptr, const int32_t* traj_ptr = nullptr);
 int scone_fused_plan_set(const scone_complex* cx, FusedState* f, int B, const int32_t* traj_ptr, const int32_t* flow_edge,
                          const float* flow_val, const int32_t* last_nodes, int* overflow, cudaStream_t st);
 int scone_fused_run_planned(const scone_complex* cx, FusedState* f, int act, int n, const int32_t* rows_dev, const float* W, const int64_t* w_off,

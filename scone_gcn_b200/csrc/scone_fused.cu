@@ -121,8 +121,11 @@ struct FuPairs {
 //   one scan      the merged rows of the live rows of a layer are walked ONCE (global loads + hash lookups); the hash slot of every
 //                 entry is kept in shared memory (ebuf) and serves the layer's forward program (or the layer-1 scalars), the marking
 //                 of the next layer's live rows and the next layer's transposed program
+//   FG            flow-gradient plan (scone_model_vjp_flows_*): every flow entry of T_0 seeds layer-1 liveness whatever its value (dL/dx
+//                 at an entry whose value is 0 reads the rows a non-zero value would make live; they hold exact zeros in the forward),
+//                 and the layer-0 transposed program goes to a.fg_off[t] (fused_flow_program)
 // ---------------------------------------------------------------------------------------------------------------------
-template <int THREADS>
+template <int THREADS, bool FG>
 __device__ __forceinline__ void plan_trajectory(const PlanArgs& a, const int t, unsigned char* sm) {
     constexpr int QUADS = THREADS / 4;
     const int HS = a.HS, LV = a.LV, EC = a.EC, L = a.L, D = a.D;
@@ -240,13 +243,13 @@ __device__ __forceinline__ void plan_trajectory(const PlanArgs& a, const int t, 
         return n;
     };
 
-    // ---- layer 1: live rows = cone edges in the merged row of a flow edge with a non-zero value ----
+    // ---- layer 1: live rows = cone edges in the merged row of a flow edge with a non-zero value (FG: any value) ----
     for (int p = fp0 + (tid >> 2); p < fp1; p += QUADS) {
         const int eo = a.flow_edge[p];
         if (eo < 0 || eo >= a.E) continue;                 // (same decision on the four lanes of the quad)
         const int e = a.rank[eo];
         const int s = set.find(e);
-        if (s < 0 || xv[s] == 0.f) continue;
+        if (s < 0 || (!FG && xv[s] == 0.f)) continue;
         const int p1 = a.mptr[e + 1];
         for (int q = a.mptr[e] + ql; q < p1; q += 4) {
             const int s2 = set.find(a.ment[q].x);
@@ -408,6 +411,26 @@ __device__ __forceinline__ void plan_trajectory(const PlanArgs& a, const int t, 
         }
     }
     __syncthreads();
+    if (FG && !s_ovf) {                                    // layer-0 transposed program: the merged row of each flow edge of T_0
+        const uint16_t* idx1 = idx0 + 1 * HS;
+        const unsigned off_fg = fused_flow_program<THREADS>(a, fp1 - fp0, s_warp, [&](int i, auto&& emit) {
+            const int eo = a.flow_edge[fp0 + i];
+            if (eo < 0 || eo >= a.E) return;
+            const int e = a.rank[eo];
+            if (set.find(e) < 0) return;
+            const int q1 = a.mptr[e + 1];
+            for (int q = a.mptr[e]; q < q1; ++q) {
+                const int2 en = a.ment[q];
+                const int s2 = set.find(en.x);
+                if (s2 >= 0 && idx1[s2] != (uint16_t)kNoRow) emit(make_int2((int)(idx1[s2] | (en.x == e ? 0x80000000u : 0u)), en.y));
+            }
+        });
+        if (tid == 0) {
+            if (off_fg == ~0u) s_ovf = 2;
+            else a.fg_off[t] = off_fg;
+        }
+        __syncthreads();
+    }
     if (s_ovf) {                                           // the arena is exhausted (the average program exceeds its share)
         if (tid == 0) {
             hdr[0] = kFusedFlagOverflow;
@@ -433,12 +456,12 @@ __device__ __forceinline__ void plan_trajectory(const PlanArgs& a, const int t, 
     }
 }
 
-template <int THREADS>
+template <int THREADS, bool FG = false>
 __global__ void __launch_bounds__(THREADS) fused_plan_kernel(const PlanArgs a) {
     extern __shared__ __align__(16) unsigned char sm[];
     const int n_work = a.tier == 0 ? a.n_work : *a.n_in;
     for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
-        plan_trajectory<THREADS>(a, a.tier == 0 ? w : a.in_list[w], sm);
+        plan_trajectory<THREADS, FG>(a, a.tier == 0 ? w : a.in_list[w], sm);
         __syncthreads();
     }
 }
@@ -465,6 +488,9 @@ struct TrajArgs {
     int big_rows;                          // rows of the per-CTA global row store
     unsigned long long* rows_done;         // optional device counters: [0] forward rows, [1] backward rows produced
     const float* cot;                      // [b][D] cotangent seed of the COT variant (target_idx / mask unused), else NULL
+    const unsigned* fg_off;                // FG variant: layer-0 transposed program of trajectory t (flow-gradient plan)
+    const int32_t* traj_ptr;               //   flow entries of trajectory t: [traj_ptr[t], traj_ptr[t + 1])
+    float* dflow;                          //   dL/dx at the flow entries, indexed like flow_val
 };
 
 template <int C>
@@ -655,7 +681,9 @@ __device__ __forceinline__ void fu_dw(float (&acc)[FuGeom<C>::TPW][4], const flo
 
 // COT (with GRAD; scone_model_vjp_*): the readout's dlogit seed is dl_j = cot_j - p_j * sum_k cot_k over ALL D slots (padded slots
 // included: quirk Q1), the NLL slot takes sum_j cot_j * logp_j and the count slot 0.  Everything after the seed is shared.
-template <int C, int ACT, bool GRAD, bool BIG, bool COT = false>
+// FG (with COT; scone_model_vjp_flows_*, flow-gradient plans): after the first layer's weight gradient, one transposed operator hop
+// without activation gives dL/dx = G_1 w0^T + S0 (G_1 w1^T) + S1 (G_1 w2^T) at the flow entries (the layer-0 program).
+template <int C, int ACT, bool GRAD, bool BIG, bool COT = false, bool FG = false>
 __global__ void __launch_bounds__(kTrajThreads, 2) fused_traj_kernel(const TrajArgs a) {
     using G = FuGeom<C>;
     extern __shared__ __align__(16) unsigned char sm[];
@@ -981,6 +1009,37 @@ __global__ void __launch_bounds__(kTrajThreads, 2) fused_traj_kernel(const TrajA
             for (int r = 0; r < n[1]; ++r) s = fmaf(l1[3 * r + k], g1[(size_t)r * G::LDH + c], s);
             acc1 = s;
         }
+        if constexpr (FG) {                                // (discarded from every other instantiation: their SASS is unchanged)
+            // u_k[r] = G_1[r] . w_k in the padding columns C .. C + 2 of the live layer-1 rows (the loop above reads columns < C) ...
+            for (int i = tid; i < 3 * n[1]; i += kTrajThreads) {
+                const int r = i / 3, k = i - 3 * r;
+                const float* g = rows + (size_t)r * G::LDH;
+                float s = 0.f;
+#pragma unroll 8
+                for (int c = 0; c < C; ++c) s = fmaf(g[c], w1s[k * C + c], s);
+                rows[(size_t)r * G::LDH + C + k] = s;
+            }
+            __syncthreads();
+            // ... then a thread per flow entry walks its row of the layer-0 program: dL/dx = sum (own ? u0 : 0) + c0 u1 + c1 u2.  The
+            // trajectory owns its output range: no atomics.  (The staging buffers may hold the next trajectory's first pieces by now:
+            // the program is read from the arena.)
+            const int nf = h[13];
+            const int* fptr = reinterpret_cast<const int*>(a.arena + a.fg_off[t]);
+            const int2* fent = reinterpret_cast<const int2*>(fptr + align2(nf + 1));
+            float* out = a.dflow + a.traj_ptr[t];
+            for (int i = tid; i < nf; i += kTrajThreads) {
+                float s = 0.f;
+                const int p1 = fptr[i + 1];
+                for (int p = fptr[i]; p < p1; ++p) {
+                    const int2 en = fent[p];
+                    const float* u = rows + (size_t)(en.x & 0xFFFF) * G::LDH + C;
+                    if (en.x < 0) s += u[0];
+                    s = fmaf((float)(short)(en.y & 0xffff), u[1], s);
+                    s = fmaf((float)(en.y >> 16), u[2], s);
+                }
+                out[i] = s;
+            }
+        }
         if (have_next && !issued_next) {                   // (no conv layer / no live row in layer 1: nothing above issued it)
             cp_async_wait_all();
             __syncthreads();
@@ -1070,31 +1129,31 @@ size_t traj_smem_bytes(int D, int cap_rows) {
     return fl * sizeof(float);
 }
 
-template <int C, int ACT, bool GRAD, bool COT>
+template <int C, int ACT, bool GRAD, bool COT, bool FG>
 int launch_traj(const TrajArgs& base, int grid_small, int grid_big, size_t smem_small, size_t smem_big, cudaStream_t st) {
     static bool configured = false;
     if (!configured) {
-        SCONE_CUDA(cudaFuncSetAttribute(fused_traj_kernel<C, ACT, GRAD, false, COT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 1024));
-        SCONE_CUDA(cudaFuncSetAttribute(fused_traj_kernel<C, ACT, GRAD, true, COT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 1024));
+        SCONE_CUDA(cudaFuncSetAttribute(fused_traj_kernel<C, ACT, GRAD, false, COT, FG>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 1024));
+        SCONE_CUDA(cudaFuncSetAttribute(fused_traj_kernel<C, ACT, GRAD, true, COT, FG>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 1024));
         configured = true;
     }
     TrajArgs a = base;
-    fused_traj_kernel<C, ACT, GRAD, false, COT><<<grid_small, kTrajThreads, smem_small, st>>>(a);
+    fused_traj_kernel<C, ACT, GRAD, false, COT, FG><<<grid_small, kTrajThreads, smem_small, st>>>(a);
     SCONE_LAUNCHED();
     if (grid_big > 0) {
         if (GRAD) a.partial = base.partial + (size_t)grid_small * (base.n_params + 2);
-        fused_traj_kernel<C, ACT, GRAD, true, COT><<<grid_big, kTrajThreads, smem_big, st>>>(a);
+        fused_traj_kernel<C, ACT, GRAD, true, COT, FG><<<grid_big, kTrajThreads, smem_big, st>>>(a);
         SCONE_LAUNCHED();
     }
     return 0;
 }
 
-template <int C, bool GRAD, bool COT = false>
+template <int C, bool GRAD, bool COT = false, bool FG = false>
 int dispatch_traj(int act, const TrajArgs& a, int gs, int gb, size_t ss, size_t sb, cudaStream_t st) {
     switch (act) {
-        case SCONE_ACT_TANH: return launch_traj<C, SCONE_ACT_TANH, GRAD, COT>(a, gs, gb, ss, sb, st);
-        case SCONE_ACT_LEAKY_RELU: return launch_traj<C, SCONE_ACT_LEAKY_RELU, GRAD, COT>(a, gs, gb, ss, sb, st);
-        case SCONE_ACT_RELU: return launch_traj<C, SCONE_ACT_RELU, GRAD, COT>(a, gs, gb, ss, sb, st);
+        case SCONE_ACT_TANH: return launch_traj<C, SCONE_ACT_TANH, GRAD, COT, FG>(a, gs, gb, ss, sb, st);
+        case SCONE_ACT_LEAKY_RELU: return launch_traj<C, SCONE_ACT_LEAKY_RELU, GRAD, COT, FG>(a, gs, gb, ss, sb, st);
+        case SCONE_ACT_RELU: return launch_traj<C, SCONE_ACT_RELU, GRAD, COT, FG>(a, gs, gb, ss, sb, st);
     }
     scone_set_error("unknown activation %d", act);
     return 2;
@@ -1134,7 +1193,9 @@ int run_traj(FusedState* f, int act, TrajArgs& t, float* grad, cudaStream_t st) 
     int rc;
     const int gs = f->grid_small, gb = f->grid_big;
     const size_t ss = f->traj_smem_small, sb = f->traj_smem_big;
-    if (f->C == 32)
+    if (want_grad && t.cot && t.dflow)
+        rc = f->C == 32 ? dispatch_traj<32, true, true, true>(act, t, gs, gb, ss, sb, st) : dispatch_traj<16, true, true, true>(act, t, gs, gb, ss, sb, st);
+    else if (f->C == 32)
         rc = !want_grad ? dispatch_traj<32, false>(act, t, gs, gb, ss, sb, st)
                         : (t.cot ? dispatch_traj<32, true, true>(act, t, gs, gb, ss, sb, st) : dispatch_traj<32, true>(act, t, gs, gb, ss, sb, st));
     else
@@ -1164,7 +1225,7 @@ bool scone_fused_supported(const scone_complex* cx, int n_layers, const int32_t*
 void scone_fused_destroy(FusedState* f) {
     if (!f) return;
     cudaFree(f->d_hdr); cudaFree(f->d_retry); cudaFree(f->d_arena); cudaFree(f->d_set_hdr); cudaFree(f->d_set_arena); cudaFree(f->d_set_bump); cudaFree(f->d_bump); cudaFree(f->d_partial); cudaFree(f->d_scratch); cudaFree(f->d_stats);
-    cudaFree(f->d_rows_done); cudaFree(f->d_sort); cudaFree(f->d_sort_tmp);
+    cudaFree(f->d_rows_done); cudaFree(f->d_sort); cudaFree(f->d_sort_tmp); cudaFree(f->d_fg_off);
     scone_table_destroy(f);
     delete f;
 }
@@ -1239,6 +1300,8 @@ int scone_fused_create(const scone_complex* cx, int L, int C, int mb, int64_t n_
     }
     SCONE_CUDA(cudaFuncSetAttribute(fused_plan_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPlanSmem));
     SCONE_CUDA(cudaFuncSetAttribute(fused_plan_kernel<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPlanSmem));
+    SCONE_CUDA(cudaFuncSetAttribute(fused_plan_kernel<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPlanSmem));
+    SCONE_CUDA(cudaFuncSetAttribute(fused_plan_kernel<1024, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxPlanSmem));
     // ---- compute kernel: shared-memory row store of the small variant, per-CTA global row store of the big one ----
     const int ldh = C + 8;
     f->cap_rows = C == 32 ? 192 : 384;
@@ -1293,11 +1356,13 @@ static int launch_plans(const scone_complex* cx, const FusedState* f, PlanArgs p
     p.HS = f->HS0; p.LV = f->LV0; p.EC = f->EC0; p.hshift = f->hshift0;
     int* retry = p.retry;
     if (!f->two_tiers) p.retry = nullptr;
-    fused_plan_kernel<256><<<b, 256, f->plan_smem0, st>>>(p);
+    if (p.fg_off) fused_plan_kernel<256, true><<<b, 256, f->plan_smem0, st>>>(p);
+    else fused_plan_kernel<256><<<b, 256, f->plan_smem0, st>>>(p);
     SCONE_LAUNCHED();
     if (f->two_tiers) {                                    // the few trajectories whose cone overflowed the first tier's tables: 1024 threads each
         p.tier = 1; p.HS = f->HS; p.LV = f->LV; p.EC = f->EC; p.hshift = f->hshift; p.n_in = p.n_retry; p.in_list = retry; p.retry = nullptr;
-        fused_plan_kernel<1024><<<std::min(b, cx->num_sms), 1024, f->plan_smem, st>>>(p);
+        if (p.fg_off) fused_plan_kernel<1024, true><<<std::min(b, cx->num_sms), 1024, f->plan_smem, st>>>(p);
+        else fused_plan_kernel<1024><<<std::min(b, cx->num_sms), 1024, f->plan_smem, st>>>(p);
         SCONE_LAUNCHED();
     }
     return 0;
@@ -1328,18 +1393,23 @@ static PlanArgs plan_args(const scone_complex* cx, FusedState* f, int off, const
 // defer_tiers (table plan only): run the first tier over this part and leave its give-ups on the chunk's work list; the later tiers
 // run once over all parts (scone_fused_plan_finish) instead of once per part — each of their launches lasts as long as its slowest
 // trajectory, whatever the number of trajectories.
+// flow_grad: a flow-gradient plan (PlanArgs::fg_off) for scone_fused_compute with dflow.
 int scone_fused_plan_part(const scone_complex* cx, FusedState* f, int off, int b, const int32_t* traj_ptr, const int32_t* flow_edge,
-                          const float* flow_val, const int32_t* last_nodes, int* overflow, cudaStream_t st, bool defer_tiers) {
+                          const float* flow_val, const int32_t* last_nodes, int* overflow, cudaStream_t st, bool defer_tiers, bool flow_grad) {
     if (b <= 0) return 0;
     SCONE_REQUIRE(off >= 0 && off + b <= f->chunk, "scone_fused_plan_part: trajectories %d .. %d exceed the planned chunk of %d", off, off + b, f->chunk);
+    if (flow_grad && !f->d_fg_off) SCONE_CUDA(cudaMalloc((void**)&f->d_fg_off, (size_t)f->chunk * sizeof(unsigned)));
     ScopedProf prof(SCONE_K_CONE, st);
     if (defer_tiers && f->tb_rows) {
         PlanArgs p = plan_args(cx, f, 0, traj_ptr, flow_edge, flow_val, last_nodes, overflow);      // absolute trajectory numbers
         p.t0 = off;
+        p.fg_off = flow_grad ? f->d_fg_off : nullptr;
         return scone_table_plan_launch(f, p, b, cx->num_sms, st, 0);
     }
     if (off > 0) SCONE_CUDA(cudaMemsetAsync(f->d_bump + 1, 0, sizeof(unsigned long long), st));   // retry counter only: the arena keeps growing
-    return launch_plans(cx, f, plan_args(cx, f, off, traj_ptr, flow_edge, flow_val, last_nodes, overflow), b, st);
+    PlanArgs p = plan_args(cx, f, off, traj_ptr, flow_edge, flow_val, last_nodes, overflow);
+    p.fg_off = flow_grad ? f->d_fg_off + off : nullptr;
+    return launch_plans(cx, f, p, b, st);
 }
 
 // The later tiers of the parts planned with defer_tiers (no-op for the hash plan, which runs its tiers per part).
@@ -1362,25 +1432,31 @@ static TrajArgs traj_args(const scone_complex* cx, const FusedState* f, const in
     t.partial = f->d_partial; t.scratch = f->d_scratch; t.scratch_stride = f->scratch_stride;
     t.cap_rows = f->cap_rows; t.big_rows = f->big_rows;
     t.rows_done = count_rows ? f->d_rows_done : nullptr;
+    t.fg_off = nullptr; t.traj_ptr = nullptr; t.dflow = nullptr;
     return t;
 }
 
 int scone_fused_compute(const scone_complex* cx, FusedState* f, int act, int b, const float* W, const int64_t* w_off, float* logprobs,
-                        const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st, const float* cot) {
+                        const int32_t* target_idx, const float* mask, float* grad, bool count_rows, cudaStream_t st, const float* cot,
+                        float* dflow, const int32_t* traj_ptr) {
     if (b <= 0) return 0;
+    SCONE_REQUIRE(dflow == nullptr || (cot && grad && traj_ptr && f->d_fg_off), "scone_fused_compute: dflow needs cot, grad, traj_ptr and a flow-gradient plan");
     TrajArgs t = traj_args(cx, f, f->d_hdr, f->d_arena, nullptr, b, W, w_off, logprobs, target_idx, mask, cot, count_rows);
+    if (dflow) {
+        t.fg_off = f->d_fg_off; t.traj_ptr = traj_ptr; t.dflow = dflow;
+    }
     return run_traj(f, act, t, grad, st);
 }
 
 int scone_fused_run(const scone_complex* cx, FusedState* f, int act, int b, const int32_t* traj_ptr, const int32_t* flow_edge,
                     const float* flow_val, const int32_t* last_nodes, const float* W, const int64_t* w_off, float* logprobs,
                     const int32_t* target_idx, const float* mask, float* grad, int* overflow, bool count_rows, cudaStream_t st,
-                    const float* cot) {
+                    const float* cot, float* dflow) {
     if (b <= 0) return 0;
     SCONE_REQUIRE(b <= f->chunk, "scone_fused_run: chunk of %d trajectories exceeds the planned %d", b, f->chunk);
     int rc = scone_fused_begin(f, st);
-    if (!rc) rc = scone_fused_plan_part(cx, f, 0, b, traj_ptr, flow_edge, flow_val, last_nodes, overflow, st);
-    if (!rc) rc = scone_fused_compute(cx, f, act, b, W, w_off, logprobs, target_idx, mask, grad, count_rows, st, cot);
+    if (!rc) rc = scone_fused_plan_part(cx, f, 0, b, traj_ptr, flow_edge, flow_val, last_nodes, overflow, st, false, dflow != nullptr);
+    if (!rc) rc = scone_fused_compute(cx, f, act, b, W, w_off, logprobs, target_idx, mask, grad, count_rows, st, cot, dflow, traj_ptr);
     return rc;
 }
 

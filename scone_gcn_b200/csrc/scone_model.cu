@@ -60,7 +60,8 @@ struct scone_model {
     int32_t *d_ptr = nullptr, *d_edge = nullptr, *d_last = nullptr, *d_tgt = nullptr, *d_nn = nullptr, *d_acc = nullptr;
     float *d_val = nullptr, *d_mask = nullptr, *d_logp_all = nullptr;
     float* d_cot = nullptr;                   // [cap_B][D] cotangents of the *_vjp_*_host entry points (allocated on first use)
-    int64_t cap_B = 0, cap_nnz = 0, cap_cot = 0;
+    float* d_dflow = nullptr;                 // [cap_dflow] flow gradients of scone_model_vjp_flows_host (allocated on first use)
+    int64_t cap_B = 0, cap_nnz = 0, cap_cot = 0, cap_dflow = 0;
     int32_t *d_choice = nullptr, *d_rand = nullptr;   // evaluation: predictions, random other targets
     float* d_evalf = nullptr;
     int64_t cap_choice = 0;
@@ -195,10 +196,18 @@ int backward_mb(scone_model* m, int32_t b, void* st) {
     return 0;
 }
 
+// dL/dx at the flow entries of a micro-batch from G_1 (after the backward; see rows_flow_grad_kernel for the three addressings)
+int flow_grad_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* G, const uint8_t* occ,
+                 const uint32_t* bm, const uint32_t* pref, float* dflow, cudaStream_t s) {
+    ScopedProf prof(SCONE_K_LAYER0_BWD, s);
+    return scone_rows_flow_grad(m->cx, b, ptr, edge, m->hidden[0], G, occ, bm, pref, m->row_cap, m->d_w + m->w_off[0], m->d_w + m->w_off[1],
+                                m->d_w + m->w_off[2], dflow, s);
+}
+
 // pipeline 0 over one micro-batch [off, off+b) (ptr / last / tgt / mask / cot: at off); grad = false: log-probs only; cot != NULL:
-// the gradient is seeded with the cotangent rows instead of tgt / mask
+// the gradient is seeded with the cotangent rows instead of tgt / mask; dflow != NULL (with cot): dL/dx at the flow entries too
 int unit_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last, float* logprobs,
-            const int32_t* tgt, const float* mask, const float* cot, bool grad, cudaStream_t s) {
+            const int32_t* tgt, const float* mask, const float* cot, float* dflow, bool grad, cudaStream_t s) {
     const int L = m->L, CL = m->hidden[L - 1];
     const float* wout = m->d_w + m->w_off[3 * L];
     m->x_clean = false;
@@ -212,7 +221,9 @@ int unit_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, 
     h.out_bm = m->d_bmG;
     rc = scone_readout_ws(m->cx, m->act, b, CL, m->d_H[L - 1], wout, last, logprobs, tgt, mask, 1.f, m->d_G[L - 1], m->d_grad + m->w_off[3 * L],
                           m->d_grad + m->n_params, m->d_grad + m->n_params + 1, 1, m->d_ws, m->d_occH[L - 1], m->d_occG[L - 1], s, &h, cot);
-    return rc ? rc : backward_mb(m, b, s);
+    if (!rc) rc = backward_mb(m, b, s);
+    if (!rc && dflow) rc = flow_grad_mb(m, b, ptr, edge, m->d_G[0], m->d_occG[0], nullptr, nullptr, dflow, s);
+    return rc;
 }
 
 // ---- buffers of the active pipeline, allocated on first use ----------------------------------------------------------
@@ -428,10 +439,14 @@ int rows_backward_mb(scone_model* m, int32_t b, cudaStream_t s) {
 
 // pipelines 1 / 2 over one micro-batch (arguments as unit_mb)
 int rows_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last, float* logprobs,
-            const int32_t* tgt, const float* mask, const float* cot, bool grad, cudaStream_t s) {
+            const int32_t* tgt, const float* mask, const float* cot, float* dflow, bool grad, cudaStream_t s) {
+    const bool compact = m->pipeline == 2;
     int rc = rows_forward_mb(m, b, ptr, edge, val, s);
     if (!rc) rc = rows_readout(m, b, last, logprobs, grad, tgt, mask, cot, s);
     if (!rc && grad) rc = rows_backward_mb(m, b, s);
+    if (!rc && grad && dflow)                              // G_1's rows: d_bmGr[0] (+ its rank prefix when compact)
+        rc = flow_grad_mb(m, b, ptr, edge, compact ? m->d_cG[0] : m->d_G[0], nullptr, m->d_bmGr[0], compact ? m->d_prefG[0] : nullptr,
+                          dflow, s);
     if (!rc) rc = rows_clear_x(m, b, ptr, edge, val, s);
     return rc;
 }
@@ -545,11 +560,13 @@ int cone_backward_mb(scone_model* m, int32_t b, cudaStream_t s) {
 
 // pipeline 3 over one micro-batch (arguments as unit_mb)
 int cone_mb(scone_model* m, int32_t b, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last, float* logprobs,
-            const int32_t* tgt, const float* mask, const float* cot, bool grad, cudaStream_t s) {
+            const int32_t* tgt, const float* mask, const float* cot, float* dflow, bool grad, cudaStream_t s) {
     int rc = cone_build_mb(m, b, ptr, edge, val, last, s);
     if (!rc) rc = cone_forward_mb(m, b, s);
     if (!rc) rc = cone_readout(m, b, last, logprobs, grad, tgt, mask, cot, s);
     if (!rc && grad) rc = cone_backward_mb(m, b, s);
+    if (!rc && grad && dflow)                              // the live rows of layer 1 (cone & support), before the bitmaps are cleared
+        rc = flow_grad_mb(m, b, ptr, edge, m->d_cG[0], nullptr, m->d_bmGr[0], m->d_prefG[0], dflow, s);
     if (!rc) rc = rows_clear_x(m, b, ptr, edge, val, s);
     if (!rc) rc = cone_clear_mb(m, b, s);
     return rc;
@@ -687,7 +704,7 @@ extern "C" int scone_model_destroy(scone_model* m) {
     if (m->ev_plan_done) cudaEventDestroy(m->ev_plan_done);
     for (auto e : m->ev_part) if (e) cudaEventDestroy(e);
     cudaFree(m->d_ptr); cudaFree(m->d_edge); cudaFree(m->d_last); cudaFree(m->d_tgt); cudaFree(m->d_val);
-    cudaFree(m->d_mask); cudaFree(m->d_logp_all); cudaFree(m->d_nn); cudaFree(m->d_acc); cudaFree(m->d_cot);
+    cudaFree(m->d_mask); cudaFree(m->d_logp_all); cudaFree(m->d_nn); cudaFree(m->d_acc); cudaFree(m->d_cot); cudaFree(m->d_dflow);
     cudaFree(m->d_choice); cudaFree(m->d_rand); cudaFree(m->d_evalf);
     delete m;
     return 0;
@@ -757,14 +774,14 @@ static int finish_call(scone_model* m, int rc, void* user_st) {
 
 // pipeline 4: the micro-batch is walked in chunks the program arena was sized for (scone_fused_create)
 static int fused_call(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last,
-                      float* logprobs, const int32_t* tgt, const float* mask, const float* cot, bool grad, cudaStream_t s) {
+                      float* logprobs, const int32_t* tgt, const float* mask, const float* cot, float* dflow, bool grad, cudaStream_t s) {
     const int step = m->fused->chunk < m->mb ? m->fused->chunk : m->mb;
     for (int32_t off = 0; off < B; off += step) {
         const int32_t b = B - off < step ? B - off : step;
         int rc = scone_fused_run(m->cx, m->fused, m->act, b, ptr + off, edge, val, last + off, m->d_w, m->w_off.data(),
                                  logprobs ? logprobs + (size_t)off * m->cx->D : nullptr, grad && !cot ? tgt + off : nullptr,
                                  grad && !cot ? mask + off : nullptr, grad ? m->d_grad : nullptr, m->d_overflow, g_scone_prof, s,
-                                 grad && cot ? cot + (size_t)off * m->cx->D : nullptr);
+                                 grad && cot ? cot + (size_t)off * m->cx->D : nullptr, grad && cot ? dflow : nullptr);
         if (rc) return rc;
     }
     return 0;
@@ -836,23 +853,23 @@ static int fused_host_overlapped(scone_model* m, int32_t B, const int32_t* ptr, 
 
 // Forward (grad = false: log-probs to logprobs [B][D]) or loss + gradient (grad = true: into d_grad, cleared first if zero_first).
 // cot != NULL (grad): the VJP — the gradient is seeded with the cotangent rows [B][D] instead of tgt / mask, and count_add is added to
-// the count slot.
+// the count slot; dflow != NULL (with cot): dL/dx at the flow entries [ptr[0], ptr[B]) too, indexed like val.
 static int run_batch(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val, const int32_t* last,
                      float* logprobs, const int32_t* tgt, const float* mask, bool grad, int32_t zero_first, void* user_st,
-                     const float* cot = nullptr, float count_add = 0.f) {
+                     const float* cot = nullptr, float count_add = 0.f, float* dflow = nullptr) {
     if (fork_to_compute(m, user_st)) return 1;
     cudaStream_t s = m->compute;
     if (grad && zero_first) SCONE_CUDA(cudaMemsetAsync(m->d_grad, 0, (m->n_params + 2) * sizeof(float), s));
     if (grad && cot && count_add != 0.f && scone_add_scalar_launch(m->d_grad + m->n_params + 1, count_add, s)) return finish_call(m, 1, user_st);
     const int pl = m->pipeline;
-    if (pl == 4) return finish_call(m, fused_call(m, B, ptr, edge, val, last, logprobs, tgt, mask, cot, grad, s), user_st);
+    if (pl == 4) return finish_call(m, fused_call(m, B, ptr, edge, val, last, logprobs, tgt, mask, cot, dflow, grad, s), user_st);
     auto step = pl == 3 ? cone_mb : pl >= 1 ? rows_mb : unit_mb;
     int rc = 0;
     for (int32_t off = 0; off < B && !rc; off += m->mb) {
         const int32_t b = B - off < m->mb ? B - off : m->mb;
         rc = step(m, b, ptr + off, edge, val, last + off, grad ? m->d_logp : logprobs + (size_t)off * m->cx->D,
                   grad && !cot ? tgt + off : nullptr, grad && !cot ? mask + off : nullptr, grad && cot ? cot + (size_t)off * m->cx->D : nullptr,
-                  grad, s);
+                  grad && cot ? dflow : nullptr, grad, s);
     }
     return finish_call(m, rc, user_st);
 }
@@ -1004,6 +1021,41 @@ extern "C" int scone_model_vjp_host(scone_model* m, int32_t B, const int32_t* pt
     if (rc) return rc;
     if (overlap) return fused_host_overlapped(m, B, ptr, edge, val, nullptr, true, zero_first, s, m->d_cot, count_add);
     return scone_model_vjp_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, B > 0 ? m->d_cot : nullptr, count_add, zero_first, st);
+}
+
+extern "C" int scone_model_vjp_flows_dev(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
+                                         const int32_t* last, const float* cot, float count_add, int32_t zero_first, float* dflow,
+                                         void* user_st) {
+    SCONE_REQUIRE(m && ptr && last && B >= 0, "scone_model_vjp_flows_dev: bad arguments");
+    SCONE_REQUIRE((cot && dflow) || B == 0, "scone_model_vjp_flows_dev: cot or dflow is NULL");
+    return run_batch(m, B, ptr, edge, val, last, nullptr, nullptr, nullptr, true, zero_first, user_st, cot, count_add, dflow);
+}
+
+// the plain staged path (no part-wise copy overlap): dflow is a host output, so the call ends with a stream synchronise anyway
+extern "C" int scone_model_vjp_flows_host(scone_model* m, int32_t B, const int32_t* ptr, const int32_t* edge, const float* val,
+                                          const int32_t* last, const float* cot, float count_add, int32_t zero_first, float* dflow,
+                                          void* st) {
+    SCONE_REQUIRE(m && ptr && last && B >= 0, "scone_model_vjp_flows_host: bad arguments");
+    SCONE_REQUIRE((cot && dflow) || B == 0, "scone_model_vjp_flows_host: cot or dflow is NULL");
+    cudaStream_t s = as_stream(st);
+    const int64_t p0 = B > 0 ? ptr[0] : 0, nnz = B > 0 ? ptr[B] : 0;
+    int rc = stage_host_inputs(m, B, ptr, last, nullptr, nullptr, nullptr, edge, val, true, s);
+    if (!rc) rc = stage_cot(m, B, cot, s);
+    if (rc) return rc;
+    if (nnz > m->cap_dflow) {
+        cudaFree(m->d_dflow);
+        m->d_dflow = nullptr;
+        m->cap_dflow = 0;
+        const int64_t cap = nnz + nnz / 4 + 16;
+        SCONE_CUDA(cudaMalloc((void**)&m->d_dflow, cap * sizeof(float)));
+        m->cap_dflow = cap;
+    }
+    rc = scone_model_vjp_flows_dev(m, B, m->d_ptr, m->d_edge, m->d_val, m->d_last, B > 0 ? m->d_cot : nullptr, count_add, zero_first,
+                                   m->d_dflow, st);
+    if (rc) return rc;
+    if (nnz > p0) SCONE_CUDA(cudaMemcpyAsync(dflow + p0, m->d_dflow + p0, (size_t)(nnz - p0) * sizeof(float), cudaMemcpyDeviceToHost, s));
+    SCONE_CUDA(cudaStreamSynchronize(s));
+    return 0;
 }
 
 extern "C" int scone_model_read_grads_async(scone_model* m, float* out_pinned, void* st) {

@@ -285,7 +285,9 @@ __host__ __device__ inline size_t table_plan_smem(int M, int LV) {
 //   3  one pass over the live rows of all layers counts the entries of every program row; ONE scan gives every row pointer and the
 //      size of the trajectory's piece of the arena (allocated inside the scan)
 //   4  one pass writes everything: layer-1 scalars, forward and transposed programs (entries in column order), readout pairs
-template <int THREADS>
+// FG (flow-gradient plan, as the hash plan's): in phase 1 every flow entry of T_0 marks its row live whatever its value, and the
+// layer-0 transposed program (the node table's row of each flow entry, filtered by the live layer-1 rows) goes to a.fg_off[t].
+template <int THREADS, bool FG>
 __device__ __forceinline__ void table_plan_trajectory(const PlanArgs& a, const int t, unsigned char* sm) {
     constexpr int QUADS = THREADS / 4;
     const int M = a.M, LV = a.LV, L = a.L, D = a.D, W = M >> 5;
@@ -389,7 +391,7 @@ __device__ __forceinline__ void table_plan_trajectory(const PlanArgs& a, const i
         if (lo >= m || keys[lo] != e) continue;
         const float v = a.flow_val[p];
         x[lo] = v;
-        if (v == 0.f) continue;
+        if (!FG && v == 0.f) continue;
         const unsigned q1 = rp[lo + 1];
         for (unsigned q = rp[lo]; q < q1; ++q) {
             const int j = ent[q].x & 0xFFFF;
@@ -612,6 +614,34 @@ __device__ __forceinline__ void table_plan_trajectory(const PlanArgs& a, const i
             edst[i] = make_int2((int)(r | ((uint32_t)pr.x & 0xFFFF0000u)), pr.y);
         }
     }
+    if (FG) {
+        const unsigned off_fg = fused_flow_program<THREADS>(a, fp1 - fp0, s_warp, [&](int i, auto&& emit) {
+            const int eo = a.flow_edge[fp0 + i];
+            if (eo < 0 || eo >= a.E) return;
+            const uint32_t e = (uint32_t)a.rank[eo];
+            int lo = 0, hi = m;
+            while (lo < hi) {
+                const int mid = (lo + hi) >> 1;
+                if (keys[mid] < e) lo = mid + 1;
+                else hi = mid;
+            }
+            if (lo >= m || keys[lo] != e) return;
+            const unsigned q1 = rp[lo + 1];
+            for (unsigned q = rp[lo]; q < q1; ++q) {
+                const int2 en = ent[q];
+                const uint32_t r = idx[en.x & 0xFFFF];        // rank among the live rows of layer 1
+                if (r != kNoRow) emit(make_int2((int)(r | ((uint32_t)en.x & 0x80000000u)), en.y));
+            }
+        });
+        if (off_fg == ~0u) {                               // (uniform) the arena is exhausted
+            if (tid == 0) {
+                hdr[0] = kFusedFlagOverflow;
+                *a.overflow = 1;
+            }
+            return;
+        }
+        if (tid == 0) a.fg_off[t] = off_fg;
+    }
     if (tid == 0) {
         hdr[0] = 0;
         for (int l = 1; l <= kFusedMaxL; ++l) hdr[l] = l <= L ? n_l[l] : 0;
@@ -630,12 +660,12 @@ __device__ __forceinline__ void table_plan_trajectory(const PlanArgs& a, const i
     }
 }
 
-template <int THREADS>
+template <int THREADS, bool FG = false>
 __global__ void __launch_bounds__(THREADS) table_plan_kernel(const PlanArgs a) {
     extern __shared__ __align__(16) unsigned char sm[];
     const int n_work = a.tier == 0 ? a.n_work : *a.n_in;
     for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
-        table_plan_trajectory<THREADS>(a, a.tier == 0 ? a.t0 + w : a.in_list[w], sm);
+        table_plan_trajectory<THREADS, FG>(a, a.tier == 0 ? a.t0 + w : a.in_list[w], sm);
         __syncthreads();
     }
 }
@@ -777,6 +807,9 @@ int scone_table_build(const scone_complex* cx, FusedState* f, int L, bool* ok) {
         SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
         SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
         SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<kTier1Threads>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
+        SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
+        SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
+        SCONE_CUDA(cudaFuncSetAttribute(table_plan_kernel<kTier1Threads, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxTablePlanSmem));
     }
     *ok = true;
     return 0;
@@ -798,8 +831,10 @@ int scone_table_plan_launch(const FusedState* f, PlanArgs p, int b, int num_sms,
     int* cnt1 = p.n_retry + 1;
     p.retry = f->tb_two_tiers ? list0 : nullptr;
     p.n_retry = cnt0;
+    const bool fg = p.fg_off != nullptr;                   // flow-gradient plan: the FG instantiations
     if (phase != 1) {
-        table_plan_kernel<128><<<b, 128, f->tb_smem0, st>>>(p);
+        if (fg) table_plan_kernel<128, true><<<b, 128, f->tb_smem0, st>>>(p);
+        else table_plan_kernel<128><<<b, 128, f->tb_smem0, st>>>(p);
         SCONE_LAUNCHED();
     }
     if (!f->tb_two_tiers || phase == 0) return 0;
@@ -808,14 +843,16 @@ int scone_table_plan_launch(const FusedState* f, PlanArgs p, int b, int num_sms,
     if (f->tb_mid_tier) {                                  // tables for all but the largest cones: 256 threads, several CTAs per SM
         p.tier = 1; p.M = f->tbM1; p.LV = f->tbLV1; p.n_in = n_in; p.in_list = in_list; p.retry = list1; p.n_retry = cnt1;
         const int per_sm = std::max(1, std::min(8, (int)((size_t)220 * 1024 / (f->tb_smem1 + 1024))));
-        table_plan_kernel<256><<<std::min(b, per_sm * num_sms), 256, f->tb_smem1, st>>>(p);
+        if (fg) table_plan_kernel<256, true><<<std::min(b, per_sm * num_sms), 256, f->tb_smem1, st>>>(p);
+        else table_plan_kernel<256><<<std::min(b, per_sm * num_sms), 256, f->tb_smem1, st>>>(p);
         SCONE_LAUNCHED();
         n_in = cnt1;
         in_list = list1;
     }
     p.tier = 2; p.M = f->tbM; p.LV = f->tbLV; p.n_in = n_in; p.in_list = in_list; p.retry = nullptr; p.n_retry = cnt0;
     const int per_sm = std::max(1, std::min(4, (int)((size_t)220 * 1024 / (f->tb_smem + 1024))));
-    table_plan_kernel<512><<<std::min(b, per_sm * num_sms), 512, f->tb_smem, st>>>(p);
+    if (fg) table_plan_kernel<512, true><<<std::min(b, per_sm * num_sms), 512, f->tb_smem, st>>>(p);
+    else table_plan_kernel<512><<<std::min(b, per_sm * num_sms), 512, f->tb_smem, st>>>(p);
     SCONE_LAUNCHED();
     return 0;
 }

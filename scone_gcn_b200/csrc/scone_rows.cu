@@ -472,6 +472,64 @@ __global__ void __launch_bounds__(32 * kL0bWarps) rows_layer0_bwd_kernel(const f
     }
 }
 
+// dL/dx at the flow entries (scone_model_vjp_flows_*): the first layer's transposed operator hop without activation,
+// dL/dx_e = sum over the merged operator row of e of G_1[col] . (own w0 + c0 w1 + c1 w2) (the operators are symmetric).  One warp
+// per trajectory walks its flow entries in CSR order; a lane owns channels lane and lane + 32, sums its terms in row order, and a
+// fixed butterfly adds the lanes: deterministic, no atomics.  G_1 is read through the pipeline's addressing — MODE 0: dense rows
+// e * b + t with byte flags (pipeline 0), 1: dense rows with a row bitmap (pipeline 1), 2: compact trajectory-major rows through the
+// bitmap and rank prefix (pipelines 2 / 3; an index at or beyond cap was never written: capacity overflow, reported by the flag).  A
+// row that is not there is an exact zero; an entry whose edge id is out of range gets 0.
+template <int MODE>
+__global__ void __launch_bounds__(256) rows_flow_grad_kernel(const int32_t* __restrict__ traj_ptr, const int32_t* __restrict__ flow_edge,
+                                                            const int32_t* __restrict__ rank, const int32_t* __restrict__ mptr,
+                                                            const int2* __restrict__ ment, const float* __restrict__ G,
+                                                            const uint8_t* __restrict__ occ, const uint32_t* __restrict__ bm,
+                                                            const uint32_t* __restrict__ pref, const float* __restrict__ w0,
+                                                            const float* __restrict__ w1, const float* __restrict__ w2,
+                                                            float* __restrict__ dflow, int b, int E, int C, int cap) {
+    const int lane = threadIdx.x & 31;
+    const int t = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    if (t >= b) return;
+    float wa[2], wb[2], wc[2];
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        const int c = lane + 32 * h;
+        wa[h] = c < C ? w0[c] : 0.f;
+        wb[h] = c < C ? w1[c] : 0.f;
+        wc[h] = c < C ? w2[c] : 0.f;
+    }
+    const int p1 = traj_ptr[t + 1];
+    for (int p = traj_ptr[t]; p < p1; ++p) {
+        const int eo = flow_edge[p];
+        float s = 0.f;
+        if (eo >= 0 && eo < E) {
+            const int e = rank[eo];
+            const int q1 = mptr[e + 1];
+            for (int q = mptr[e]; q < q1; ++q) {
+                const int2 en = ment[q];
+                const float* g = nullptr;
+                if (MODE == 2) {
+                    unsigned idx;
+                    if (rank_lookup(bm, pref, (unsigned)t * (unsigned)E + (unsigned)en.x, idx) && idx < (unsigned)cap) g = G + (size_t)idx * C;
+                } else {
+                    const size_t row = (size_t)en.x * b + t;
+                    if (MODE == 0 ? occ[row] != 0 : bit_test(bm, row)) g = G + row * C;
+                }
+                if (g == nullptr) continue;                // (warp-uniform)
+                const float own = en.x == e ? 1.f : 0.f, c0 = (float)(short)(en.y & 0xffff), c1 = (float)(en.y >> 16);
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    const int c = lane + 32 * h;
+                    if (c < C) s = fmaf(g[c], fmaf(c1, wc[h], fmaf(c0, wb[h], own * wa[h])), s);
+                }
+            }
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        if (lane == 0) dflow[p] = s;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // Backward over a row list (the candidate rows of Gprev = rows where S G can be non-zero): same gather as the forward row
 // kernel on G (flag test = row bitmap of G), the three gathered terms A_k are (1) stored compactly, row i of the list at
@@ -1387,6 +1445,23 @@ int scone_rows_layer0_backward(const scone_complex* cx, int b, int cout, const f
 #undef SCONE_L0B
     SCONE_LAUNCHED();
     rows_reduce_kernel<<<(3 * cout + 31) / 32, 256, 0, st>>>(ws, kDwCtas, 3 * cout, dW, accumulate);
+    SCONE_LAUNCHED();
+    return 0;
+}
+
+int scone_rows_flow_grad(const scone_complex* cx, int b, const int32_t* traj_ptr, const int32_t* flow_edge, int C, const float* G,
+                         const uint8_t* occ, const uint32_t* bm, const uint32_t* pref, int cap, const float* w0, const float* w1,
+                         const float* w2, float* dflow, cudaStream_t st) {
+    SCONE_REQUIRE(C >= 1 && C <= 64, "scone_rows_flow_grad: width %d", C);
+    if (b <= 0) return 0;
+    const unsigned grid = (unsigned)((b + 7) / 8);
+#define SCONE_FLOWG(MODE)                                                                                                       \
+    rows_flow_grad_kernel<MODE><<<grid, 256, 0, st>>>(traj_ptr, flow_edge, cx->d_rank, cx->d_mptr, cx->d_ment, G, occ, bm, pref, w0, w1, w2, \
+                                                      dflow, b, cx->E, C, cap)
+    if (occ) SCONE_FLOWG(0);
+    else if (pref) SCONE_FLOWG(2);
+    else SCONE_FLOWG(1);
+#undef SCONE_FLOWG
     SCONE_LAUNCHED();
     return 0;
 }

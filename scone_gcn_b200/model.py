@@ -124,6 +124,19 @@ class SconeModel:
                    'scone_model_vjp_host')
         return self.read_grads(stream) if read else None
 
+    def vjp_flows(self, traj_ptr, flow_edge, flow_val, last_nodes, cot, count_add, zero_first=True, stream=None):
+        """vjp() that also differentiates with respect to the flow values: returns (buffer, dflow), the [grads | nll_sum | count]
+        buffer and dflow[p] = d(sum cot * logprob) / d flow_val[p] (float32, shaped like flow_val; entries outside
+        [traj_ptr[0], traj_ptr[B]) are 0)."""
+        B = len(last_nodes)
+        a = [np.ascontiguousarray(traj_ptr, np.int32), np.ascontiguousarray(flow_edge, np.int32),
+             np.ascontiguousarray(flow_val, np.float32), np.ascontiguousarray(last_nodes, np.int32),
+             np.ascontiguousarray(cot, np.float32).reshape(B, self.cx.D)]
+        dflow = np.zeros(a[2].shape, np.float32)
+        _lib.check(_lib.lib().scone_model_vjp_flows_host(self.handle, B, *[_lib.ptr(x) for x in a], float(count_add), int(zero_first),
+                                                         _lib.ptr(dflow), stream), 'scone_model_vjp_flows_host')
+        return self.read_grads(stream), dflow
+
     def accuracy(self, traj_ptr, flow_edge, flow_val, last_nodes, n_nbrs, target_idx, mask, stream=None):
         """(correct, counted) over the trajectories with mask != 0: forward + argmax on the device
         (scone_trajectory_model.py:59-71; slots >= n_nbrs count as -100, first maximum wins)."""

@@ -5,10 +5,12 @@
     loss.backward()                                      # w_flat.grad = dloss/dW through scone_model_vjp_dev
 
 The forward runs scone_model_forward_dev and the backward scone_model_vjp_dev (which recomputes the forward inside the same
-fused pass), both on the current torch stream.  The op uses the model's own device buffers: forward and backward each write
-w_flat into net.weights_tensor() first, and the backward overwrites the gradient buffer net.grads_tensor() (zero_first); anything
-the caller keeps in those buffers across a call is replaced.  The flows get no gradient (the reference never differentiates
-w.r.t. them)."""
+fused pass), both on the current torch stream.  When flow_val requires grad (a learned flow encoder, a trained per-edge mask or
+scale, a saliency map over the edges of a path, an adversarial perturbation) the backward runs scone_model_vjp_flows_dev instead
+and flow_val.grad receives dloss/dflow_val; the weight gradient is the same either way.  The op uses the model's own device
+buffers: forward and backward each write w_flat into net.weights_tensor() first, and the backward overwrites the gradient buffer
+net.grads_tensor() (zero_first); anything the caller keeps in those buffers across a call is replaced.  traj_ptr, flow_edge and
+last_nodes are integer inputs and get no gradient."""
 import torch
 
 from . import _lib
@@ -47,13 +49,20 @@ class _LogProbs(torch.autograd.Function):
         net = ctx.net
         B = last_nodes.numel()
         stream = torch.cuda.current_stream().cuda_stream
+        want_flows = ctx.needs_input_grad[3]
+        dflow = torch.zeros_like(flow_val) if want_flows else None      # (entries outside [traj_ptr[0], traj_ptr[B]) stay 0)
         if B == 0:
-            return torch.zeros_like(w_flat), None, None, None, None, None
+            return torch.zeros_like(w_flat), None, None, dflow, None, None
         cot = grad_out.to(torch.float32).contiguous()
         net.weights_tensor().copy_(w_flat)                 # the model's weights may have changed since the forward
-        _lib.check(_lib.lib().scone_model_vjp_dev(net.handle, B, _lib.dptr(traj_ptr), _lib.dptr(flow_edge), _lib.dptr(flow_val),
-                                                  _lib.dptr(last_nodes), _lib.dptr(cot), 0.0, 1, stream), 'scone_model_vjp_dev')
-        return net.grads_tensor()[:net.n_params].clone(), None, None, None, None, None
+        if want_flows:
+            _lib.check(_lib.lib().scone_model_vjp_flows_dev(net.handle, B, _lib.dptr(traj_ptr), _lib.dptr(flow_edge), _lib.dptr(flow_val),
+                                                            _lib.dptr(last_nodes), _lib.dptr(cot), 0.0, 1, _lib.dptr(dflow), stream),
+                       'scone_model_vjp_flows_dev')
+        else:
+            _lib.check(_lib.lib().scone_model_vjp_dev(net.handle, B, _lib.dptr(traj_ptr), _lib.dptr(flow_edge), _lib.dptr(flow_val),
+                                                      _lib.dptr(last_nodes), _lib.dptr(cot), 0.0, 1, stream), 'scone_model_vjp_dev')
+        return net.grads_tensor()[:net.n_params].clone(), None, None, dflow, None, None
 
 
 def logprobs(net, w_flat, traj_ptr, flow_edge, flow_val, last_nodes):

@@ -1,7 +1,8 @@
 """Trajectories/s of the log-prob VJP (scone_model_vjp_dev, dense random cotangent) against the one-hot loss + gradient
 (scone_model_loss_grad_dev) on bench.py's workload shape, inputs resident on the device, the two calls timed alternately with CUDA
-events.  A report, not a gate.  Prints one JSON line with the GPU's name and power limit.
-    python tools/vjp_bench.py [--config cfg5] [--steps 20] [--warmup 5] [--rounds 3]"""
+events.  A report, not a gate.  Prints one JSON line with the GPU's name and power limit.  --flows times the VJP that also returns
+the gradient with respect to the flow values (scone_model_vjp_flows_dev) against scone_model_vjp_dev instead.
+    python tools/vjp_bench.py [--config cfg5] [--steps 20] [--warmup 5] [--rounds 3] [--flows]"""
 import argparse
 import json
 import os
@@ -31,6 +32,7 @@ def main():
     ap.add_argument('--steps', type=int, default=20)
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--rounds', type=int, default=3)
+    ap.add_argument('--flows', action='store_true', help='vjp_flows_dev against vjp_dev')
     args = ap.parse_args()
     import scone_gcn_b200 as sg
     from scone_gcn_b200 import _lib
@@ -48,7 +50,7 @@ def main():
     d = {k: torch.as_tensor(np.ascontiguousarray(v), device=dev) for k, v in dict(
         ptr=sp.traj_ptr[:B + 1].astype(np.int32), edge=sp.flow_edge[:p1].astype(np.int32), val=sp.flow_val[:p1].astype(np.float32),
         last=sp.last_nodes[:B].astype(np.int32), tgt=sp.target_idx[:B].astype(np.int32), mask=np.ones(B, np.float32),
-        cot=rs.uniform(-0.25, 1.0, size=(B, cx.D)).astype(np.float32)).items()}
+        cot=rs.uniform(-0.25, 1.0, size=(B, cx.D)).astype(np.float32), dflow=np.zeros(p1, np.float32)).items()}
     stream = torch.cuda.current_stream().cuda_stream
     L = _lib.lib()
     flows = [_lib.dptr(d[k]) for k in ('ptr', 'edge', 'val', 'last')]
@@ -58,6 +60,10 @@ def main():
         'vjp_dev': lambda: _lib.check(L.scone_model_vjp_dev(net.handle, B, *flows, _lib.dptr(d['cot']), float(B), 1, stream),
                                       'scone_model_vjp_dev'),
     }
+    if args.flows:
+        del calls['loss_grad_dev']
+        calls['vjp_flows_dev'] = lambda: _lib.check(L.scone_model_vjp_flows_dev(net.handle, B, *flows, _lib.dptr(d['cot']), float(B), 1,
+                                                                                _lib.dptr(d['dflow']), stream), 'scone_model_vjp_flows_dev')
     for f in calls.values():
         for _ in range(args.warmup):
             f()
@@ -78,7 +84,10 @@ def main():
     for name, v in ms.items():
         out[name] = {'ms_per_call_median': float(np.median(v)), 'ms_per_call_rounds': [round(x, 4) for x in v],
                      'trajectories_per_s': B / (float(np.median(v)) * 1e-3)}
-    out['vjp_over_loss_grad_time'] = out['vjp_dev']['ms_per_call_median'] / out['loss_grad_dev']['ms_per_call_median']
+    if args.flows:
+        out['vjp_flows_over_vjp_time'] = out['vjp_flows_dev']['ms_per_call_median'] / out['vjp_dev']['ms_per_call_median']
+    else:
+        out['vjp_over_loss_grad_time'] = out['vjp_dev']['ms_per_call_median'] / out['loss_grad_dev']['ms_per_call_median']
     print(json.dumps(out), flush=True)
 
 
